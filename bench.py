@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...   # the reference's CPU arithmetic (oracle port)
     python bench.py --workload netflix|powerlaw256|rank ...   # BASELINE.json configs 3, 4 (scaled) and 5
+    python bench.py ... --dump-outputs DIR                    # also write the last timed step's outputs as DIR/*.npy
 
 A "step" is one ALS epoch (user half-step + item half-step, each with its Gram) over a synthetic count matrix,
 weighted, log preprocessing; metric = 2*nnz / t_epoch. `value` is measured with the matrices resident in HBM;
@@ -24,6 +25,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True   # the bench writes nothing into the source tree, which may be read-only
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -41,6 +43,19 @@ WORKLOADS = {
 }
 GAMMA, ALPHA, BETA = 0.1, 10, 1
 L2_NOTE = "inputs larger than L2, no flush (CSR + transpose + factors streamed every epoch)"
+DUMP_BYTES = 64_000_000   # --dump-outputs writes at most this much in all
+
+
+def dump_outputs(dirname, arrays):
+    """Write each float32 array as <dirname>/<name>.npy. An array larger than its equal share of DUMP_BYTES keeps a
+    fixed sample of its rows (seed 0, ascending), the same rows for the same workload on every run and build."""
+    os.makedirs(dirname, exist_ok=True)
+    share = DUMP_BYTES // len(arrays) - 4096   # room for the .npy header
+    for name, a in arrays.items():
+        if a.nbytes > share:
+            keep = share // (a.nbytes // len(a))
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))]
+        np.save(os.path.join(dirname, name + ".npy"), a)
 
 
 def env_int(name, default):
@@ -295,6 +310,8 @@ def run_rank(args, device, world, rank):
         ids = engine.score_topk(users_d, cand_d, U, V, 100)
     e1.record()
     torch.cuda.synchronize(device)
+    # the last step's top-100 item ids of this rank's users (ids below 2**24 are exact in float32)
+    outputs = {"topk_ids": ids.float().cpu().numpy()} if args.dump_outputs and rank == 0 else None
     ms = torch.tensor([e0.elapsed_time(e1) / args.steps], dtype=torch.float64, device=device)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
@@ -326,6 +343,8 @@ def run_rank(args, device, world, rank):
                         "what": "WMF.rank_batch(all items, this rank's users, 100) with host arrays"},
                 "gpu_launches": None, "clocks": clocks}
         print(json.dumps(line), flush=True)
+        if outputs:
+            dump_outputs(args.dump_outputs, outputs)
 
 
 def run_ours(args):
@@ -416,6 +435,8 @@ def run_ours(args):
         epoch(record=True)
     stop.record()
     sync_all()
+    # the factors the last epoch left (full matrices on every rank), before the legs below run anything else
+    outputs = {"users": loop.users.cpu().numpy(), "items": loop.items.cpu().numpy()} if args.dump_outputs and rank == 0 else None
     elapsed_ms = torch.tensor([start.elapsed_time(stop)], dtype=torch.float64, device=device)
     if world > 1:
         dist.all_reduce(elapsed_ms, op=dist.ReduceOp.MAX)
@@ -465,7 +486,6 @@ def run_ours(args):
         tr_host, te_host = split_train_test(C_host, train=0.8, seed=1993)
         if not args.pageable:
             tr_host, te_host = pin_csr(tr_host), pin_csr(te_host)   # the contract's e2e inputs: pinned host memory
-        e2e_steps = max(1, min(args.steps, 5))
 
         def e2e_step():
             t0 = time.perf_counter()
@@ -478,7 +498,7 @@ def run_ours(args):
         e2e_step()  # second warm-up: pinned staging / host allocator caches reach steady state
         sync_all()
         times, marks = [], []
-        for _ in range(e2e_steps):
+        for _ in range(args.steps):
             sync_all()
             t, d2h = e2e_step()
             times.append(t)
@@ -555,6 +575,8 @@ def run_ours(args):
             "clocks": clocks,
         }
         print(json.dumps(line), flush=True)
+        if outputs:
+            dump_outputs(args.dump_outputs, outputs)
     loop.graphs = None
     del loop
     finish(world, device)
@@ -588,7 +610,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true", help="kernel tuning runs: skip the end-to-end leg (the line's e2e is NaN)")
     ap.add_argument("--no-graphs", action="store_true", help="launch the epoch from Python instead of replaying CUDA graphs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps write what the last one computed as DIR/<name>.npy (float32, at most "
+                         "64 MB in all; a fixed sample of rows where an output is larger): users.npy and items.npy, the "
+                         "factors after the last epoch, or topk_ids.npy for --workload rank")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of this package's CUDA path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,3 +1,4 @@
+import hashlib
 import os
 import sys
 
@@ -40,6 +41,33 @@ def pytest_sessionfinish(session, exitstatus):
 def load_golden(name):
     z = np.load(os.path.join(GOLDEN_DIR, name + ".npz"))
     return {k: z[k] for k in z.files}
+
+
+def array_digest(*arrays):
+    h = hashlib.sha256()
+    for a in arrays:
+        h.update(np.ascontiguousarray(a).tobytes())
+    return h.hexdigest()
+
+
+def load_golden_2000x1500():
+    """The reference's two half-steps at 2000 x 1500, f = 128 (tests/golden/make_golden.py::case_half_steps) in the
+    layout of load_golden(). Only the reference's outputs are stored, to keep the files small: the user half-step in
+    full (the item half-step's input) and the item half-step on the rows in ``items_half1_rows``. The inputs are
+    regenerated from their seeds and checked against digests of what the reference was given."""
+    from oracle.wmf_oracle import init_items
+    from recmodel_b200.synthetic import make_counts
+    g = load_golden("weighted_nobias_f128_2000x1500")
+    g.update(load_golden("weighted_nobias_f128_2000x1500_items"))
+    C = make_counts(2000, 1500, 150_000, seed=18, planted_rank=8)
+    g.update(train_indptr=C.indptr.astype(np.int64), train_indices=C.indices.astype(np.int32),
+             train_data=C.data.astype(np.float32), train_shape=np.array(C.shape, dtype=np.int64))
+    g["items0"] = init_items(1500, 128, False, seed=1993)
+    assert array_digest(g["train_indptr"], g["train_indices"], g["train_data"]) == str(g["train_sha256"]), \
+        "recmodel_b200.synthetic.make_counts no longer generates the matrix the reference was given"
+    assert array_digest(g["items0"]) == str(g["items0_sha256"]), \
+        "oracle.wmf_oracle.init_items no longer generates the factors the reference was given"
+    return g
 
 
 def csr_from(g, prefix):

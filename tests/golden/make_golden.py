@@ -1,11 +1,11 @@
-"""Generate tests/golden/*.npz by EXECUTING the unmodified reference (this container only).
+"""Generate tests/golden/*.npz by EXECUTING the unmodified reference.
 
-    python tests/golden/make_golden.py
+    WMF_REFERENCE_ROOT=<checkout of titoeb/RecModel> python tests/golden/make_golden.py
 
-Runs /root/reference/RecModel/wmf_model.py through oracle/ref_shim.py on small seeded
+Runs the reference's RecModel/wmf_model.py through oracle/ref_shim.py on small seeded
 synthetic inputs (recmodel_b200.synthetic) and stores inputs + reference outputs. The
-committed .npz files are what the oracle and the CUDA path are checked against on machines
-where /root/reference does not exist (the GPU box).
+committed .npz files are what the oracle and the CUDA path are checked against; the tests
+need no copy of the reference.
 """
 import io
 import os
@@ -16,7 +16,9 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.abspath(os.path.join(HERE, "..", "..")))
+sys.path.insert(0, os.path.abspath(os.path.join(HERE, "..")))
 
+from conftest import array_digest  # noqa: E402
 from oracle.ref_shim import load_reference_wmf  # noqa: E402
 from recmodel_b200.synthetic import make_counts, split_train_test  # noqa: E402
 
@@ -107,20 +109,23 @@ def case_unweighted(name, users, items, nnz, dim, iterations, seed):
 
 
 def case_half_steps(name, users, items, nnz, dim, seed):
-    """A larger fixture for the tensor-core shapes: only the two half-steps of the reference (no train loop), so the
-    file stays small enough to commit."""
+    """A larger fixture for the tensor-core shapes: only the two half-steps of the reference (no train loop). The
+    inputs are not stored (tests/conftest.py::load_golden_2000x1500 regenerates them and checks them against the
+    digests), nor the item half-step beyond every fifth row, so that each file stays under 1 MB."""
     WMF = load_reference_wmf()
     full = make_counts(users, items, nnz, seed=seed, planted_rank=8)
-    out = {}
-    out.update(csr_parts("train", full))
+    parts = csr_parts("train", full)
     m = WMF(num_items=items, num_users=users, dim=dim, gamma=0.1, weighted=True, bias=False, seed=1993)
-    out["items0"] = m.items.copy()
+    items0 = m.items.copy()
     C = full.copy()
     C.data = 10 * np.log(1 + 1 * C.data)
     u1 = m.recompute_factors(m.items, C, 0.1)
     i1 = m.recompute_factors(u1, C.T.tocsr(), 0.1)
-    out["users_half1"], out["items_half1"] = u1, i1
-    np.savez_compressed(os.path.join(HERE, name + ".npz"), **out)
+    np.savez_compressed(os.path.join(HERE, name + ".npz"), users_half1=u1,
+                        train_sha256=np.str_(array_digest(parts["train_indptr"], parts["train_indices"], parts["train_data"])),
+                        items0_sha256=np.str_(array_digest(items0)))
+    rows = np.arange(0, items, 5, dtype=np.int64)
+    np.savez_compressed(os.path.join(HERE, name + "_items.npz"), items_half1_rows=rows, items_half1=i1[rows])
     print(name, u1.shape, i1.shape)
 
 

@@ -9,7 +9,7 @@ import pytest
 import scipy.sparse
 import torch
 
-from conftest import WEIGHTED_CASES, csr_from, ledger_add, load_golden, row_rel_err
+from conftest import ROOT, WEIGHTED_CASES, csr_from, ledger_add, load_golden, load_golden_2000x1500, row_rel_err
 from oracle import wmf_oracle as orc
 from recmodel_b200 import WMF, _lib, engine
 from recmodel_b200.engine import DeviceCSR
@@ -723,7 +723,7 @@ def test_half_step_dual_rows_every_length(cuda_device, f, bias):
 def test_half_step_vs_reference_golden_2000x1500(cuda_device, algo_name, algo):
     """The executed reference at 2000 x 1500, f = 128 (tests/golden/make_golden.py::case_half_steps): both tensor-core
     kernels (dual for the short rows, primal for the rest) against reference output, not only against the oracle."""
-    g = load_golden("weighted_nobias_f128_2000x1500")
+    g = load_golden_2000x1500()
     C = csr_from(g, "train")
     C.data = orc.preprocess_counts(C.data)
     CT = C.T.tocsr()
@@ -732,8 +732,8 @@ def test_half_step_vs_reference_golden_2000x1500(cuda_device, algo_name, algo):
     check_half_step("golden/2000x1500_f128/users_half1", algo_name, X[rows], g["users_half1"][rows],
                     orc.half_step(g["items0"], C[rows], 0.1, np.float64))
     Xi, _ = run_half_step(g["users_half1"], CT, False, algo, cuda_device)
-    rows = np.arange(0, 1500, 5)
-    check_half_step("golden/2000x1500_f128/items_half1", algo_name, Xi[rows], g["items_half1"][rows],
+    rows = g["items_half1_rows"]
+    check_half_step("golden/2000x1500_f128/items_half1", algo_name, Xi[rows], g["items_half1"],
                     orc.half_step(g["users_half1"], CT[rows], 0.1, np.float64), steady=True)
 
 
@@ -760,6 +760,32 @@ def test_ease_vs_reference_golden(cuda_device):
     rec = m.eval_topn(te.copy(), topn=g["topn"], rand_sampled=100, cores=1, random_state=7)
     np.testing.assert_allclose([rec[f"Recall@{k}"] for k in g["topn"]], g["recall"], atol=1e-12)
     assert m.predict(np.array([], dtype=np.int32), np.array([], dtype=np.int32)).shape == (1,)
+
+
+def test_bench_dump_outputs_reproducible(cuda_device, tmp_path):
+    """bench.py --dump-outputs: the factors of the last timed epoch, identical from run to run (the end-to-end leg
+    that follows leaves them alone), and --steps sets the number of timed steps of both legs."""
+    import json
+    import os
+    import subprocess
+    import sys
+    dumps = []
+    for k, extra in enumerate((["--steps", "3"], ["--steps", "3", "--no-e2e"])):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--workload", "ml1m",
+                              "--warmup", "1", "--no-cpu-baseline", "--dump-outputs", str(tmp_path / str(k)), *extra],
+                             capture_output=True, text=True, timeout=900, cwd=ROOT)
+        assert out.returncode == 0, out.stderr[-3000:]
+        lines = [ln for ln in out.stdout.splitlines() if ln.strip()]
+        assert len(lines) == 1, lines
+        d = json.loads(lines[0])
+        assert d["steps"] == 3 and d["value"] > 0
+        if k == 0:
+            assert len(d["e2e"]["ms_steps_rank0"]) == 3
+        dumps.append({n: np.load(tmp_path / str(k) / f"{n}.npy") for n in ("users", "items")})
+    for n, shape in (("users", (6040, 64)), ("items", (3706, 64))):
+        a, b = dumps[0][n], dumps[1][n]
+        assert a.dtype == np.float32 and a.shape == shape and np.all(np.isfinite(a)) and np.any(a != 0)
+        np.testing.assert_array_equal(a, b)
 
 
 def test_ease_larger_matrix_against_fp64(cuda_device):

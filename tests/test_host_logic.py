@@ -172,3 +172,29 @@ def test_bench_reference_arm_contract():
     assert cb["kind"] == "port" and cb["cores"] >= 1 and cb["value"] == d["value"] and cb["sample"]
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0 and d["e2e"]["value"] == d["value"]
     assert d["gpu_launches"] == 0
+
+
+def test_bench_rejects_bad_step_counts_and_reference_dumps():
+    """Argument errors end the bench before any work (exit status 2, no result line)."""
+    for extra in (["--steps", "0"], ["--warmup", "-1"], ["--impl", "reference", "--dump-outputs", "unused"]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "ml1m", *extra],
+                             capture_output=True, text=True, timeout=120, cwd=ROOT)
+        assert out.returncode == 2 and out.stdout == "", (extra, out.stderr)
+
+
+def test_bench_dump_outputs_stays_within_budget(tmp_path):
+    """bench.py --dump-outputs: an output larger than its share of the budget keeps a fixed, ascending sample of its
+    rows (the same on every call); smaller outputs are written whole."""
+    import bench
+    big = np.arange(70_000 * 128, dtype=np.float32).reshape(70_000, 128)   # 35.8 MB, over its half of the budget
+    small = np.random.default_rng(1).random((300, 128)).astype(np.float32)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"users": big, "items": small})
+    assert sorted(p.name for p in (tmp_path / "a").iterdir()) == ["items.npy", "users.npy"]
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) <= bench.DUMP_BYTES
+    u = np.load(tmp_path / "a" / "users.npy")
+    assert u.dtype == np.float32 and u.shape[1] == 128 and 60_000 < u.shape[0] < 70_000
+    assert np.all(np.diff(u[:, 0]) > 0)   # distinct rows in ascending order
+    np.testing.assert_array_equal(u, big[(u[:, 0] / 128).astype(np.int64)])
+    np.testing.assert_array_equal(u, np.load(tmp_path / "b" / "users.npy"))
+    np.testing.assert_array_equal(np.load(tmp_path / "a" / "items.npy"), small)

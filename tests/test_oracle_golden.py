@@ -3,7 +3,7 @@ reference (tests/golden/make_golden.py). CPU only."""
 import numpy as np
 import pytest
 
-from conftest import WEIGHTED_CASES, csr_from, load_golden, row_rel_err
+from conftest import WEIGHTED_CASES, csr_from, load_golden, load_golden_2000x1500, row_rel_err
 from oracle import wmf_oracle as orc
 
 HALF_STEP_TOL = 1e-4  # BASELINE.json north_star: 1e-4 relative per half-step
@@ -165,26 +165,23 @@ def test_algorithmic_bytes_match_survey():
     assert abs(b / 1e9 - 20.97) < 0.02
 
 
-def test_live_reference_if_mounted():
-    """When /root/reference is present (build container) re-run one half-step through it."""
-    from oracle import ref_shim
-    if not ref_shim.available():
-        pytest.skip("reference not mounted (expected on the GPU box)")
-    WMF = ref_shim.load_reference_wmf()
+def test_reference_constructor_and_half_step_golden():
+    """The reference's WMF constructed with its default seed, and its recompute_factors from there, as stored by
+    tests/golden/make_golden.py: this package's WMF starts from the same factors, and the oracle's half-step
+    reproduces the reference's to BLAS rounding."""
+    from recmodel_b200 import WMF
     g = load_golden("weighted_nobias_f16")
     _, _, C, _ = _prep(g, "log")
     m = WMF(num_items=C.shape[1], num_users=C.shape[0], dim=16, gamma=0.1, weighted=True)
     np.testing.assert_array_equal(m.items, g["items0"])
-    ref = m.recompute_factors(m.items, C, 0.1)
-    np.testing.assert_array_equal(ref, g["users_half1"])
-    assert row_rel_err(orc.half_step(g["items0"], C, 0.1), ref) < 1e-5
+    assert row_rel_err(orc.half_step(m.items, C, 0.1), g["users_half1"]) < 1e-5
 
 
 # ------------------------------------------------------------------------------- larger f = 128 fixture, EASE (N4)
 def test_large_f128_half_steps_fp32_and_fp64():
     """2000 x 1500 fixture of the executed reference (tests/golden/make_golden.py::case_half_steps): the oracle's
     fp32 arithmetic reproduces it to BLAS rounding, the fp64 restatement within the first-half-step noise."""
-    g = load_golden("weighted_nobias_f128_2000x1500")
+    g = load_golden_2000x1500()
     C = csr_from(g, "train")
     C.data = orc.preprocess_counts(C.data)
     rows = slice(0, 300)
