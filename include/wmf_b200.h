@@ -186,6 +186,19 @@ size_t wmf_score_topk_workspace_bytes(int64_t nu, int64_t ni, int topn);
 int wmf_score_topk(const int64_t* users, int64_t nu, const int64_t* cand, int64_t ni, const float* U,
                    int64_t ldu, const float* V, int64_t ldv, int f, int bias, int topn, int64_t* out_ids,
                    float* out_scores, void* ws, size_t ws_bytes, void* stream);
+/* K4+K5 with exclusion: top-N over all items 0..ni-1 minus the items each user has interacted with: replaces the
+ * rank(np.delete(all_items, seen)) loop of test_coverage (RecModel/utils.py:3-18).
+ * ex_indptr int64[rows+1] / ex_indices int32 are a CSR matrix whose row `user` lists the item ids to leave out for
+ * that user (rows indexed by user id, ids in [0, ni) sorted ascending within each row, duplicates allowed; values
+ * are not read). Same scores, order and tie rule as wmf_score_topk over the remaining items; a user with fewer than
+ * topn of them gets id -1 (score NaN) in the rest of its row. The tensor-core path masks the excluded ids in both
+ * GEMM passes; a user whose candidate list overflows makes the exact kernels redo the call, and fixup_users
+ * (nullable, device int32) receives the number of such users (0: the tensor-core path alone answered). */
+size_t wmf_score_topk_exclude_workspace_bytes(int64_t nu, int64_t ni, int topn);
+int wmf_score_topk_exclude(const int64_t* users, int64_t nu, const int64_t* ex_indptr, const int32_t* ex_indices,
+                           int64_t ni, const float* U, int64_t ldu, const float* V, int64_t ldv, int f, int bias,
+                           int topn, int64_t* out_ids, float* out_scores, int32_t* fixup_users, void* ws,
+                           size_t ws_bytes, void* stream);
 
 /* K7. Unweighted half-step X = R * (Ginv * Y^T)^T:       replaces wmf_model.py:85,:88.
  * wmf_inverse: Ginv = inv(G) for a small dense f x f matrix (np.linalg.inv), one CTA.

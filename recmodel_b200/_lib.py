@@ -47,6 +47,9 @@ SIGNATURES = {
     "wmf_predict_pairs": (_i32, [_p, _i64, _p, _i64, _p, _i64, _p, _i64, _i32, _i32, _p, _p]),
     "wmf_score_topk_workspace_bytes": (_sz, [_i64, _i64, _i32]),
     "wmf_score_topk": (_i32, [_p, _i64, _p, _i64, _p, _i64, _p, _i64, _i32, _i32, _i32, _p, _p, _p, _sz, _p]),
+    "wmf_score_topk_exclude_workspace_bytes": (_sz, [_i64, _i64, _i32]),
+    "wmf_score_topk_exclude": (_i32, [_p, _i64, _p, _p, _i64, _p, _i64, _p, _i64, _i32, _i32, _i32, _p, _p, _p, _p, _sz,
+                                      _p]),
     "wmf_inverse_workspace_bytes": (_sz, [_i32]),
     "wmf_inverse": (_i32, [_p, _i32, _p, _p, _sz, _p]),
     "wmf_dense_right_multiply": (_i32, [_p, _i64, _i64, _p, _i32, _p, _i64, _p]),

@@ -145,16 +145,34 @@ __global__ __launch_bounds__(SC_THREADS) void score_tile_kernel(const int64_t* _
     }
 }
 
+// Excluded items of the users of a score tile: their scores become the bit pattern 0xFFFFFFFF, which order_key maps
+// to 0, below every other score. One CTA per user row (grid-stride).
+constexpr uint32_t EXCLUDED_BITS = 0xFFFFFFFFu;
+
+__global__ __launch_bounds__(256) void score_exclude_kernel(const int64_t* __restrict__ users, int64_t u_begin, int ub,
+                                                            const int64_t* __restrict__ ex_indptr,
+                                                            const int32_t* __restrict__ ex_indices, int64_t ni,
+                                                            float* __restrict__ S, const int* __restrict__ run_if) {
+    if (run_if != nullptr && *run_if == 0) return;
+    for (int r = blockIdx.x; r < ub; r += gridDim.x) {
+        const int64_t user = users[u_begin + r];
+        const int64_t lo = ex_indptr[user], hi = ex_indptr[user + 1];
+        for (int64_t e = lo + threadIdx.x; e < hi; e += blockDim.x)
+            S[(size_t)r * ni + ex_indices[e]] = __uint_as_float(EXCLUDED_BITS);
+    }
+}
+
 constexpr int TK_THREADS = 256;
 constexpr int TK_MAX = 1024;  // largest topn this kernel sorts in shared memory
 
 // One CTA per user row of S: k-th largest key by 4x8-bit radix select, gather winners
-// (ties at the threshold taken in candidate order), bitonic sort descending.
+// (ties at the threshold taken in candidate order), bitonic sort descending. `excl`: winners with key 0 are
+// excluded items (score_exclude_kernel) a user with fewer than topn others is left with: id -1, score NaN.
 __global__ __launch_bounds__(TK_THREADS) void topk_rows_kernel(const float* __restrict__ S, int64_t ni, int topn,
                                                                const int64_t* __restrict__ cand,
                                                                int64_t* __restrict__ out_ids,
                                                                float* __restrict__ out_scores,
-                                                               const int* __restrict__ run_if) {
+                                                               const int* __restrict__ run_if, int excl) {
     __shared__ unsigned hist[256];
     if (run_if != nullptr && *run_if == 0) return;
     __shared__ unsigned long long keys[TK_MAX];
@@ -243,7 +261,8 @@ __global__ __launch_bounds__(TK_THREADS) void topk_rows_kernel(const float* __re
     for (int t = tid; t < topn; t += TK_THREADS) {
         const unsigned long long k = keys[t];
         const uint32_t pos = 0xFFFFFFFFu - (uint32_t)(k & 0xFFFFFFFFull);
-        out_ids[(size_t)blockIdx.x * topn + t] = cand ? cand[pos] : (int64_t)pos;
+        const bool none = excl && (k >> 32) == 0ull;
+        out_ids[(size_t)blockIdx.x * topn + t] = none ? -1 : (cand ? cand[pos] : (int64_t)pos);
         if (out_scores) out_scores[(size_t)blockIdx.x * topn + t] = row[pos];
     }
 }
@@ -272,24 +291,33 @@ size_t wmf_score_topk_workspace_bytes(int64_t nu, int64_t ni, int topn) {
     return exact > tc ? exact : tc;
 }
 
-int wmf_score_topk(const int64_t* users, int64_t nu, const int64_t* cand, int64_t ni, const float* U, int64_t ldu,
-                   const float* V, int64_t ldv, int f, int bias, int topn, int64_t* out_ids, float* out_scores,
-                   void* ws, size_t ws_bytes, void* stream) {
-    WMF_REQUIRE(f > 0 && f <= WMF_MAX_F && (!bias || f >= 2), "wmf_score_topk: f=%d out of range", f);
-    WMF_REQUIRE(nu >= 0 && ni >= 0, "wmf_score_topk: negative size");
+size_t wmf_score_topk_exclude_workspace_bytes(int64_t nu, int64_t ni, int topn) {
+    return wmf_score_topk_workspace_bytes(nu, ni, topn);
+}
+
+}  // extern "C"
+
+// wmf_score_topk, and wmf_score_topk_exclude when ex_indptr is not null
+static int score_topk(const char* name, const int64_t* users, int64_t nu, const int64_t* cand,
+                      const int64_t* ex_indptr, const int32_t* ex_indices, int64_t ni, const float* U, int64_t ldu,
+                      const float* V, int64_t ldv, int f, int bias, int topn, int64_t* out_ids, float* out_scores,
+                      int32_t* fixup_users, void* ws, size_t ws_bytes, void* stream) {
+    WMF_REQUIRE(f > 0 && f <= WMF_MAX_F && (!bias || f >= 2), "%s: f=%d out of range", name, f);
+    WMF_REQUIRE(nu >= 0 && ni >= 0, "%s: negative size", name);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (fixup_users) WMF_CUDA(cudaMemsetAsync(fixup_users, 0, sizeof(int32_t), st));
     if (nu == 0 || topn == 0) return WMF_OK;
-    WMF_REQUIRE(users && U && V && out_ids, "wmf_score_topk: null argument");
-    WMF_REQUIRE(ni < (1ll << 32), "wmf_score_topk: more than 2^32 candidates");
+    WMF_REQUIRE(users && U && V && out_ids, "%s: null argument", name);
+    WMF_REQUIRE(ni < (1ll << 32), "%s: more than 2^32 candidates", name);
     if (topn < 0 || topn > ni || topn > TK_MAX) {
-        set_error("wmf_score_topk: topn=%d outside 1..min(ni=%lld, %d)", topn, (long long)ni, TK_MAX);
+        set_error("%s: topn=%d outside 1..min(ni=%lld, %d)", name, topn, (long long)ni, TK_MAX);
         return WMF_ERR_UNSUPPORTED;
     }
     size_t need = wmf_score_topk_workspace_bytes(nu, ni, topn);
     if (ws == nullptr || ws_bytes < need) {
-        set_error("wmf_score_topk: workspace %zu < %zu", ws_bytes, need);
+        set_error("%s: workspace %zu < %zu", name, ws_bytes, need);
         return WMF_ERR_WORKSPACE;
     }
-    cudaStream_t st = (cudaStream_t)stream;
     const int FS = f + 1;
     const size_t smem = (size_t)(SC_THREADS + SC_USERS) * FS * sizeof(float);
     WMF_CUDA(cudaFuncSetAttribute(score_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -306,7 +334,7 @@ int wmf_score_topk(const int64_t* users, int64_t nu, const int64_t* cand, int64_
         for (int64_t u0 = 0; u0 < nu; u0 += tb) {
             const int ub = (int)((nu - u0) < tb ? (nu - u0) : tb);
             int rc = score_topk_tc_batch(users, u0, ub, tb, cand, ni, U, ldu, V, ldv, f, bias, topn, out_ids, out_scores,
-                                         (char*)ws + exact_bytes, u0 == 0, &redo, st);
+                                         (char*)ws + exact_bytes, u0 == 0, &redo, st, ex_indptr, ex_indices, fixup_users);
             if (rc) return rc;
         }
     }
@@ -325,11 +353,35 @@ int wmf_score_topk(const int64_t* users, int64_t nu, const int64_t* cand, int64_
         const unsigned grid = (unsigned)(tiles < cap ? tiles : cap);
         score_tile_kernel<<<grid, SC_THREADS, smem, st>>>(users, u0, ub, cand, ni, U, ldu, V, ldv, f, bias, S, redo);
         WMF_LAUNCH_CHECK("score_tile_kernel");
+        if (ex_indptr) {
+            score_exclude_kernel<<<(unsigned)(ub < 65535 ? ub : 65535), 256, 0, st>>>(users, u0, ub, ex_indptr, ex_indices,
+                                                                                      ni, S, redo);
+            WMF_LAUNCH_CHECK("score_exclude_kernel");
+        }
         topk_rows_kernel<<<ub, TK_THREADS, 0, st>>>(S, ni, topn, cand, out_ids + (size_t)u0 * topn,
-                                                    out_scores ? out_scores + (size_t)u0 * topn : nullptr, redo);
+                                                    out_scores ? out_scores + (size_t)u0 * topn : nullptr, redo,
+                                                    ex_indptr != nullptr);
         WMF_LAUNCH_CHECK("topk_rows_kernel");
     }
     return WMF_OK;
+}
+
+extern "C" {
+
+int wmf_score_topk(const int64_t* users, int64_t nu, const int64_t* cand, int64_t ni, const float* U, int64_t ldu,
+                   const float* V, int64_t ldv, int f, int bias, int topn, int64_t* out_ids, float* out_scores,
+                   void* ws, size_t ws_bytes, void* stream) {
+    return score_topk("wmf_score_topk", users, nu, cand, nullptr, nullptr, ni, U, ldu, V, ldv, f, bias, topn, out_ids,
+                      out_scores, nullptr, ws, ws_bytes, stream);
+}
+
+int wmf_score_topk_exclude(const int64_t* users, int64_t nu, const int64_t* ex_indptr, const int32_t* ex_indices,
+                           int64_t ni, const float* U, int64_t ldu, const float* V, int64_t ldv, int f, int bias,
+                           int topn, int64_t* out_ids, float* out_scores, int32_t* fixup_users, void* ws,
+                           size_t ws_bytes, void* stream) {
+    WMF_REQUIRE(ex_indptr, "wmf_score_topk_exclude: null exclusion matrix");  // ex_indices may be null when it is empty
+    return score_topk("wmf_score_topk_exclude", users, nu, nullptr, ex_indptr, ex_indices, ni, U, ldu, V, ldv, f, bias,
+                      topn, out_ids, out_scores, fixup_users, ws, ws_bytes, stream);
 }
 
 }  // extern "C"

@@ -17,6 +17,6 @@ void score_tc_fixup_region(int64_t nu, int64_t ni, size_t* offset, size_t* bytes
 int score_topk_tc_batch(const int64_t* users, int64_t u0, int ub, int64_t ubatch, const int64_t* cand, int64_t ni,
                         const float* U, int64_t ldu, const float* V, int64_t ldv, int f, int bias, int topn,
                         int64_t* out_ids, float* out_scores, void* ws, bool first_batch, int** overflow_flag,
-                        cudaStream_t st);
+                        cudaStream_t st, const int64_t* ex_indptr, const int32_t* ex_indices, int* fixup_users);
 
 }  // namespace wmf

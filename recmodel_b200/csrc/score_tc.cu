@@ -20,6 +20,14 @@
 //       NumPy order and the final top-N is selected from them, ties by candidate position: the same index
 //       set and order as the exact path. If a user collects more than 1024 candidates (e.g. all scores
 //       equal) a flag makes the caller redo the call with the exact CUDA-core kernels.
+//   Exclusion (wmf_score_topk_exclude, EXCL = true): every epilogue thread walks its user's sorted list of
+//       excluded item ids with one cursor, in step with the ascending 32-column blocks, and turns the ids that
+//       fall into the block into a 32-bit mask. Pass 1 leaves masked columns out of the block maximum (a block
+//       with nothing left gives -3e38), so tau' is still reached by N distinct items that may be returned and
+//       the bound above holds for the top-N over the unseen items; pass 2 drops masked columns from the hits.
+//       A user with fewer than N unseen items has -3e38 as its N-th block maximum: the threshold admits every
+//       unseen item, the list is complete, and the rescoring pads it with id -1 instead of raising the flag.
+#include <climits>
 #include <cuda_fp16.h>
 #include "common.cuh"
 #include "score.cuh"
@@ -181,12 +189,14 @@ __global__ void stc_maxnorm_kernel(const float* __restrict__ norms, int64_t n, u
 // ---------------------------------------------------------------------------------------------------
 // K4: S~ = U~ V~^T tile by tile, one CTA per 128 users, item tiles streamed by bulk copies.
 // MODE 0: per user maxima of every 32-column block.  MODE 1: append the items with S~ >= thr[user].
+// EXCL: the item ids ex_indices[ex_indptr[user] ..) (ascending) of user = users[u_begin + row] take no part.
 // ---------------------------------------------------------------------------------------------------
-template <int MODE>
+template <int MODE, bool EXCL>
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
 stc_gemm_kernel(const uint8_t* __restrict__ a_tiles, const uint8_t* __restrict__ b_tiles, int n_item_tiles, int ub,
                 int64_t ni, float* __restrict__ maxima, const float* __restrict__ thr, int* __restrict__ cnt,
-                uint32_t* __restrict__ lists) {
+                uint32_t* __restrict__ lists, const int64_t* __restrict__ users, int64_t u_begin,
+                const int64_t* __restrict__ ex_indptr, const int32_t* __restrict__ ex_indices) {
     extern __shared__ uint8_t smem_raw[];
     const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
     const uint32_t bars = base + OFF_BARS;
@@ -254,6 +264,17 @@ stc_gemm_kernel(const uint8_t* __restrict__ a_tiles, const uint8_t* __restrict__
         float my_thr = 0.0f;
         int my_cnt = 0;  // this thread is the only writer of its user's candidate list: no atomics
         if (MODE == 1 && live) my_thr = thr[u];
+        // cursor into the user's excluded ids: ex_next = ex_indices[ex], ex_after the one behind it (INT_MAX: none),
+        // loaded one step ahead so that the walk rarely waits for a load
+        int64_t ex = 0, ex_end = 0;
+        int ex_next = INT_MAX, ex_after = INT_MAX;
+        if (EXCL && live) {
+            const int64_t user = users[u_begin + u];
+            ex = ex_indptr[user];
+            ex_end = ex_indptr[user + 1];
+            if (ex < ex_end) ex_next = ex_indices[ex];
+            if (ex + 1 < ex_end) ex_after = ex_indices[ex + 1];
+        }
         for (int it = 0; it < n_item_tiles; ++it) {
             const int acc = it & 1;
             mbar_wait(bar_accfull(acc), (it >> 1) & 1u);
@@ -264,9 +285,24 @@ stc_gemm_kernel(const uint8_t* __restrict__ a_tiles, const uint8_t* __restrict__
                 uint32_t r[32];
                 tmem_ld32(t_row + c * SUB, r);
                 const int64_t col0 = (int64_t)it * TN + c * SUB;
+                uint32_t xmask = 0;  // excluded columns of this block (duplicate ids set the same bit again)
+                if (EXCL) {
+                    const int c0 = (int)col0;  // ids are int32
+                    while (ex_next < c0 + SUB) {
+                        xmask |= 1u << (uint32_t)(ex_next - c0);
+                        ex_next = ex_after;
+                        ++ex;
+                        ex_after = ex + 1 < ex_end ? ex_indices[ex + 1] : INT_MAX;
+                    }
+                }
                 if (MODE == 0) {
                     float m = -3.0e38f;
-                    if (col0 + SUB <= ni) {
+                    if (EXCL) {  // branch-free: nearly every block has an excluded column in some lane of the warp
+                        uint32_t keep = ~xmask;
+                        if (col0 + SUB > ni) keep &= (col0 < ni) ? (0xFFFFFFFFu >> (32 - (int)(ni - col0))) : 0u;
+#pragma unroll
+                        for (int j = 0; j < SUB; ++j) m = fmaxf(m, ((keep >> j) & 1u) ? __uint_as_float(r[j]) : -3.0e38f);
+                    } else if (col0 + SUB <= ni) {
 #pragma unroll
                         for (int j = 0; j < SUB; ++j) m = fmaxf(m, __uint_as_float(r[j]));
                     } else {
@@ -280,6 +316,7 @@ stc_gemm_kernel(const uint8_t* __restrict__ a_tiles, const uint8_t* __restrict__
 #pragma unroll
                     for (int j = 0; j < SUB; ++j) hits |= (__uint_as_float(r[j]) >= my_thr ? 1u : 0u) << j;
                     if (col0 + SUB > ni) hits &= (col0 < ni) ? (0xFFFFFFFFu >> (32 - (int)(ni - col0))) : 0u;  // padding items
+                    if (EXCL) hits &= ~xmask;
                     while (hits) {
                         const int j = __ffs(hits) - 1;
                         hits &= hits - 1;
@@ -351,17 +388,26 @@ __global__ __launch_bounds__(128) void stc_threshold_kernel(const float* __restr
 // ---------------------------------------------------------------------------------------------------
 constexpr int TK_THREADS = 256;
 
+// EXCL: a list shorter than topn is complete when the threshold is the -3e38 sentinel (fewer than topn unseen
+// items: pass 2 admitted all of them); the rest of the row is id -1, score NaN. `fixup_users` (nullable) counts
+// the users that make the exact path redo the call.
+template <bool EXCL>
 __global__ __launch_bounds__(TK_THREADS) void stc_rescore_kernel(
     const int* __restrict__ cnt, const uint32_t* __restrict__ lists, int topn, const int64_t* __restrict__ users,
     int64_t u_begin, const int64_t* __restrict__ cand, const float* __restrict__ U, int64_t ldu,
     const float* __restrict__ V, int64_t ldv, int f, int bias, int64_t* __restrict__ out_ids,
-    float* __restrict__ out_scores, int* __restrict__ overflow) {
+    float* __restrict__ out_scores, int* __restrict__ overflow, const float* __restrict__ thr,
+    int* __restrict__ fixup_users) {
     __shared__ unsigned long long keys[CAND_MAX];
     __shared__ float su[K + 1];
     const int tid = threadIdx.x, lane = tid & 31;
     const int n_cand = cnt[blockIdx.x];
-    if (n_cand > CAND_MAX || n_cand < topn) {  // too many near-ties for the candidate buffer: the exact path redoes the call
-        if (tid == 0) atomicOr(overflow, 1);
+    const bool short_ok = EXCL && thr[blockIdx.x] <= -3.0e38f;
+    if (n_cand > CAND_MAX || (n_cand < topn && !short_ok)) {  // too many near-ties for the candidate buffer: the exact path redoes the call
+        if (tid == 0) {
+            atomicOr(overflow, 1);
+            if (EXCL && fixup_users) atomicAdd(fixup_users, 1);
+        }
         return;
     }
     const uint32_t* cpos = lists + (size_t)blockIdx.x * CAND_MAX;
@@ -413,6 +459,11 @@ __global__ __launch_bounds__(TK_THREADS) void stc_rescore_kernel(
         }
     }
     for (int t = tid; t < topn; t += TK_THREADS) {
+        if (EXCL && t >= n_cand) {
+            out_ids[(size_t)blockIdx.x * topn + t] = -1;
+            if (out_scores) out_scores[(size_t)blockIdx.x * topn + t] = __uint_as_float(0x7FFFFFFFu);
+            continue;
+        }
         const unsigned long long k = keys[t];
         const uint32_t pos = 0xFFFFFFFFu - (uint32_t)(k & 0xFFFFFFFFull);
         out_ids[(size_t)blockIdx.x * topn + t] = cand ? cand[pos] : (int64_t)pos;
@@ -475,7 +526,7 @@ void score_tc_fixup_region(int64_t nu, int64_t ni, size_t* offset, size_t* bytes
 int score_topk_tc_batch(const int64_t* users, int64_t u0, int ub, int64_t ubatch, const int64_t* cand, int64_t ni,
                         const float* U, int64_t ldu, const float* V, int64_t ldv, int f, int bias, int topn,
                         int64_t* out_ids, float* out_scores, void* ws, bool first_batch, int** overflow_flag,
-                        cudaStream_t st) {
+                        cudaStream_t st, const int64_t* ex_indptr, const int32_t* ex_indices, int* fixup_users) {
     char* tc = reinterpret_cast<char*>(ws);
     const TcLayout l = tc_layout(ubatch, ni);
     uint32_t* hdr = reinterpret_cast<uint32_t*>(tc + l.off_hdr);  // [0] overflow, [1] absmax U, [2] absmax V, [3] max ||v~||
@@ -490,8 +541,10 @@ int score_topk_tc_batch(const int64_t* users, int64_t u0, int ub, int64_t ubatch
     *overflow_flag = reinterpret_cast<int*>(hdr);
     static bool attr_set = false;
     if (!attr_set) {
-        WMF_CUDA(cudaFuncSetAttribute(stc_gemm_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-        WMF_CUDA(cudaFuncSetAttribute(stc_gemm_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+        WMF_CUDA(cudaFuncSetAttribute(stc_gemm_kernel<0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+        WMF_CUDA(cudaFuncSetAttribute(stc_gemm_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+        WMF_CUDA(cudaFuncSetAttribute(stc_gemm_kernel<0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+        WMF_CUDA(cudaFuncSetAttribute(stc_gemm_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
         attr_set = true;
     }
     const int sms = sm_count();
@@ -514,17 +567,21 @@ int score_topk_tc_batch(const int64_t* users, int64_t u0, int ub, int64_t ubatch
                                                                                hdr + 1, a_tiles, unorm);
     WMF_LAUNCH_CHECK("stc_convert_kernel(users)");
     const unsigned grid = (unsigned)(ub_pad / 128);
-    stc_gemm_kernel<0><<<grid, GEMM_THREADS, SMEM_BYTES, st>>>(a_tiles, b_tiles, n_tiles, ub, ni, maxima, nullptr, nullptr,
-                                                               nullptr);
+    const bool excl = ex_indptr != nullptr;
+    auto gemm0 = excl ? stc_gemm_kernel<0, true> : stc_gemm_kernel<0, false>;
+    auto gemm1 = excl ? stc_gemm_kernel<1, true> : stc_gemm_kernel<1, false>;
+    gemm0<<<grid, GEMM_THREADS, SMEM_BYTES, st>>>(a_tiles, b_tiles, n_tiles, ub, ni, maxima, nullptr, nullptr, nullptr,
+                                                  users, u0, ex_indptr, ex_indices);
     WMF_LAUNCH_CHECK("stc_gemm_kernel<maxima>");
     stc_threshold_kernel<<<ub, 128, (size_t)n_sub * 4, st>>>(maxima, n_sub, topn, unorm, hdr + 3, thr, cnt);
     WMF_LAUNCH_CHECK("stc_threshold_kernel");
-    stc_gemm_kernel<1><<<grid, GEMM_THREADS, SMEM_BYTES, st>>>(a_tiles, b_tiles, n_tiles, ub, ni, nullptr, thr, cnt, lists);
+    gemm1<<<grid, GEMM_THREADS, SMEM_BYTES, st>>>(a_tiles, b_tiles, n_tiles, ub, ni, nullptr, thr, cnt, lists, users, u0,
+                                                  ex_indptr, ex_indices);
     WMF_LAUNCH_CHECK("stc_gemm_kernel<filter>");
-    stc_rescore_kernel<<<ub, TK_THREADS, 0, st>>>(cnt, lists, topn, users, u0, cand, U, ldu, V, ldv, f, bias,
-                                                  out_ids + (size_t)u0 * topn,
-                                                  out_scores ? out_scores + (size_t)u0 * topn : nullptr,
-                                                  reinterpret_cast<int*>(hdr));
+    auto rescore = excl ? stc_rescore_kernel<true> : stc_rescore_kernel<false>;
+    rescore<<<ub, TK_THREADS, 0, st>>>(cnt, lists, topn, users, u0, cand, U, ldu, V, ldv, f, bias,
+                                       out_ids + (size_t)u0 * topn, out_scores ? out_scores + (size_t)u0 * topn : nullptr,
+                                       reinterpret_cast<int*>(hdr), thr, fixup_users);
     WMF_LAUNCH_CHECK("stc_rescore_kernel");
     return WMF_OK;
 }

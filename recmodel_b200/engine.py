@@ -142,6 +142,7 @@ class DeviceCSR:
         self.nnz = int(indices.numel())
         self._row_order = None
         self._split_segments = None
+        self._sorted = None
 
     @classmethod
     def from_scipy(cls, mat, device=None):
@@ -204,11 +205,19 @@ class DeviceCSR:
             _lib.check(lib.wmf_csr_transpose(_ptr(self.indptr), _ptr(self.indices), _ptr(self.data), rows, cols, self.nnz,
                                              _ptr(out_indptr), _ptr(out_indices), _ptr(out_data), _ptr(ws), ws.numel(),
                                              _stream(dev)), "wmf_csr_transpose")
-        return DeviceCSR(out_indptr, out_indices, out_data, (cols, rows))
+        out = DeviceCSR(out_indptr, out_indices, out_data, (cols, rows))
+        out._sorted = out
+        return out
 
     def canonical(self):
         """The same matrix with sorted column indices inside every row (two transposes)."""
         return self.transpose().transpose()
+
+    def sorted(self):
+        """``canonical()``, computed once: ``self`` when its rows are known to be sorted (a transpose's are)."""
+        if self._sorted is None:
+            self._sorted = self.canonical()
+        return self._sorted
 
     def row_slice(self, r0, r1):
         """Rows [r0, r1) as an independent DeviceCSR (used to shard rows across GPUs)."""
@@ -514,6 +523,28 @@ def score_topk(users, cand, U, V, topn, bias=False, want_scores=False):
                                   U.shape[1], int(bool(bias)), int(topn), _ptr(ids), _ptr(scores), _ptr(ws), ws.numel(),
                                   _stream()), "wmf_score_topk")
     return (ids, scores) if want_scores else ids
+
+
+@_device_of(2)
+def score_topk_exclude(users, exclude, U, V, topn, bias=False, want_scores=False):
+    """Top-``topn`` item ids [nu x topn] (int64) over all items minus the stored entries of row ``users[k]`` of
+    ``exclude`` (a DeviceCSR with sorted rows, indexed by user id), -1 where a user has fewer unseen items
+    (include/wmf_b200.h: wmf_score_topk_exclude). Returns (ids, scores or None, fixup_users): the last is a device
+    int32 [1], the number of users whose candidate list made the exact kernels redo the call."""
+    lib = _lib.load()
+    _f32(U)
+    _f32(V)
+    nu, ni = users.numel(), V.shape[0]
+    assert exclude.shape[1] == ni and exclude.indices.dtype == torch.int32 and exclude.indptr.dtype == torch.int64
+    ids = torch.empty((nu, topn), dtype=torch.int64, device=U.device)
+    scores = torch.empty((nu, topn), dtype=torch.float32, device=U.device) if want_scores else None
+    fixup = torch.zeros(1, dtype=torch.int32, device=U.device)
+    ws = workspace(lib.wmf_score_topk_exclude_workspace_bytes(nu, ni, topn), U.device)
+    _lib.check(lib.wmf_score_topk_exclude(_ptr(users), nu, _ptr(exclude.indptr), _ptr(exclude.indices), ni, _ptr(U),
+                                          U.stride(0), _ptr(V), V.stride(0), U.shape[1], int(bool(bias)), int(topn),
+                                          _ptr(ids), _ptr(scores), _ptr(fixup), _ptr(ws), ws.numel(), _stream()),
+               "wmf_score_topk_exclude")
+    return ids, scores, fixup
 
 
 @_device_of(1)

@@ -3,11 +3,11 @@
 
 * ``train_test_split_sparse_mat`` (utils.py:20-37): the 80/20 split with the reference's RNG semantics.
 * ``test_coverage`` (utils.py:3-18): how often each item appears in the users' top-N over the items they
-  have not interacted with; the ranking runs on the device in batches instead of one ``rank`` call per user.
+  have not interacted with; the ranking runs on the device in one ``recommend`` call instead of one ``rank``
+  call per user.
 """
 import numpy as np
 
-from . import _lib
 from .synthetic import split_train_test
 
 
@@ -22,39 +22,22 @@ def train_test_split_sparse_mat(matrix, train=0.8, seed=1993):
 def test_coverage(cls, Train, topN):
     """``item_counts[i]`` = number of users whose top-``topN`` over their unseen items contains item i
     (utils.py:3-18). Like the reference the result has ``Train.shape[0]`` entries (it sizes the array by the
-    row count, utils.py:7). ``cls`` is any model with the RecModel ``rank``; models with ``rank_batch`` (WMF)
-    rank all items for a batch of users in one device pass and the seen items are dropped afterwards, which
-    leaves the relative order of the unseen ones unchanged (ties are ordered by item id either way)."""
+    row count, utils.py:7). ``cls`` is any model with the RecModel ``rank``; models with ``recommend`` (WMF)
+    rank every user's unseen items on the device in one call, with the stored entries of ``Train`` excluded
+    there (ties are ordered by item id, as ``rank`` orders them over the ascending candidate list)."""
     Train = Train.tocsr()
     n_users, n_items = Train.shape
     item_counts = np.zeros(n_users, dtype=np.int32)
-    seen_n = np.diff(Train.indptr)
+    if hasattr(cls, "recommend"):
+        ranked = cls.recommend(np.arange(n_users), topN, exclude=Train)
+        np.add.at(item_counts, ranked[ranked >= 0], 1)  # each row holds distinct ids: one count per (user, item)
+        return item_counts
     all_items = np.arange(n_items, dtype=np.int32)
-
-    def one_user(user):  # the reference's loop body
+    for user in range(n_users):  # the reference's loop
         lo, hi = Train.indptr[user], Train.indptr[user + 1]
         items_to_rank = np.delete(all_items, Train.indices[lo:hi])
         ranked = np.asarray(cls.rank(users=user, items=items_to_rank, topn=topN)).reshape(-1)
         item_counts[ranked[:topN]] += 1
-
-    if not hasattr(cls, "rank_batch"):
-        for user in range(n_users):
-            one_user(user)
-        return item_counts
-    order = np.argsort(seen_n, kind="stable")  # users with few seen items first: the batches need a short list
-    batch = 4096
-    for b0 in range(0, n_users, batch):
-        users = order[b0:b0 + batch]
-        k = int(topN + seen_n[users].max())
-        if k > min(_lib.TOPK_MAX, n_items):
-            for user in users:  # very active users: their own candidate list, as the reference does
-                one_user(int(user))
-            continue
-        ranked = cls.rank_batch(all_items, users.astype(np.int64), k)       # [len(users) x k], best first
-        for row, user in zip(ranked, users):
-            lo, hi = Train.indptr[user], Train.indptr[user + 1]
-            keep = row[~np.isin(row, Train.indices[lo:hi])][:topN]
-            item_counts[keep] += 1
     return item_counts
 
 

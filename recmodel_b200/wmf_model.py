@@ -170,6 +170,67 @@ class WMF(RecModel):
             ids = torch.cat(rows) if rows else torch.empty((0, k), dtype=torch.int64, device=self.device)
         return ids.cpu().numpy().astype(items.dtype, copy=False)
 
+    def recommend(self, users, topn, exclude=None, distributed=False):
+        """int64 [len(users) x topn]: the top-``topn`` of all items for each user, best first, leaving out the stored
+        entries of row ``users[k]`` of ``exclude`` (users x items, any SciPy format or a DeviceCSR; every stored entry
+        excludes its item whatever its value). Row k is ``rank(np.delete(np.arange(num_items), seen), users[k],
+        topn)`` followed by -1 where the user has fewer than ``topn`` unseen items; ties go to the lower item id.
+        ``exclude=None`` is ``rank_batch(np.arange(num_items), users, topn)``. ``distributed=True`` is a collective
+        like in ``rank_batch``: each rank scores an equal slice of the users and the id lists are all-gathered."""
+        V = self.items_device
+        ni = V.shape[0]
+        if exclude is None:
+            return self.rank_batch(np.arange(ni, dtype=np.int64), users, topn, distributed=distributed)
+        users = np.ascontiguousarray(users, dtype=np.int64).reshape(-1)
+        if exclude.shape[1] != ni:
+            raise ValueError(f"exclude has {exclude.shape[1]} columns but the model has {ni} items")
+        if len(users) and (users.min() < 0 or users.max() >= exclude.shape[0]):
+            raise ValueError(f"user ids must lie in [0, {exclude.shape[0]}) (the rows of exclude)")
+        topn = int(topn)
+        k = min(topn, ni)
+        out = np.full((len(users), topn), -1, dtype=np.int64)
+        if k <= 0 or len(users) == 0:
+            return out
+        ex = exclude if isinstance(exclude, DeviceCSR) else DeviceCSR.from_scipy(exclude, self.device)
+        ex = ex.sorted()
+        users_d = torch.from_numpy(users).to(self.device)
+        U, bias = self.users_device, self.bias is True
+        rank_id, world = sharding.dist_info()
+        if distributed and world > 1 and k <= _lib.TOPK_MAX:
+            per = -(-len(users) // world)
+            mine = users_d[rank_id * per:(rank_id + 1) * per]
+            local = torch.full((per, k), -1, dtype=torch.int64, device=self.device)
+            if mine.numel():
+                local[:mine.numel()] = engine.score_topk_exclude(mine, ex, U, V, k, bias=bias)[0]
+            ids = torch.empty((world * per, k), dtype=torch.int64, device=self.device)
+            torch.distributed.all_gather_into_tensor(ids, local)
+            ids = ids[:len(users)]
+        elif k <= _lib.TOPK_MAX:
+            ids = engine.score_topk_exclude(users_d, ex, U, V, k, bias=bias)[0]
+        else:  # very long lists: exact device scores, excluded entries masked, then stable device sorts
+            rows = []
+            per = max(1, (1 << 24) // ni)
+            items_d = torch.arange(ni, dtype=torch.int64, device=self.device)
+            for u0 in range(0, users_d.numel(), per):
+                chunk = users_d[u0:u0 + per]
+                n = chunk.numel()
+                s = engine.predict_pairs(chunk.repeat_interleave(ni), items_d.repeat(n), U, V, bias=bias).view(n, ni)
+                lo, cnt = ex.indptr[chunk], ex.indptr[chunk + 1] - ex.indptr[chunk]
+                total = int(cnt.sum())
+                row = torch.repeat_interleave(torch.arange(n, device=self.device), cnt, output_size=total)
+                entry = torch.arange(total, device=self.device) + torch.repeat_interleave(lo - (torch.cumsum(cnt, 0) - cnt),
+                                                                                         cnt, output_size=total)
+                seen = torch.zeros((n, ni), dtype=torch.bool, device=self.device)
+                seen[row, ex.indices[entry].long()] = True
+                order = torch.sort(s, dim=1, descending=True, stable=True).indices
+                # unseen first, each group in score order (a seen item never displaces an unseen one, whatever the scores)
+                seen_sorted = seen.gather(1, order)
+                regroup = torch.sort(seen_sorted.to(torch.uint8), dim=1, stable=True).indices[:, :k]
+                rows.append(torch.where(seen_sorted.gather(1, regroup), -1, order.gather(1, regroup)))
+            ids = torch.cat(rows)
+        out[:, :k] = ids.cpu().numpy()
+        return out
+
     # ---------------------------------------------------------------- train (R2, R7, R11)
     def train(self, utility_mat, iterations, verbose=0, eval_mat=None, count_mat=None, alpha=10,
               cores=4, stopping_rounds=3, dtype="float64", min_improvement=0.0001,
