@@ -174,6 +174,25 @@ int wmf_rank_ahead(const float* S, const int32_t* cand, const int32_t* slot, int
                    const int32_t* pair_user, const int32_t* pair_item, const float* pair_score, int64_t np,
                    int32_t* ahead, void* stream);
 
+/* N5. Full-ranking quality of top-N lists (WMF.eval_ranking). No reference call site: the reference's only ranking
+ * measure is the sampled Recall@N of eval_topn (N2 above). ids [nu x K] are the lists wmf_score_topk_exclude returns
+ * (-1 padding is never a hit) for the users users[nu]; the test matrix t_* is a CSR indexed by user id with ids sorted
+ * within each row, duplicates and explicit zeros allowed. T_u = the distinct ids of row u with a non-zero stored
+ * value, h_i = hits among positions 1..i. For each cutoff k of ks_host (int32[nk], nk <= 16 distinct values in
+ * [1, K]) per_user[(row * nk + j) * 5 + m] receives, for k = ks_host[j], m = 0..4:
+ *   Recall h_k/|T_u|, Precision h_k/k, NDCG (sum of 1/log2(i+1) over hits i <= k) / (the same over i <= min(k,|T_u|)),
+ *   MAP (sum of h_i/i over hits i <= k) / min(k,|T_u|), HitRate [h_k > 0],
+ * or NaN for all of them when T_u is empty. Doubles, each user's row summed in an order fixed by its data alone.
+ * wmf_topn_metrics_reduce: sums[nk*5 + 1] = the per-value sums over the rows whose first value is not NaN, then the
+ * number of such rows; rows added in blocks whose size is fixed, the blocks in order (bitwise reproducible, whatever
+ * calls filled per_user). */
+size_t wmf_topn_metrics_workspace_bytes(int64_t nu, int nk);
+int wmf_topn_metrics(const int64_t* ids, int64_t nu, int K, const int64_t* users, const int64_t* t_indptr,
+                     const int32_t* t_indices, const float* t_data, const int32_t* ks_host, int nk, double* per_user,
+                     void* stream);
+int wmf_topn_metrics_reduce(const double* per_user, int64_t nu, int nk, double* sums, void* ws, size_t ws_bytes,
+                            void* stream);
+
 /* K4+K5. Top-N over a candidate list for a batch of users: replaces WMF.rank (:25-47).
  * Scores are the bit-exact fp32 scores of wmf_predict_pairs, so the selected index SET equals
  * the reference's; order is descending score, ties broken by lower candidate position.

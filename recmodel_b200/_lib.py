@@ -50,6 +50,9 @@ SIGNATURES = {
     "wmf_score_topk_exclude_workspace_bytes": (_sz, [_i64, _i64, _i32]),
     "wmf_score_topk_exclude": (_i32, [_p, _i64, _p, _p, _i64, _p, _i64, _p, _i64, _i32, _i32, _i32, _p, _p, _p, _p, _sz,
                                       _p]),
+    "wmf_topn_metrics_workspace_bytes": (_sz, [_i64, _i32]),
+    "wmf_topn_metrics": (_i32, [_p, _i64, _i32, _p, _p, _p, _p, _p, _i32, _p, _p]),
+    "wmf_topn_metrics_reduce": (_i32, [_p, _i64, _i32, _p, _p, _sz, _p]),
     "wmf_inverse_workspace_bytes": (_sz, [_i32]),
     "wmf_inverse": (_i32, [_p, _i32, _p, _p, _sz, _p]),
     "wmf_dense_right_multiply": (_i32, [_p, _i64, _i64, _p, _i32, _p, _i64, _p]),

@@ -10,7 +10,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(CSRC, "libwmf_b200.so")
 SOURCES = ["api.cu", "csr.cu", "ease.cu", "eval_topn.cu", "exchange.cu", "gram.cu", "half_step_api.cu", "half_step_simt.cu", "half_step_tc.cu", "half_step_tc256.cu", "half_step_dual.cu", "whiten.cu", "loss.cu", "score.cu", "score_tc.cu",
-           "unweighted.cu"]
+           "topn_metrics.cu", "unweighted.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC"]
 
 

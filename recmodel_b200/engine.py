@@ -547,6 +547,43 @@ def score_topk_exclude(users, exclude, U, V, topn, bias=False, want_scores=False
     return ids, scores, fixup
 
 
+TOPN_METRICS = ("Recall", "Precision", "NDCG", "MAP", "HitRate")  # the 5 values per cutoff, in buffer order
+
+
+@_device_of(0)
+def topn_metrics(ids, users, test_csr, ks, out=None):
+    """float64 [nu x len(ks) x 5] (``TOPN_METRICS`` order): ranking quality of the lists ``ids`` [nu x K] (int64, -1
+    padding) for the users ``users`` against the rows of ``test_csr`` (a DeviceCSR with sorted rows, indexed by user
+    id), one row of NaN per user without a non-zero test entry (include/wmf_b200.h: wmf_topn_metrics). ``ks``: host
+    sequence of at most 16 distinct cutoffs in [1, K]. ``out``: a contiguous buffer of that shape to write into."""
+    lib = _lib.load()
+    nu, K = ids.shape
+    ks_h = np.ascontiguousarray(ks, dtype=np.int32)
+    assert ids.dtype == torch.int64 and ids.is_contiguous() and users.dtype == torch.int64 and users.numel() == nu
+    assert test_csr.indices.dtype == torch.int32 and test_csr.indptr.dtype == torch.int64
+    if out is None:
+        out = torch.empty((nu, len(ks_h), 5), dtype=torch.float64, device=ids.device)
+    assert out.dtype == torch.float64 and out.is_contiguous() and tuple(out.shape) == (nu, len(ks_h), 5)
+    _lib.check(lib.wmf_topn_metrics(_ptr(ids), nu, K, _ptr(users), _ptr(test_csr.indptr), _ptr(test_csr.indices),
+                                    _ptr(test_csr.data), ks_h.ctypes.data, len(ks_h), _ptr(out), _stream()),
+               "wmf_topn_metrics")
+    return out
+
+
+@_device_of(0)
+def topn_metrics_reduce(per_user, nk):
+    """float64 device [nk*5 + 1]: the sums of the per-user values of ``topn_metrics`` over the rows that are not NaN,
+    then the number of those rows (include/wmf_b200.h: wmf_topn_metrics_reduce; bitwise reproducible)."""
+    lib = _lib.load()
+    nu = per_user.shape[0]
+    assert per_user.dtype == torch.float64 and per_user.is_contiguous() and per_user.numel() == nu * nk * 5
+    sums = torch.empty(nk * 5 + 1, dtype=torch.float64, device=per_user.device)
+    ws = workspace(lib.wmf_topn_metrics_workspace_bytes(nu, nk), per_user.device)
+    _lib.check(lib.wmf_topn_metrics_reduce(_ptr(per_user), nu, nk, _ptr(sums), _ptr(ws), ws.numel(), _stream()),
+               "wmf_topn_metrics_reduce")
+    return sums
+
+
 @_device_of(1)
 def unweighted_half_step(csr, Y, lam):
     """X = R (inv(Y^T Y + lam I) Y^T)^T  (wmf_model.py:85 / :88)."""
