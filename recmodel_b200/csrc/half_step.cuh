@@ -44,8 +44,8 @@ int simt_half_step(const HalfStepParams& in, void* ws, size_t ws_bytes, cudaStre
 bool tc_half_step_supported(int f, int bias);
 size_t tc_half_step_workspace_bytes(int64_t rows, int64_t cols, int f, int bias, int64_t segments);  // segments < 0: default scratch
 int tc_half_step(const HalfStepParams& in, void* ws, size_t ws_bytes, cudaStream_t st);
-// dual (n x n) kernel for the rows of the dual table (half_step_dual.cu)
-int tc_dual_launch(const HalfStepParams& p, const int4* dtab, const uint32_t* hdr_u, int grid, cudaStream_t st);
+// dual (n x n) kernel for the packs of short rows of the pack table (half_step_dual.cu)
+int tc_dual_launch(const HalfStepParams& p, const int4* ptab, const uint32_t* hdr_u, int grid, cudaStream_t st);
 int tc_dual_max_entries();
 int tc_cg_max_products();   // default budget of the conjugate-gradient solver (WMF_TC_CG=<n> overrides, 0 = off)
 // primal kernel for 128 < f <= 256 (half_step_tc256.cu); same tables and scratch conventions as the 128-wide one

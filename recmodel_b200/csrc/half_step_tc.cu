@@ -153,6 +153,7 @@ static bool profile_enabled() {
 }
 constexpr int DEFAULT_PARTS = 2048;  // partial slots the legacy workspace query (rows only) provides
 constexpr size_t PART_FLOATS = (size_t)F * F + F;  // a segment's S^2 W (chunk-major) and its rhs partial
+constexpr int PACK_CHUNK = 1024;   // schedule slots per dual-row counter quad (tc_prep_rows_kernel, tc_pack_dual_kernel)
 // ---------------------------------------------------------------------------------------------------
 // prep: the schedule tables (one 16-byte entry per slot and kernel), the per-row FP16 scale, zero rows
 // without entries, and the fix-up list.
@@ -166,9 +167,11 @@ constexpr size_t PART_FLOATS = (size_t)F * F + F;  // a segment's S^2 W (chunk-m
 // Rows longer than SPLIT_LEN are cut into equal segments (a function of the row length only, so a row's
 // arithmetic never depends on the launch it is in): segment 0 stays in the row's slot, the others go to
 // extra slots behind the schedule, which the persistent CTAs reach round-robin like every other slot.
+// Dual rows are also counted per chunk of PACK_CHUNK slots and per size class (32-lane TMEM slices: 1 ... 4) for the
+// pack table (tc_pack_dual_kernel).
 __global__ void tc_prep_rows_kernel(HalfStepParams p, int4* __restrict__ tab, int4* __restrict__ segtab,
-                                    int4* __restrict__ dtab, uint32_t* __restrict__ hdr_u, int64_t extra_slot0,
-                                    int max_extra, int max_parts, int SPLIT_LEN, int primal_ok) {
+                                    int4* __restrict__ dtab, uint32_t* __restrict__ pcnt, uint32_t* __restrict__ hdr_u,
+                                    int64_t extra_slot0, int max_extra, int max_parts, int SPLIT_LEN, int primal_ok) {
     const int64_t s = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
     __shared__ int64_t sh_lo[8], sh_hi[8];
@@ -251,7 +254,11 @@ __global__ void tc_prep_rows_kernel(HalfStepParams p, int4* __restrict__ tab, in
             float4* x = reinterpret_cast<float4*>(p.X + row * p.ldx);  // whitened solution: ld = FP, 16-byte aligned
             for (int i = lane; i < p.FP / 4; i += 32) x[i] = make_float4(0.f, 0.f, 0.f, 0.f);
         } else if (dual) {
-            if (lane == 0) { atomicMax(hdr_u + 10, 0x7fffffffu - (uint32_t)s); atomicMax(hdr_u + 11, (uint32_t)s + 1u); }
+            if (lane == 0) {
+                atomicMax(hdr_u + 10, 0x7fffffffu - (uint32_t)s);
+                atomicMax(hdr_u + 11, (uint32_t)s + 1u);
+                atomicAdd(pcnt + (s / PACK_CHUNK) * 4 + (dual_slices((int)n) - 1), 1u);
+            }
             de.y = (int32_t)n;
             de.z = (int32_t)(uint32_t)lo;
             de.w = (int32_t)((uint32_t)((lo >> 32) & 0xFFFF) | sbits);
@@ -304,10 +311,118 @@ __global__ void tc_prep_rows_kernel(HalfStepParams p, int4* __restrict__ tab, in
     if (lane == 0) { tab[s] = e; dtab[s] = de; }
 }
 
-// total slots = schedule (rounded up to a multiple of the grid) + extra segment slots
-__global__ void tc_finish_prep_kernel(uint32_t* __restrict__ hdr_u, int64_t extra_slot0, int max_extra) {
-    const uint32_t extra = hdr_u[7] < (uint32_t)max_extra ? hdr_u[7] : (uint32_t)max_extra;
-    hdr_u[4] = (uint32_t)(extra_slot0 + extra);
+__device__ __forceinline__ uint4 add4u(uint4 a, uint4 b) { return make_uint4(a.x + b.x, a.y + b.y, a.z + b.z, a.w + b.w); }
+__device__ __forceinline__ uint32_t get4u(uint4 a, int k) { return k == 0 ? a.x : k == 1 ? a.y : k == 2 ? a.z : a.w; }
+__device__ __forceinline__ uint4 warp_scan4u(uint4 x) {   // inclusive
+    const int lane = threadIdx.x & 31;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const uint4 y = make_uint4(__shfl_up_sync(0xffffffffu, x.x, o), __shfl_up_sync(0xffffffffu, x.y, o),
+                                   __shfl_up_sync(0xffffffffu, x.z, o), __shfl_up_sync(0xffffffffu, x.w, o));
+        if (lane >= o) x = add4u(x, y);
+    }
+    return x;
+}
+
+// Packs of the dual kernel, longest first: every system of 4 slices alone; every 3-slice system with a 1-slice one
+// from the short end of the 1-slice list while they last; the 2-slice systems in pairs, an odd one out with up to two
+// more 1-slice systems; the remaining 1-slice systems in fours. With the dual rows of one size class in slot order
+// (longest first on a sorted schedule), the row of rank i in class cls goes to (pack, first slice); `empty` gets
+// the slices of that pack nobody takes when the row is its slice-0 system.
+struct DualPackCounts {
+    uint32_t c1, c2, c3, c4, m31, r1, p2, m21, r1b, packs;
+    __device__ explicit DualPackCounts(const uint32_t* cnt) {
+        c1 = cnt[0]; c2 = cnt[1]; c3 = cnt[2]; c4 = cnt[3];
+        m31 = c1 < c3 ? c1 : c3;                   // 1-slice systems sharing a pack with a 3-slice one
+        r1 = c1 - m31;
+        p2 = (c2 + 1) / 2;
+        m21 = (c2 & 1u) ? (r1 < 2u ? r1 : 2u) : 0u;   // 1-slice systems beside the odd 2-slice one
+        r1b = r1 - m21;
+        packs = c4 + c3 + p2 + (r1b + 3) / 4;
+    }
+    __device__ void place(int cls, uint32_t i, int64_t& pack, int& slice, uint32_t& empty) const {
+        empty = 0;
+        if (cls == 3) { pack = i; slice = 0; }
+        else if (cls == 2) { pack = c4 + i; slice = 0; if (i >= m31) empty = 8u; }
+        else if (cls == 1) {
+            pack = c4 + c3 + i / 2; slice = 2 * (int)(i & 1u);
+            if ((c2 & 1u) && i == c2 - 1) empty = (m21 < 1 ? 4u : 0u) | (m21 < 2 ? 8u : 0u);
+        } else if (i >= r1) { pack = c4 + (c1 - 1 - i); slice = 3; }   // rank c1 - 1 - j joins 3-slice system j
+        else if (i >= r1b) { pack = c4 + c3 + p2 - 1; slice = 2 + (int)(r1 - 1 - i); }
+        else {
+            pack = c4 + c3 + p2 + i / 4; slice = (int)(i & 3u);
+            if (slice == 0)
+                for (uint32_t k = 1; k < 4; ++k) if (i + k >= r1b) empty |= 1u << k;
+        }
+    }
+};
+
+// total slots = schedule (rounded up to a multiple of the grid) + extra segment slots. The per-chunk dual-row counts
+// become exclusive prefixes per size class (in place); the class totals go to hdr[14 .. 17], the number of packs to hdr[13].
+__global__ void __launch_bounds__(1024) tc_finish_prep_kernel(uint32_t* __restrict__ hdr_u, int64_t extra_slot0, int max_extra,
+                                                              uint4* __restrict__ pcnt, int nchunks) {
+    __shared__ uint4 wsum[32];
+    __shared__ uint4 carry;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    if (tid == 0) {
+        const uint32_t extra = hdr_u[7] < (uint32_t)max_extra ? hdr_u[7] : (uint32_t)max_extra;
+        hdr_u[4] = (uint32_t)(extra_slot0 + extra);
+        carry = make_uint4(0u, 0u, 0u, 0u);
+    }
+    __syncthreads();
+    for (int c0 = 0; c0 < nchunks; c0 += 1024) {
+        const int c = c0 + tid;
+        const uint4 v = c < nchunks ? pcnt[c] : make_uint4(0u, 0u, 0u, 0u);
+        const uint4 x = warp_scan4u(v);
+        if (lane == 31) wsum[warp] = x;
+        __syncthreads();
+        if (warp == 0) wsum[lane] = warp_scan4u(wsum[lane]);
+        __syncthreads();
+        uint4 ex = add4u(carry, make_uint4(x.x - v.x, x.y - v.y, x.z - v.z, x.w - v.w));
+        if (warp > 0) ex = add4u(ex, wsum[warp - 1]);
+        if (c < nchunks) pcnt[c] = ex;
+        __syncthreads();
+        if (tid == 0) carry = add4u(carry, wsum[31]);
+        __syncthreads();
+    }
+    if (tid == 0) {
+        const uint32_t cnt[4] = {carry.x, carry.y, carry.z, carry.w};
+        for (int k = 0; k < 4; ++k) hdr_u[14 + k] = cnt[k];
+        hdr_u[13] = DualPackCounts(cnt).packs;
+    }
+}
+
+// One block per chunk of the schedule: each dual row gets its rank in its size class (slot order: chunk prefix, then
+// warps, then lanes) and from it its place in the pack table; its entry is written to every slice it covers.
+__global__ void __launch_bounds__(PACK_CHUNK) tc_pack_dual_kernel(const int4* __restrict__ dtab, const uint4* __restrict__ pcnt,
+                                                                  const uint32_t* __restrict__ hdr_u, int4* __restrict__ ptab,
+                                                                  int64_t sched_len) {
+    __shared__ uint32_t wcnt[PACK_CHUNK / 32][4];
+    const int64_t s = (int64_t)blockIdx.x * PACK_CHUNK + threadIdx.x;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int4 de = s < sched_len ? dtab[s] : make_int4(-1, 0, 0, 0);
+    const int cls = de.y > 0 ? dual_slices(de.y) - 1 : -1;
+    uint32_t rank = 0;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        const uint32_t m = __ballot_sync(0xffffffffu, cls == k);
+        if (lane == 0) wcnt[warp][k] = __popc(m);
+        if (cls == k) rank = __popc(m & ((1u << lane) - 1u));
+    }
+    __syncthreads();
+    if (cls < 0) return;
+    for (int w = 0; w < warp; ++w) rank += wcnt[w][cls];
+    rank += get4u(pcnt[blockIdx.x], cls);
+    const DualPackCounts pc(hdr_u + 14);
+    int64_t pack;
+    int slice;
+    uint32_t empty;
+    pc.place(cls, rank, pack, slice, empty);
+    int4 ent = de;
+    ent.w = (int32_t)((uint32_t)ent.w | ((uint32_t)slice << 24));
+    for (int k = 0; k <= cls; ++k) ptab[pack * 4 + slice + k] = ent;
+    for (int k = 1; k < 4; ++k)
+        if (empty & (1u << k)) ptab[pack * 4 + k] = make_int4(-1, 0, 0, 0);
 }
 
 }  // namespace tc
@@ -946,16 +1061,19 @@ bool tc_half_step_supported(int f, int bias) { return f >= 1 && f <= 256 && (!bi
 //   [0, 1024)   header: [1] flags (1 unused, 2 failed pivot, 8 G not positive definite), [2] max y~^2 (float bits),
 //               [4] total slots, [5] split rows, [6] partial slots, [7] extra slots, [8] fix-up rows, [9] end of the
 //               primal rows' slots, [10] 0x7fffffff - first dual slot, [11] end of the dual rows' slots, [12] nonzero when the
-//               conjugate gradients of some row did not converge (factorised instead); [256, 768) profile
-//   tables      primal row table + split table (32 B per slot), dual row table (16 B per slot), split-row counters,
-//               fix-up list (4 B per row)
+//               conjugate gradients of some row did not converge (factorised instead), [13] packs of the dual kernel,
+//               [14 .. 17] dual rows of 1 ... 4 slices; [256, 768) profile
+//   tables      primal row table + split table (32 B per slot), dual row table (16 B per slot), dual-row counts per
+//               chunk of PACK_CHUNK slots (16 B), split-row counters, fix-up list (4 B per row), dual pack table (64 B per
+//               row: a pack holds at least one row, and a schedule names a row at most once, as the fix-up list assumes)
 //   whitening   double scratch of the Cholesky, the two FP x FP multipliers, Y~ (cols x FP), X' (rows x FP)
 //   simt        the CUDA-core kernel's own workspace (fix-up rows)
 //   parts       partial-Gram scratch for the segments of split rows: whatever is left
 struct TcLayout {
     int64_t cap_slots, max_parts;
-    size_t off_tab, off_seg, off_dtab, off_cnt, off_fix, zero_end, off_chol, off_mw, off_mu, off_eye, off_yt, off_xp,
-        off_simt, off_parts, total;
+    int64_t pack_chunks;
+    size_t off_tab, off_seg, off_dtab, off_pcnt, off_cnt, off_fix, zero_end, off_ptab, off_chol, off_mw, off_mu, off_eye,
+        off_yt, off_xp, off_simt, off_parts, total;
 };
 static int tc_fp(int f) { return f <= 128 ? 128 : 256; }
 static size_t part_floats(int f) { return f <= F ? PART_FLOATS : tc256_part_floats(); }  // a parked segment: matrix + rhs
@@ -967,10 +1085,13 @@ static TcLayout tc_layout(int64_t sched_slots, int64_t rows, int64_t cols, int f
     L.off_tab = WS_TABLES;
     L.off_seg = L.off_tab + 16 * (size_t)L.cap_slots;
     L.off_dtab = L.off_seg + 16 * (size_t)L.cap_slots;
-    L.off_cnt = L.off_dtab + 16 * (size_t)sched_slots;
+    L.pack_chunks = (sched_slots + PACK_CHUNK - 1) / PACK_CHUNK;
+    L.off_pcnt = L.off_dtab + 16 * (size_t)sched_slots;
+    L.off_cnt = L.off_pcnt + 16 * (size_t)L.pack_chunks;
     L.off_fix = align_up(L.off_cnt + 4 * (size_t)(L.max_parts / 2 + 1), 256);
     L.zero_end = L.off_fix;  // header, tables and counters are cleared per call; the list is bounded by its counter
-    L.off_chol = align_up(L.off_fix + 4 * (size_t)(rows + 1), 256);
+    L.off_ptab = align_up(L.off_fix + 4 * (size_t)(rows + 1), 256);   // written in full up to its pack count
+    L.off_chol = align_up(L.off_ptab + 64 * (size_t)(rows < sched_slots ? rows : sched_slots), 256);
     L.off_mw = L.off_chol + whiten_scratch_bytes(f);
     L.off_mu = L.off_mw + FP * FP * sizeof(float);
     L.off_eye = L.off_mu + FP * FP * sizeof(float);           // f x f identity: the whitened G of the fix-up kernel
@@ -1040,14 +1161,20 @@ int tc_half_step(const HalfStepParams& in, void* ws, size_t ws_bytes, cudaStream
     p.nd_max = dual_enabled() ? (FP > F ? 128 : tc_dual_max_entries()) : 0;
     p.prof = profile_enabled() ? reinterpret_cast<long long*>(base + WS_PROF) : nullptr;
     const int primal_ok = 1;   // 128-wide kernel of this file, or the 256-wide one (half_step_tc256.cu)
-    tc_prep_rows_kernel<<<(unsigned)((in.sched_len + 7) / 8), 256, 0, st>>>(p, tab, segtab, dtab, hdr_u, extra_slot0,
+    uint32_t* pcnt = reinterpret_cast<uint32_t*>(base + L.off_pcnt);
+    tc_prep_rows_kernel<<<(unsigned)((in.sched_len + 7) / 8), 256, 0, st>>>(p, tab, segtab, dtab, pcnt, hdr_u, extra_slot0,
                                                                             (int)max_parts, (int)max_parts, split_len(),
                                                                             primal_ok);
     WMF_LAUNCH_CHECK("tc_prep_rows_kernel");
-    tc_finish_prep_kernel<<<1, 1, 0, st>>>(hdr_u, extra_slot0, (int)max_parts);
+    const int pack_chunks = (int)((in.sched_len + PACK_CHUNK - 1) / PACK_CHUNK);
+    tc_finish_prep_kernel<<<1, 1024, 0, st>>>(hdr_u, extra_slot0, (int)max_parts, reinterpret_cast<uint4*>(pcnt), pack_chunks);
     WMF_LAUNCH_CHECK("tc_finish_prep_kernel");
     if (p.nd_max > 0) {
-        rc = tc_dual_launch(p, dtab, hdr_u, grid, st);
+        int4* ptab = reinterpret_cast<int4*>(base + L.off_ptab);
+        tc_pack_dual_kernel<<<(unsigned)pack_chunks, PACK_CHUNK, 0, st>>>(dtab, reinterpret_cast<const uint4*>(pcnt), hdr_u,
+                                                                          ptab, in.sched_len);
+        WMF_LAUNCH_CHECK("tc_pack_dual_kernel");
+        rc = tc_dual_launch(p, ptab, hdr_u, grid, st);
         if (rc) return rc;
     }
     if (in.f > F) {

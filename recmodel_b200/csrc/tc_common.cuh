@@ -22,6 +22,12 @@ __device__ __forceinline__ RowEnt unpack_ent(const int4 v, int slot) {
     e.part = (v.w < 0) ? slot : -1;
     return e;
 }
+// Dual kernel (half_step_dual.cu): an n-entry system takes dual_slices(n) 32-lane slices of its group's 128 TMEM
+// lanes, and up to four systems share them on the block diagonal. The pack table holds four entries per pack, one per
+// slice: the entry of the system covering that slice, with its first slice in bits 24-25 of the last word (n = 0: no
+// system there).
+__host__ __device__ __forceinline__ int dual_slices(int n) { return (n + 31) >> 5; }
+__device__ __forceinline__ int pack_first_slice(const int4 v) { return (int)(((uint32_t)v.w >> 24) & 3u); }
 // second table, one 16-byte record per segment of a split row
 struct __align__(16) SegEnt {
     int32_t split_id;    // counter slot of the row
