@@ -243,6 +243,23 @@ int wmf_ease_train(const int64_t* indptr, const int32_t* indices, const float* d
 int wmf_ease_predict(const int64_t* indptr, const int32_t* indices, const float* data, const float* W, int64_t n,
                      const int64_t* users, int64_t user_stride, const int64_t* items, int64_t count, double* out,
                      void* stream);
+/* N4 ranking: top-N of all n items minus the ones each user has interacted with, for nu users in one call: replaces
+ * the per-user Ease.rank(np.delete(all_items, seen), user) loop of test_coverage (RecModel/utils.py:3-18). No
+ * reference call site ranks EASE over all items in one call.
+ * Score s(u, i) = the sum over the stored entries e of row u of X (x_*, in stored order, from +0.0) of
+ * (double)(x_e * W[j_e, i]) with the product rounded to FP32: bitwise what wmf_ease_predict returns. Unsorted rows,
+ * duplicates and explicit zeros in X take part as stored. The double scores are ranked as they are (no FP32 rounding),
+ * descending, ties to the lower item id. ex_indptr (nullable: nothing excluded) / ex_indices: a CSR indexed by user
+ * id whose row users[k] lists the item ids to leave out (unsorted rows and duplicates allowed, values not read).
+ * out_ids [nu*topn] receives item ids, out_scores (nullable) [nu*topn] their scores; a user with fewer than topn
+ * unseen items gets id -1 and score NaN in the rest of its row. 1 <= topn <= min(n, 1024) (else
+ * WMF_ERR_UNSUPPORTED), 0 < n < 2^31. The workspace holds one [ub x n] double score tile, ub from n and a fixed
+ * byte budget. */
+size_t wmf_ease_score_topk_workspace_bytes(int64_t nu, int64_t n, int topn);
+int wmf_ease_score_topk(const int64_t* x_indptr, const int32_t* x_indices, const float* x_data, const float* W,
+                        int64_t n, const int64_t* users, int64_t nu, const int64_t* ex_indptr,
+                        const int32_t* ex_indices, int topn, int64_t* out_ids, double* out_scores, void* ws,
+                        size_t ws_bytes, void* stream);
 
 #ifdef __cplusplus
 }

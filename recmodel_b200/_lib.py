@@ -60,6 +60,8 @@ SIGNATURES = {
     "wmf_ease_workspace_bytes": (_sz, [_i64]),
     "wmf_ease_train": (_i32, [_p, _p, _p, _i64, _i64, _f32, _p, _p, _sz, _p]),
     "wmf_ease_predict": (_i32, [_p, _p, _p, _p, _i64, _p, _i64, _p, _i64, _p, _p]),
+    "wmf_ease_score_topk_workspace_bytes": (_sz, [_i64, _i64, _i32]),
+    "wmf_ease_score_topk": (_i32, [_p, _p, _p, _p, _i64, _p, _i64, _p, _p, _i32, _p, _p, _p, _sz, _p]),
 }
 
 

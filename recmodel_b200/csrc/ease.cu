@@ -4,9 +4,11 @@
 //   P = inv(G)                               :102                  -> blocked in-place Gauss-Jordan (no pivoting: G is SPD)
 //   W = P / (-diag(P) + 1e-9), diag(W) = 0   :106-108              -> ease_finish_kernel
 //   predict: sum_j X[u, j] W[j, item]        fast_utils/ease_utils.pyx:15-30 -> ease_predict_kernel
+//   top-N of a user's unseen items (Ease.recommend)                 -> ease_score_tile_kernel + the exact selection
 // The inverse is n^3 FP32 FMAs as rank-64 updates (register-blocked 128 x 128 tiles): compute-bound on the CUDA
 // cores, 0.6 s at the 26 744 items of ML-20M; the reference does the same arithmetic in FP32 LAPACK (sgetri).
 #include "common.cuh"
+#include "score.cuh"
 
 namespace wmf {
 
@@ -165,6 +167,54 @@ __global__ void ease_predict_kernel(const int64_t* __restrict__ indptr, const in
     out[k] = acc;
 }
 
+constexpr int ES_THREADS = 128;  // item columns per CTA (one per thread)
+constexpr int ES_USERS = 4;      // users per CTA
+
+// S[r][i] = sum_j X[users[u_begin + r], j] W[j, i] for the ub users of a batch, with the arithmetic of
+// ease_predict_kernel (so every score is bitwise what wmf_ease_predict returns). CTA = (item panel, group of ES_USERS
+// users); the item panel is the outer index, so the CTAs running together share a panel of W, which is fetched from
+// HBM about once per batch and read from L2 by the other users of the batch.
+__global__ __launch_bounds__(ES_THREADS) void ease_score_tile_kernel(const int64_t* __restrict__ indptr,
+                                                                     const int32_t* __restrict__ indices,
+                                                                     const float* __restrict__ data,
+                                                                     const float* __restrict__ W, int64_t n,
+                                                                     const int64_t* __restrict__ users, int64_t u_begin,
+                                                                     int ub, double* __restrict__ S) {
+    const int groups = (ub + ES_USERS - 1) / ES_USERS;
+    const int64_t panel = blockIdx.x / groups;
+    const int g = (int)(blockIdx.x % groups);
+    const int64_t i = panel * ES_THREADS + threadIdx.x;
+    if (i >= n) return;
+    const float* __restrict__ Wi = W + i;
+    for (int q = 0; q < ES_USERS; ++q) {
+        const int r = g * ES_USERS + q;
+        if (r >= ub) break;
+        const int64_t u = users[u_begin + r];
+        const int64_t lo = indptr[u], hi = indptr[u + 1];
+        double acc = 0.0;
+        int64_t e = lo;
+        for (; e + 4 <= hi; e += 4) {  // loads first, then the adds in stored order
+            const float w0 = Wi[(int64_t)indices[e] * n], w1 = Wi[(int64_t)indices[e + 1] * n];
+            const float w2 = Wi[(int64_t)indices[e + 2] * n], w3 = Wi[(int64_t)indices[e + 3] * n];
+            acc += (double)__fmul_rn(data[e], w0);
+            acc += (double)__fmul_rn(data[e + 1], w1);
+            acc += (double)__fmul_rn(data[e + 2], w2);
+            acc += (double)__fmul_rn(data[e + 3], w3);
+        }
+        for (; e < hi; ++e) acc += (double)__fmul_rn(data[e], Wi[(int64_t)indices[e] * n]);
+        S[(size_t)r * n + i] = acc;
+    }
+}
+
+// users per score tile: keep the [ub x n] double tile near 64 MiB so the selection passes hit L2 (126 MB)
+int64_t ease_user_batch(int64_t nu, int64_t n) {
+    int64_t ub = (64ll << 20) / (n * 8);
+    if (ub < ES_USERS) ub = ES_USERS;
+    ub = ub / ES_USERS * ES_USERS;
+    if (ub > nu) ub = nu;
+    return ub;
+}
+
 }  // namespace
 
 }  // namespace wmf
@@ -220,6 +270,45 @@ int wmf_ease_predict(const int64_t* indptr, const int32_t* indices, const float*
     ease_predict_kernel<<<(unsigned)((count + 127) / 128), 128, 0, (cudaStream_t)stream>>>(indptr, indices, data, W, n, users,
                                                                                       user_stride, items, count, out);
     WMF_LAUNCH_CHECK("ease_predict_kernel");
+    return WMF_OK;
+}
+
+size_t wmf_ease_score_topk_workspace_bytes(int64_t nu, int64_t n, int topn) {
+    (void)topn;
+    if (nu <= 0 || n <= 0 || n >= (1ll << 31)) return 0;
+    return align_up((size_t)ease_user_batch(nu, n) * (size_t)n * sizeof(double), 1024);
+}
+
+int wmf_ease_score_topk(const int64_t* x_indptr, const int32_t* x_indices, const float* x_data, const float* W,
+                        int64_t n, const int64_t* users, int64_t nu, const int64_t* ex_indptr,
+                        const int32_t* ex_indices, int topn, int64_t* out_ids, double* out_scores, void* ws,
+                        size_t ws_bytes, void* stream) {
+    WMF_REQUIRE(n > 0 && n < (1ll << 31), "wmf_ease_score_topk: n=%lld outside 1..2^31-1", (long long)n);
+    WMF_REQUIRE(nu >= 0, "wmf_ease_score_topk: nu=%lld < 0", (long long)nu);
+    if (topn < 1 || topn > n || topn > TK_MAX) {
+        set_error("wmf_ease_score_topk: topn=%d outside 1..min(n=%lld, %d)", topn, (long long)n, TK_MAX);
+        return WMF_ERR_UNSUPPORTED;
+    }
+    if (nu == 0) return WMF_OK;
+    WMF_REQUIRE(x_indptr && W && users && out_ids, "wmf_ease_score_topk: null argument");
+    const size_t need = wmf_ease_score_topk_workspace_bytes(nu, n, topn);
+    if (ws == nullptr || ws_bytes < need) {
+        set_error("wmf_ease_score_topk: workspace %zu < %zu", ws_bytes, need);
+        return WMF_ERR_WORKSPACE;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    const int64_t ubatch = ease_user_batch(nu, n);
+    double* S = (double*)ws;
+    const int64_t panels = (n + ES_THREADS - 1) / ES_THREADS;
+    for (int64_t u0 = 0; u0 < nu; u0 += ubatch) {
+        const int ub = (int)((nu - u0) < ubatch ? (nu - u0) : ubatch);
+        const int64_t grid = panels * ((ub + ES_USERS - 1) / ES_USERS);
+        ease_score_tile_kernel<<<(unsigned)grid, ES_THREADS, 0, st>>>(x_indptr, x_indices, x_data, W, n, users, u0, ub, S);
+        WMF_LAUNCH_CHECK("ease_score_tile_kernel");
+        const int rc = select_topk_double(users, u0, ub, ex_indptr, ex_indices, S, n, topn, out_ids + (size_t)u0 * topn,
+                                          out_scores ? out_scores + (size_t)u0 * topn : nullptr, st);
+        if (rc) return rc;
+    }
     return WMF_OK;
 }
 

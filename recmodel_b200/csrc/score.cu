@@ -16,6 +16,7 @@ namespace wmf {
 
 constexpr int SC_THREADS = 128;  // items per tile (one per thread)
 constexpr int SC_USERS = 32;     // users per CTA pass (8 groups of 4)
+constexpr int TK_THREADS = 256;
 
 // NumPy pairwise block (n <= 128) for 4 users sharing one item row; u rows are in smem.
 __device__ __forceinline__ void np_block4(const float* __restrict__ u0, const float* __restrict__ u1,
@@ -145,49 +146,51 @@ __global__ __launch_bounds__(SC_THREADS) void score_tile_kernel(const int64_t* _
     }
 }
 
-// Excluded items of the users of a score tile: their scores become the bit pattern 0xFFFFFFFF, which order_key maps
+// Excluded items of the users of a score tile: their scores become the all-ones bit pattern, which order_key maps
 // to 0, below every other score. One CTA per user row (grid-stride).
-constexpr uint32_t EXCLUDED_BITS = 0xFFFFFFFFu;
-
+template <typename T>
 __global__ __launch_bounds__(256) void score_exclude_kernel(const int64_t* __restrict__ users, int64_t u_begin, int ub,
                                                             const int64_t* __restrict__ ex_indptr,
                                                             const int32_t* __restrict__ ex_indices, int64_t ni,
-                                                            float* __restrict__ S, const int* __restrict__ run_if) {
+                                                            T* __restrict__ S, const int* __restrict__ run_if) {
     if (run_if != nullptr && *run_if == 0) return;
     for (int r = blockIdx.x; r < ub; r += gridDim.x) {
         const int64_t user = users[u_begin + r];
         const int64_t lo = ex_indptr[user], hi = ex_indptr[user + 1];
         for (int64_t e = lo + threadIdx.x; e < hi; e += blockDim.x)
-            S[(size_t)r * ni + ex_indices[e]] = __uint_as_float(EXCLUDED_BITS);
+            S[(size_t)r * ni + ex_indices[e]] = RankKey<T>::excluded();
     }
 }
 
-constexpr int TK_THREADS = 256;
-constexpr int TK_MAX = 1024;  // largest topn this kernel sorts in shared memory
-
-// One CTA per user row of S: k-th largest key by 4x8-bit radix select, gather winners
+// One CTA per user row of S: k-th largest key by 8-bit radix select (4 passes for float, 8 for double), gather winners
 // (ties at the threshold taken in candidate order), bitonic sort descending. `excl`: winners with key 0 are
 // excluded items (score_exclude_kernel) a user with fewer than topn others is left with: id -1, score NaN.
-__global__ __launch_bounds__(TK_THREADS) void topk_rows_kernel(const float* __restrict__ S, int64_t ni, int topn,
+template <typename T>
+__global__ __launch_bounds__(TK_THREADS) void topk_rows_kernel(const T* __restrict__ S, int64_t ni, int topn,
                                                                const int64_t* __restrict__ cand,
                                                                int64_t* __restrict__ out_ids,
-                                                               float* __restrict__ out_scores,
+                                                               T* __restrict__ out_scores,
                                                                const int* __restrict__ run_if, int excl) {
+    using R = RankKey<T>;
+    using Key = typename R::Key;
+    using Entry = typename R::Entry;
     __shared__ unsigned hist[256];
     if (run_if != nullptr && *run_if == 0) return;
-    __shared__ unsigned long long keys[TK_MAX];
-    __shared__ unsigned s_prefix, s_need, s_count, s_tie_base;
+    __shared__ Entry keys[TK_MAX];
+    __shared__ Key s_prefix;
+    __shared__ unsigned s_need, s_count, s_tie_base;
     __shared__ unsigned s_scan[TK_THREADS / 32];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const float* row = S + (size_t)blockIdx.x * ni;
+    const T* row = S + (size_t)blockIdx.x * ni;
     // --- radix select: find key T = topn-th largest
-    unsigned prefix = 0, mask = 0, need = (unsigned)topn;
-    for (int shift = 24; shift >= 0; shift -= 8) {
+    Key prefix = 0, mask = 0;
+    unsigned need = (unsigned)topn;
+    for (int shift = R::BITS - 8; shift >= 0; shift -= 8) {
         hist[tid] = 0;
         __syncthreads();
         for (int64_t i = tid; i < ni; i += TK_THREADS) {
-            const uint32_t k = order_key(row[i]);
-            if ((k & mask) == prefix) atomicAdd(&hist[(k >> shift) & 255u], 1u);
+            const Key k = order_key(row[i]);
+            if ((k & mask) == prefix) atomicAdd(&hist[(unsigned)(k >> shift) & 255u], 1u);
         }
         __syncthreads();
         if (tid == 0) {
@@ -197,25 +200,25 @@ __global__ __launch_bounds__(TK_THREADS) void topk_rows_kernel(const float* __re
                 if (acc + hist[b] >= need) break;
                 acc += hist[b];
             }
-            s_prefix = prefix | ((unsigned)b << shift);
+            s_prefix = prefix | ((Key)b << shift);
             s_need = need - acc;  // how many still needed inside bucket b
         }
         __syncthreads();
         prefix = s_prefix;
         need = s_need;
-        mask |= 255u << shift;
+        mask |= (Key)255u << shift;
         __syncthreads();
     }
-    const uint32_t T = prefix;       // threshold key
-    const unsigned need_ties = need; // winners with key == T, lowest positions first
+    const Key T_ = prefix;           // threshold key
+    const unsigned need_ties = need; // winners with key == T_, lowest positions first
     if (tid == 0) { s_count = 0; s_tie_base = 0; }
     __syncthreads();
     // --- strictly greater: any order (sorted afterwards)
     for (int64_t i = tid; i < ni; i += TK_THREADS) {
-        const uint32_t k = order_key(row[i]);
-        if (k > T) {
+        const Key k = order_key(row[i]);
+        if (k > T_) {
             unsigned slot = atomicAdd(&s_count, 1u);
-            keys[slot] = ((unsigned long long)k << 32) | (unsigned long long)(0xFFFFFFFFu - (uint32_t)i);
+            keys[slot] = R::entry(k, (uint32_t)i);
         }
     }
     __syncthreads();
@@ -225,7 +228,7 @@ __global__ __launch_bounds__(TK_THREADS) void topk_rows_kernel(const float* __re
         const unsigned taken = s_tie_base;
         if (taken >= need_ties) break;  // uniform (read after the barrier below / initial barrier)
         const int64_t i = base + tid;
-        const bool is_tie = i < ni && order_key(row[i]) == T;
+        const bool is_tie = i < ni && order_key(row[i]) == T_;
         const unsigned bal = __ballot_sync(0xffffffffu, is_tie);
         if (lane == 0) s_scan[warp] = __popc(bal);
         __syncthreads();
@@ -235,16 +238,15 @@ __global__ __launch_bounds__(TK_THREADS) void topk_rows_kernel(const float* __re
             total += s_scan[w];
         }
         const unsigned rank = taken + before + __popc(bal & ((1u << lane) - 1u));
-        if (is_tie && rank < need_ties)
-            keys[n_gt + rank] = ((unsigned long long)T << 32) | (unsigned long long)(0xFFFFFFFFu - (uint32_t)i);
+        if (is_tie && rank < need_ties) keys[n_gt + rank] = R::entry(T_, (uint32_t)i);
         __syncthreads();
         if (tid == 0) s_tie_base = taken + total;
         __syncthreads();
     }
-    // --- bitonic sort (descending) of topn composite keys, padded to a power of two with 0
+    // --- bitonic sort (descending) of topn composite keys, padded to a power of two with key 0
     int npow = 1;
     while (npow < topn) npow <<= 1;
-    for (int i = topn + tid; i < npow; i += TK_THREADS) keys[i] = 0ull;
+    for (int i = topn + tid; i < npow; i += TK_THREADS) keys[i] = R::entry(0, 0xFFFFFFFFu);
     __syncthreads();
     for (int size = 2; size <= npow; size <<= 1) {
         for (int stride = size >> 1; stride > 0; stride >>= 1) {
@@ -252,19 +254,32 @@ __global__ __launch_bounds__(TK_THREADS) void topk_rows_kernel(const float* __re
                 const int lo = 2 * t - (t & (stride - 1));
                 const int hi = lo + stride;
                 const bool desc = ((lo & size) == 0);
-                const unsigned long long a = keys[lo], b = keys[hi];
-                if ((a < b) == desc) { keys[lo] = b; keys[hi] = a; }
+                const Entry a = keys[lo], b = keys[hi];
+                if (R::less(a, b) == desc) { keys[lo] = b; keys[hi] = a; }
             }
             __syncthreads();
         }
     }
     for (int t = tid; t < topn; t += TK_THREADS) {
-        const unsigned long long k = keys[t];
-        const uint32_t pos = 0xFFFFFFFFu - (uint32_t)(k & 0xFFFFFFFFull);
-        const bool none = excl && (k >> 32) == 0ull;
+        const Entry k = keys[t];
+        const uint32_t pos = R::pos(k);
+        const bool none = excl && R::key(k) == 0;
         out_ids[(size_t)blockIdx.x * topn + t] = none ? -1 : (cand ? cand[pos] : (int64_t)pos);
         if (out_scores) out_scores[(size_t)blockIdx.x * topn + t] = row[pos];
     }
+}
+
+int select_topk_double(const int64_t* users, int64_t u_begin, int ub, const int64_t* ex_indptr, const int32_t* ex_indices,
+                       double* S, int64_t ni, int topn, int64_t* out_ids, double* out_scores, cudaStream_t st) {
+    if (ex_indptr) {
+        score_exclude_kernel<double><<<(unsigned)(ub < 65535 ? ub : 65535), 256, 0, st>>>(users, u_begin, ub, ex_indptr,
+                                                                                           ex_indices, ni, S, nullptr);
+        WMF_LAUNCH_CHECK("score_exclude_kernel<double>");
+    }
+    topk_rows_kernel<double><<<ub, TK_THREADS, 0, st>>>(S, ni, topn, nullptr, out_ids, out_scores, nullptr,
+                                                        ex_indptr != nullptr);
+    WMF_LAUNCH_CHECK("topk_rows_kernel<double>");
+    return WMF_OK;
 }
 
 static int64_t score_user_batch(int64_t nu, int64_t ni) {

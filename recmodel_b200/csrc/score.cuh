@@ -1,14 +1,60 @@
-// Shared by the exact (score.cu) and tensor-core (score_tc.cu) ranking paths.
+// Shared by the exact (score.cu) and tensor-core (score_tc.cu) ranking paths, and by the EASE ranking (ease.cu).
 #pragma once
 #include "common.cuh"
 
 namespace wmf {
+
+constexpr int TK_MAX = 1024;  // largest topn the selection kernel sorts in shared memory
 
 // order-preserving map float -> uint32 (larger float -> larger key)
 __device__ __forceinline__ uint32_t order_key(float x) {
     uint32_t b = __float_as_uint(x);
     return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
 }
+
+// order-preserving map double -> uint64
+__device__ __forceinline__ unsigned long long order_key(double x) {
+    const unsigned long long b = (unsigned long long)__double_as_longlong(x);
+    return (b & 0x8000000000000000ull) ? ~b : (b | 0x8000000000000000ull);
+}
+
+// What the selection kernel (topk_rows_kernel) sorts for each score type. The all-ones score (`excluded()`) maps to
+// key 0, below every other score. An Entry packs the order key with 0xFFFFFFFF - position, so that the larger entry
+// is the larger score and, among equal scores, the lower position.
+template <typename T> struct RankKey;
+
+template <> struct RankKey<float> {
+    using Key = uint32_t;
+    using Entry = unsigned long long;
+    static constexpr int BITS = 32;
+    __device__ static float excluded() { return __uint_as_float(0xFFFFFFFFu); }
+    __device__ static Entry entry(Key k, uint32_t pos) {
+        return ((unsigned long long)k << 32) | (unsigned long long)(0xFFFFFFFFu - pos);
+    }
+    __device__ static bool less(Entry a, Entry b) { return a < b; }
+    __device__ static uint32_t pos(Entry e) { return 0xFFFFFFFFu - (uint32_t)(e & 0xFFFFFFFFull); }
+    __device__ static Key key(Entry e) { return (Key)(e >> 32); }
+};
+
+template <> struct RankKey<double> {
+    using Key = unsigned long long;
+    struct Entry {
+        unsigned long long k;
+        uint32_t p;  // 0xFFFFFFFF - position
+    };
+    static constexpr int BITS = 64;
+    __device__ static double excluded() { return __longlong_as_double(-1ll); }
+    __device__ static Entry entry(Key k, uint32_t pos) { return Entry{k, 0xFFFFFFFFu - pos}; }
+    __device__ static bool less(Entry a, Entry b) { return a.k < b.k || (a.k == b.k && a.p < b.p); }
+    __device__ static uint32_t pos(Entry e) { return 0xFFFFFFFFu - e.p; }
+    __device__ static Key key(Entry e) { return e.k; }
+};
+
+// Exact selection over a [ub x ni] tile of double scores S (row r: user users[u_begin + r]), the kernels of the exact
+// ranking path instantiated for double (score.cu). ex_indptr (nullable) / ex_indices: the exclusion CSR by user id.
+// out_ids / out_scores (nullable) [ub x topn]; topn in 1..min(ni, TK_MAX).
+int select_topk_double(const int64_t* users, int64_t u_begin, int ub, const int64_t* ex_indptr, const int32_t* ex_indices,
+                       double* S, int64_t ni, int topn, int64_t* out_ids, double* out_scores, cudaStream_t st);
 
 bool score_tc_supported(int64_t ni, int f, int bias, int topn);
 size_t score_tc_workspace_bytes(int64_t nu, int64_t ni);

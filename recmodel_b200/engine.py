@@ -630,3 +630,27 @@ def ease_predict(csr, W, users, items):
     _lib.check(lib.wmf_ease_predict(_ptr(csr.indptr), _ptr(csr.indices), _ptr(csr.data), _ptr(W), W.shape[0], _ptr(users), stride,
                                     _ptr(items), n, _ptr(out), _stream()), "wmf_ease_predict")
     return out
+
+
+@_device_of(1)
+def ease_score_topk(X_csr, W, users, topn, exclude=None, want_scores=False):
+    """Top-``topn`` item ids [nu x topn] (int64) of the EASE scores sum_j X[user, j] W[j, item] (float64, bitwise those
+    of ``ease_predict``) for each user in ``users`` over all items minus the stored entries of row ``users[k]`` of
+    ``exclude`` (a DeviceCSR indexed by user id, any row order, or None), best first, ties to the lower item id, -1
+    where a user has fewer unseen items (include/wmf_b200.h: wmf_ease_score_topk). With ``want_scores`` returns
+    (ids, float64 scores, NaN at the -1 entries)."""
+    lib = _lib.load()
+    _f32(W)
+    n = W.shape[0]
+    nu = users.numel()
+    assert users.dtype == torch.int64 and X_csr.shape[1] == n
+    if exclude is not None:
+        assert exclude.shape[1] == n and exclude.indices.dtype == torch.int32 and exclude.indptr.dtype == torch.int64
+    ids = torch.empty((nu, topn), dtype=torch.int64, device=W.device)
+    scores = torch.empty((nu, topn), dtype=torch.float64, device=W.device) if want_scores else None
+    ws = workspace(lib.wmf_ease_score_topk_workspace_bytes(nu, n, topn), W.device)
+    _lib.check(lib.wmf_ease_score_topk(_ptr(X_csr.indptr), _ptr(X_csr.indices), _ptr(X_csr.data), _ptr(W), n,
+                                       _ptr(users), nu, _ptr(None if exclude is None else exclude.indptr),
+                                       _ptr(None if exclude is None else exclude.indices), int(topn), _ptr(ids),
+                                       _ptr(scores), _ptr(ws), ws.numel(), _stream()), "wmf_ease_score_topk")
+    return (ids, scores) if want_scores else ids

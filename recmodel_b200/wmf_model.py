@@ -18,13 +18,13 @@ import time
 import numpy as np
 import torch
 
-from . import _lib, engine, sharding
+from . import _lib, engine, ranking, sharding
 from .base_model import RecModel
 from .engine import DeviceCSR
 
 _ALGOS = {"auto": _lib.ALGO_AUTO, "simt": _lib.ALGO_SIMT, "tcgen05": _lib.ALGO_TCGEN05,
           "tcgen05_direct": _lib.ALGO_TCGEN05_DIRECT}
-_EVAL_CHUNK_IDS = 1 << 25  # eval_ranking ranks users in chunks of at most this many list entries (32 M ids, 256 MB)
+_EVAL_CHUNK_IDS = ranking.EVAL_CHUNK_IDS
 
 
 class WMF(RecModel):
@@ -221,30 +221,9 @@ class WMF(RecModel):
             return ids[:users_d.numel()]
         if k <= _lib.TOPK_MAX:
             return topk(users_d)
-        # very long lists: exact device scores, excluded entries masked, then stable device sorts
-        rows = []
-        per = max(1, (1 << 24) // ni)
-        items_d = torch.arange(ni, dtype=torch.int64, device=self.device)
-        for u0 in range(0, users_d.numel(), per):
-            chunk = users_d[u0:u0 + per]
-            n = chunk.numel()
-            s = engine.predict_pairs(chunk.repeat_interleave(ni), items_d.repeat(n), U, V, bias=bias).view(n, ni)
-            order = torch.sort(s, dim=1, descending=True, stable=True).indices
-            if ex is None:
-                rows.append(order[:, :k])
-                continue
-            lo, cnt = ex.indptr[chunk], ex.indptr[chunk + 1] - ex.indptr[chunk]
-            total = int(cnt.sum())
-            row = torch.repeat_interleave(torch.arange(n, device=self.device), cnt, output_size=total)
-            entry = torch.arange(total, device=self.device) + torch.repeat_interleave(lo - (torch.cumsum(cnt, 0) - cnt),
-                                                                                     cnt, output_size=total)
-            seen = torch.zeros((n, ni), dtype=torch.bool, device=self.device)
-            seen[row, ex.indices[entry].long()] = True
-            # unseen first, each group in score order (a seen item never displaces an unseen one, whatever the scores)
-            seen_sorted = seen.gather(1, order)
-            regroup = torch.sort(seen_sorted.to(torch.uint8), dim=1, stable=True).indices[:, :k]
-            rows.append(torch.where(seen_sorted.gather(1, regroup), -1, order.gather(1, regroup)))
-        return torch.cat(rows) if rows else torch.empty((0, k), dtype=torch.int64, device=self.device)
+        # very long lists: exact device scores, then stable device sorts with the excluded entries regrouped last
+        return ranking.sort_path_ids(users_d, ni, k, ex, lambda chunk, items_d: engine.predict_pairs(
+            chunk.repeat_interleave(ni), items_d.repeat(chunk.numel()), U, V, bias=bias).view(chunk.numel(), ni))
 
     def eval_ranking(self, test_mat, topn=np.array([10]), exclude=None, users=None, distributed=False):
         """Full-ranking quality of ``recommend``: for each cutoff k of ``topn`` (an int or at most 16 distinct positive
@@ -265,62 +244,10 @@ class WMF(RecModel):
         Lists, metrics and their sums stay on the device (the per-user rows are reduced once, in a fixed order: the
         result is bitwise reproducible). ``distributed=True`` is a collective like in ``recommend``: every rank gets
         the same result, bitwise equal to the local call."""
-        ks = np.asarray(topn)
-        if ks.ndim == 0:
-            ks = ks.reshape(1)
-        if (ks.ndim != 1 or not 1 <= len(ks) <= 16 or not np.issubdtype(ks.dtype, np.integer) or ks.min() < 1
-                or len(np.unique(ks)) != len(ks)):
-            raise ValueError("topn must be an int or a 1-D sequence of at most 16 distinct positive ints")
-        ks = ks.astype(np.int64)
-        V, U = self.items_device, self.users_device
-        ni = V.shape[0]
-        if test_mat.shape[1] != ni:
-            raise ValueError(f"test_mat has {test_mat.shape[1]} columns but the model has {ni} items")
-        if exclude is not None and tuple(exclude.shape) != tuple(test_mat.shape):
-            raise ValueError(f"exclude has shape {tuple(exclude.shape)}, test_mat {tuple(test_mat.shape)}")
-        n_ok = min(test_mat.shape[0], U.shape[0])
-        bad_users = ValueError(f"user ids must lie in [0, {n_ok}) (the rows of test_mat and of the user factors)")
-        if users is not None:
-            users = np.ascontiguousarray(users, dtype=np.int64).reshape(-1)
-            if len(users) and (users.min() < 0 or users.max() >= n_ok):
-                raise bad_users
-        dev = self.device
-        T = (test_mat if isinstance(test_mat, DeviceCSR) else DeviceCSR.from_scipy(test_mat, dev)).sorted()
-        ex = None
-        if exclude is not None:
-            ex = (exclude if isinstance(exclude, DeviceCSR) else DeviceCSR.from_scipy(exclude, dev)).sorted()
-        if users is None:
-            users_d = torch.nonzero(T.indptr[1:] > T.indptr[:-1]).squeeze(1)
-            if users_d.numel() and int(users_d[-1]) >= n_ok:
-                raise bad_users
-        else:
-            users_d = torch.from_numpy(users).to(dev)
-        sums = self._eval_ranking_sums(T, ex, users_d, ks, distributed).cpu().numpy()
-        count = int(sums[-1])
-        out = {}
-        for j, kk in enumerate(ks.tolist()):
-            for m, name in enumerate(engine.TOPN_METRICS):
-                out[f"{name}@{kk}"] = float(sums[j * 5 + m] / count) if count else float("nan")
-        out["users"] = count
-        return out
-
-    def _eval_ranking_sums(self, T, ex, users_d, ks, distributed=False):
-        """The device part of ``eval_ranking`` (T, ex: DeviceCSRs with sorted rows, ex may be None): the users are ranked
-        in chunks of at most ``_EVAL_CHUNK_IDS`` list entries, each chunk's per-user metrics land in one buffer, and one
-        reduce returns the device float64 [len(ks)*5 + 1] sums and the evaluated-user count. No ids leave the device."""
-        dev = self.device
-        K = int(max(ks))
-        k = min(K, self.items_device.shape[0])
-        n = users_d.numel()
-        per_user = torch.empty((n, len(ks), 5), dtype=torch.float64, device=dev)
-        chunk = max(1, _EVAL_CHUNK_IDS // K)
-        for u0 in range(0, n, chunk):
-            part = users_d[u0:u0 + chunk]
-            ids = self._recommend_ids(part, k, ex, distributed)
-            if k < K:  # cutoffs past the number of items: -1 padding, as recommend returns it
-                ids = torch.cat((ids, torch.full((part.numel(), K - k), -1, dtype=torch.int64, device=dev)), dim=1)
-            engine.topn_metrics(ids, part, T, ks, out=per_user[u0:u0 + chunk])
-        return engine.topn_metrics_reduce(per_user, len(ks))
+        return ranking.eval_ranking(
+            lambda users_d, k, ex: self._recommend_ids(users_d, k, None if ex is None else ex.sorted(), distributed),
+            lambda: (self.items_device.shape[0], self.users_device.shape[0]),
+            "the rows of test_mat and of the user factors", self.device, test_mat, topn, exclude, users, _EVAL_CHUNK_IDS)
 
     # ---------------------------------------------------------------- train (R2, R7, R11)
     def train(self, utility_mat, iterations, verbose=0, eval_mat=None, count_mat=None, alpha=10,

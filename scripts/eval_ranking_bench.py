@@ -24,7 +24,7 @@ import numpy as np
 import torch
 
 from recommend_bench import gpu_info
-from recmodel_b200 import WMF, engine, utils
+from recmodel_b200 import WMF, engine, ranking, utils
 from recmodel_b200.engine import DeviceCSR
 from recmodel_b200.synthetic import make_counts_cached
 
@@ -83,7 +83,7 @@ def main():
     ids_d = m._recommend_ids(users_d, K, ex)
 
     def device_path():
-        return m._eval_ranking_sums(T, ex, users_d, KS)
+        return ranking.eval_ranking_sums(lambda u, k, e: m._recommend_ids(u, k, e), ITEMS, T, ex, users_d, KS)
 
     def metrics_only():
         return engine.topn_metrics_reduce(engine.topn_metrics(ids_d, users_d, T, KS), len(KS))
