@@ -261,6 +261,44 @@ int wmf_ease_score_topk(const int64_t* x_indptr, const int32_t* x_indices, const
                         const int32_t* ex_indices, int topn, int64_t* out_ids, double* out_scores, void* ws,
                         size_t ws_bytes, void* stream);
 
+/* ItemKNN: an item-item neighbourhood model (DESIGN.md 4.6). No reference call site: the neighbourhood sources of
+ * RecModel are not part of this repository, and this model is defined here, not ported.
+ * X is the `rows` x n interaction matrix in canonical CSR: sorted column indices, no duplicates, no explicit zeros
+ * (duplicates would count twice; scores walk each row in stored order). P is its binary pattern and
+ * c_ab = sum_u P[u, a] P[u, b], an exact integer; c_aa is the number of users of a.
+ * wmf_knn_train: sim(a, b) in double, every operation rounded to nearest, no fused multiply-add:
+ *   WMF_KNN_COSINE       c_ab / (sqrt(c_aa) * sqrt(c_bb) + shrink)
+ *   WMF_KNN_JACCARD      c_ab / ((c_aa + c_bb - c_ab) + shrink)
+ *   WMF_KNN_CONDITIONAL  c_ab / (c_aa + shrink)            (P(b | a): W is not symmetric)
+ * Row a of W holds the top-min(k, n) items b != a with c_ab > 0 by sim(a, b), ties to the lower id, fewer when a has
+ * fewer such items; W[a, b] = sim(a, b). W is written as an n x n CSR with sorted column indices: w_indptr [n+1], and
+ * w_indices / w_data with room for n * min(k, n) entries, of which the first w_indptr[n] are used. xt_indptr /
+ * xt_indices: the CSR of X^T (wmf_csr_transpose). 1 <= k <= 1024, similarity one of WMF_KNN_*, shrink finite and
+ * >= 0, 0 < n < 2^31: else WMF_ERR_INVALID before any CUDA call. The workspace holds an int32 and a double [B x n]
+ * tile (B item rows from n and a fixed byte budget) and the selected rows of all n items.
+ * wmf_knn_predict: out[k] = s(users[k*user_stride], items[k]); user_stride 0 broadcasts one user. The score
+ * s(u, i) is the sum over the entries j of row u of X, in ascending j, from +0.0, of (double)x_uj * W[j, i], each
+ * product and each addition rounded to nearest; an item no entry of W votes for scores +0.0. W is any n x n CSR
+ * with sorted column indices (w_data double).
+ * wmf_knn_score_topk: wmf_ease_score_topk's contract (exclusion CSR, ordering, -1 / NaN padding, 1 <= topn <=
+ * min(n, 1024) else WMF_ERR_UNSUPPORTED) with the scores of wmf_knn_predict, bitwise. The workspace holds one
+ * [ub x n] double score tile. */
+#define WMF_KNN_COSINE 0
+#define WMF_KNN_JACCARD 1
+#define WMF_KNN_CONDITIONAL 2
+size_t wmf_knn_train_workspace_bytes(int64_t n, int k);
+int wmf_knn_train(const int64_t* x_indptr, const int32_t* x_indices, int64_t rows, const int64_t* xt_indptr,
+                  const int32_t* xt_indices, int64_t n, int k, int similarity, double shrink, int64_t* w_indptr,
+                  int32_t* w_indices, double* w_data, void* ws, size_t ws_bytes, void* stream);
+int wmf_knn_predict(const int64_t* x_indptr, const int32_t* x_indices, const float* x_data, const int64_t* w_indptr,
+                    const int32_t* w_indices, const double* w_data, const int64_t* users, int64_t user_stride,
+                    const int64_t* items, int64_t count, double* out, void* stream);
+size_t wmf_knn_score_topk_workspace_bytes(int64_t nu, int64_t n, int topn);
+int wmf_knn_score_topk(const int64_t* x_indptr, const int32_t* x_indices, const float* x_data, const int64_t* w_indptr,
+                       const int32_t* w_indices, const double* w_data, int64_t n, const int64_t* users, int64_t nu,
+                       const int64_t* ex_indptr, const int32_t* ex_indices, int topn, int64_t* out_ids,
+                       double* out_scores, void* ws, size_t ws_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

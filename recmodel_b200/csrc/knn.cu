@@ -1,0 +1,348 @@
+// ItemKNN: an item-item neighbourhood model (DESIGN.md 4.6). For the users x n binary pattern P of the canonical X:
+//   c_ab = sum_u P[u, a] P[u, b]                          -> knn_cooc_kernel (int32 counts, [B x n] tile per item block)
+//   sim(a, b) from c_ab, c_aa, c_bb, shrink                -> knn_similarity_kernel (double, no FMA contraction)
+//   W[a, :] = top-k of sim(a, b), b != a, c_ab > 0          -> topk_rows_kernel<double> (score.cu), knn_sort_rows_kernel
+//   s(u, i) = sum over j of row u, ascending, of x_uj W[j, i] -> knn_score_tile_kernel (recommend), knn_predict_kernel
+// Every double operation is an explicit round-to-nearest intrinsic, so a NumPy restatement of the definitions
+// reproduces each similarity and each score bitwise.
+#include "common.cuh"
+#include "score.cuh"
+
+namespace wmf {
+
+namespace {
+
+constexpr int KN_THREADS = 256;
+constexpr size_t KN_TILE_BYTES = 64ull << 20;   // double tiles near 64 MiB: the selection passes stay in L2 (126 MB)
+
+__device__ __forceinline__ double knn_pop(const int64_t* __restrict__ xt_indptr, int64_t a) {
+    return (double)(xt_indptr[a + 1] - xt_indptr[a]);
+}
+
+// C[a - a0][j] += 1 for every stored entry (a, u) of rows [a0, a0 + B) of X^T and every stored entry j of row u of X.
+// One warp per (a, u) entry, flattened over the block so that a popular item spreads over many warps; lanes over row
+// u. The integer atomics make the counts independent of the order.
+__global__ __launch_bounds__(KN_THREADS) void knn_cooc_kernel(const int64_t* __restrict__ x_indptr,
+                                                              const int32_t* __restrict__ x_indices,
+                                                              const int64_t* __restrict__ xt_indptr,
+                                                              const int32_t* __restrict__ xt_indices, int64_t n,
+                                                              int64_t a0, int B, int* __restrict__ C) {
+    const int64_t base = xt_indptr[a0], cnt = xt_indptr[a0 + B] - base;
+    const int lane = threadIdx.x & 31;
+    const int64_t warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    for (int64_t w = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; w < cnt; w += warps) {
+        const int64_t e = base + w;
+        int lo = 0, hi = B - 1;   // the block row holding entry e: the last r with xt_indptr[a0 + r] <= e
+        while (lo < hi) {
+            const int mid = (lo + hi + 1) >> 1;
+            if (xt_indptr[a0 + mid] <= e) lo = mid; else hi = mid - 1;
+        }
+        const int64_t u = xt_indices[e];
+        int* crow = C + (int64_t)lo * n;
+        for (int64_t t = x_indptr[u] + lane; t < x_indptr[u + 1]; t += 32) atomicAdd(crow + x_indices[t], 1);
+    }
+}
+
+// S[r][b] = sim(a0 + r, b) from the counts; self and c_ab = 0 get RankKey<double>::excluded(). c_bb is the column
+// count of X (X^T row length): the canonical X stores each (u, b) once.
+__global__ __launch_bounds__(KN_THREADS) void knn_similarity_kernel(const int* __restrict__ C,
+                                                                    const int64_t* __restrict__ xt_indptr, int64_t n,
+                                                                    int64_t a0, int sim, double shrink,
+                                                                    double* __restrict__ S) {
+    const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= n) return;
+    const int64_t r = blockIdx.y, a = a0 + r, e = r * n + b;
+    const int c = C[e];
+    double s = RankKey<double>::excluded();
+    if (c != 0 && b != a) {
+        const double cab = (double)c, caa = knn_pop(xt_indptr, a), cbb = knn_pop(xt_indptr, b);
+        double den;
+        if (sim == WMF_KNN_COSINE) den = __dadd_rn(__dmul_rn(__dsqrt_rn(caa), __dsqrt_rn(cbb)), shrink);
+        else if (sim == WMF_KNN_JACCARD) den = __dadd_rn(__dsub_rn(__dadd_rn(caa, cbb), cab), shrink);
+        else den = __dadd_rn(caa, shrink);
+        s = __ddiv_rn(cab, den);
+    }
+    S[e] = s;
+}
+
+// One CTA per block row: the selected (id, similarity) pairs (ids -1 where the row had fewer than kk candidates)
+// sorted by id into row a0 + r of the [n x kk] staging area; cnt[a0 + r] = their number. The rank of an entry is the
+// number of selected ids below it (ids are distinct).
+__global__ __launch_bounds__(KN_THREADS) void knn_sort_rows_kernel(const int64_t* __restrict__ ids,
+                                                                   const double* __restrict__ vals, int kk, int64_t a0,
+                                                                   int32_t* __restrict__ st_idx,
+                                                                   double* __restrict__ st_val,
+                                                                   int64_t* __restrict__ cnt) {
+    __shared__ int32_t sid[TK_MAX];
+    __shared__ unsigned s_m;
+    const int64_t r = blockIdx.x, row = a0 + r;
+    if (threadIdx.x == 0) s_m = 0;
+    __syncthreads();
+    for (int t = threadIdx.x; t < kk; t += KN_THREADS) {
+        const int32_t id = (int32_t)ids[r * kk + t];
+        sid[t] = id;
+        if (id >= 0) atomicAdd(&s_m, 1u);
+    }
+    __syncthreads();
+    for (int t = threadIdx.x; t < kk; t += KN_THREADS) {
+        const int32_t id = sid[t];
+        if (id < 0) continue;
+        int pos = 0;
+        for (int q = 0; q < kk; ++q) pos += (sid[q] >= 0 && sid[q] < id);
+        st_idx[row * kk + pos] = id;
+        st_val[row * kk + pos] = vals[r * kk + t];
+    }
+    if (threadIdx.x == 0) cnt[row] = s_m;
+}
+
+// indptr[0] = 0, indptr[a + 1] = cnt[0] + ... + cnt[a]: one CTA, chunks of KN_THREADS rows
+__global__ __launch_bounds__(KN_THREADS) void knn_scan_kernel(const int64_t* __restrict__ cnt, int64_t n,
+                                                              int64_t* __restrict__ indptr) {
+    __shared__ int64_t warp_tot[KN_THREADS / 32];
+    __shared__ int64_t s_carry;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    if (tid == 0) { s_carry = 0; indptr[0] = 0; }
+    __syncthreads();
+    for (int64_t c0 = 0; c0 < n; c0 += KN_THREADS) {
+        const int64_t a = c0 + tid;
+        int64_t v = a < n ? cnt[a] : 0;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int64_t y = __shfl_up_sync(0xffffffffu, v, o);
+            if (lane >= o) v += y;
+        }
+        if (lane == 31) warp_tot[warp] = v;
+        __syncthreads();
+        int64_t before = s_carry;
+        for (int w = 0; w < warp; ++w) before += warp_tot[w];
+        if (a < n) indptr[a + 1] = before + v;
+        __syncthreads();
+        if (tid == KN_THREADS - 1) s_carry = before + v;
+        __syncthreads();
+    }
+}
+
+// the staged rows into the CSR: one warp per row
+__global__ __launch_bounds__(KN_THREADS) void knn_compact_kernel(const int32_t* __restrict__ st_idx,
+                                                                 const double* __restrict__ st_val, int kk, int64_t n,
+                                                                 const int64_t* __restrict__ indptr,
+                                                                 int32_t* __restrict__ w_indices,
+                                                                 double* __restrict__ w_data) {
+    const int64_t a = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (a >= n) return;
+    const int lane = threadIdx.x & 31;
+    const int64_t lo = indptr[a], m = indptr[a + 1] - lo;
+    for (int64_t t = lane; t < m; t += 32) {
+        w_indices[lo + t] = st_idx[a * kk + t];
+        w_data[lo + t] = st_val[a * kk + t];
+    }
+}
+
+// S[r][i] = s(users[u_begin + r], i) on a zeroed [ub x n] tile. One warp per user walks row u of X in ascending j
+// (32 entries and their W row bounds fetched at once, then broadcast); lanes over the entries of W row j, which are
+// distinct ids. The __syncwarp between rows j orders the read-modify-writes of one item, so every score is summed
+// from +0.0 in ascending j without atomics: the sum of knn_predict_kernel.
+__global__ __launch_bounds__(KN_THREADS) void knn_score_tile_kernel(
+    const int64_t* __restrict__ x_indptr, const int32_t* __restrict__ x_indices, const float* __restrict__ x_data,
+    const int64_t* __restrict__ w_indptr, const int32_t* __restrict__ w_indices, const double* __restrict__ w_data,
+    int64_t n, const int64_t* __restrict__ users, int64_t u_begin, int ub, double* S) {
+    const int64_t r = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (r >= ub) return;
+    const int lane = threadIdx.x & 31;
+    const int64_t u = users[u_begin + r];
+    const int64_t hi = x_indptr[u + 1];
+    double* srow = S + r * n;
+    for (int64_t e0 = x_indptr[u]; e0 < hi; e0 += 32) {
+        double x = 0.0;
+        int64_t wlo = 0, whi = 0;
+        if (e0 + lane < hi) {
+            const int32_t j = x_indices[e0 + lane];
+            x = (double)x_data[e0 + lane];
+            wlo = w_indptr[j];
+            whi = w_indptr[j + 1];
+        }
+        const int m = (int)(hi - e0 < 32 ? hi - e0 : 32);
+        for (int q = 0; q < m; ++q) {
+            const double xq = __shfl_sync(0xffffffffu, x, q);
+            const int64_t lo = __shfl_sync(0xffffffffu, wlo, q), end = __shfl_sync(0xffffffffu, whi, q);
+            for (int64_t t = lo + lane; t < end; t += 32) {
+                const int32_t i = w_indices[t];
+                srow[i] = __dadd_rn(srow[i], __dmul_rn(xq, w_data[t]));
+            }
+            __syncwarp();
+        }
+    }
+}
+
+// out[k] = s(users[k * user_stride], items[k]): row u of X in ascending j, a binary search of the item in W row j
+__global__ __launch_bounds__(KN_THREADS) void knn_predict_kernel(
+    const int64_t* __restrict__ x_indptr, const int32_t* __restrict__ x_indices, const float* __restrict__ x_data,
+    const int64_t* __restrict__ w_indptr, const int32_t* __restrict__ w_indices, const double* __restrict__ w_data,
+    const int64_t* __restrict__ users, int64_t user_stride, const int64_t* __restrict__ items, int64_t count,
+    double* __restrict__ out) {
+    const int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= count) return;
+    const int64_t u = users[k * user_stride];
+    const int32_t it = (int32_t)items[k];
+    double acc = 0.0;
+    for (int64_t e = x_indptr[u]; e < x_indptr[u + 1]; ++e) {
+        const int32_t j = x_indices[e];
+        int64_t lo = w_indptr[j], hi = w_indptr[j + 1];   // first entry >= it
+        while (lo < hi) {
+            const int64_t mid = (lo + hi) >> 1;
+            if (w_indices[mid] < it) lo = mid + 1; else hi = mid;
+        }
+        if (lo < w_indptr[j + 1] && w_indices[lo] == it) acc = __dadd_rn(acc, __dmul_rn((double)x_data[e], w_data[lo]));
+    }
+    out[k] = acc;
+}
+
+// rows per [B x n] similarity tile (and users per score tile): the double tile near KN_TILE_BYTES, at least one row
+int64_t knn_batch(int64_t rows, int64_t n) {
+    int64_t b = (int64_t)(KN_TILE_BYTES / ((size_t)n * 8));
+    if (b < 1) b = 1;
+    if (b > rows) b = rows;
+    return b;
+}
+
+struct TrainLayout {
+    size_t C, S, ids, vals, st_idx, st_val, cnt, total;
+};
+
+TrainLayout train_layout(int64_t n, int kk) {
+    const size_t B = (size_t)knn_batch(n, n);
+    TrainLayout L;
+    size_t off = 0;
+    auto take = [&](size_t bytes) { const size_t at = off; off += align_up(bytes, 256); return at; };
+    L.C = take(B * n * 4);
+    L.S = take(B * n * 8);
+    L.ids = take(B * kk * 8);
+    L.vals = take(B * kk * 8);
+    L.st_idx = take((size_t)n * kk * 4);
+    L.st_val = take((size_t)n * kk * 8);
+    L.cnt = take((size_t)n * 8);
+    L.total = off;
+    return L;
+}
+
+int check_knn_args(const char* name, int64_t n, int k, int similarity, double shrink) {
+    WMF_REQUIRE(n > 0 && n < (1ll << 31), "%s: n=%lld outside 1..2^31-1", name, (long long)n);
+    WMF_REQUIRE(k >= 1 && k <= TK_MAX, "%s: k=%d outside 1..%d", name, k, TK_MAX);
+    WMF_REQUIRE(similarity == WMF_KNN_COSINE || similarity == WMF_KNN_JACCARD || similarity == WMF_KNN_CONDITIONAL,
+                "%s: unknown similarity %d", name, similarity);
+    WMF_REQUIRE(shrink >= 0.0 && shrink <= 1.7976931348623157e308, "%s: shrink=%g is not finite and >= 0", name, shrink);
+    return WMF_OK;
+}
+
+}  // namespace
+
+}  // namespace wmf
+
+using namespace wmf;
+
+extern "C" {
+
+size_t wmf_knn_train_workspace_bytes(int64_t n, int k) {
+    if (n <= 0 || n >= (1ll << 31) || k < 1 || k > TK_MAX) return 0;
+    return train_layout(n, (int)(k < n ? k : n)).total;
+}
+
+int wmf_knn_train(const int64_t* x_indptr, const int32_t* x_indices, int64_t rows, const int64_t* xt_indptr,
+                  const int32_t* xt_indices, int64_t n, int k, int similarity, double shrink, int64_t* w_indptr,
+                  int32_t* w_indices, double* w_data, void* ws, size_t ws_bytes, void* stream) {
+    if (int rc = check_knn_args("wmf_knn_train", n, k, similarity, shrink)) return rc;
+    WMF_REQUIRE(rows >= 0, "wmf_knn_train: rows=%lld < 0", (long long)rows);
+    WMF_REQUIRE(x_indptr && xt_indptr && w_indptr && w_indices && w_data, "wmf_knn_train: null argument");
+    const size_t need = wmf_knn_train_workspace_bytes(n, k);
+    if (ws == nullptr || ws_bytes < need) {
+        set_error("wmf_knn_train: workspace %zu < %zu", ws_bytes, need);
+        return WMF_ERR_WORKSPACE;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    const int kk = (int)(k < n ? k : n);
+    const TrainLayout L = train_layout(n, kk);
+    char* base = reinterpret_cast<char*>(ws);
+    int* C = reinterpret_cast<int*>(base + L.C);
+    double* S = reinterpret_cast<double*>(base + L.S);
+    int64_t* ids = reinterpret_cast<int64_t*>(base + L.ids);
+    double* vals = reinterpret_cast<double*>(base + L.vals);
+    int32_t* st_idx = reinterpret_cast<int32_t*>(base + L.st_idx);
+    double* st_val = reinterpret_cast<double*>(base + L.st_val);
+    int64_t* cnt = reinterpret_cast<int64_t*>(base + L.cnt);
+    const int64_t bmax = knn_batch(n, n);
+    const unsigned cooc_grid = (unsigned)sm_count() * 8;
+    for (int64_t a0 = 0; a0 < n; a0 += bmax) {
+        const int B = (int)(n - a0 < bmax ? n - a0 : bmax);
+        WMF_CUDA(cudaMemsetAsync(C, 0, (size_t)B * n * 4, st));
+        if (rows > 0) {
+            knn_cooc_kernel<<<cooc_grid, KN_THREADS, 0, st>>>(x_indptr, x_indices, xt_indptr, xt_indices, n, a0, B, C);
+            WMF_LAUNCH_CHECK("knn_cooc_kernel");
+        }
+        knn_similarity_kernel<<<dim3((unsigned)((n + KN_THREADS - 1) / KN_THREADS), (unsigned)B), KN_THREADS, 0, st>>>(
+            C, xt_indptr, n, a0, similarity, shrink, S);
+        WMF_LAUNCH_CHECK("knn_similarity_kernel");
+        const int rc = select_topk_double(nullptr, 0, B, nullptr, nullptr, S, n, kk, ids, vals, st, true);
+        if (rc) return rc;
+        knn_sort_rows_kernel<<<(unsigned)B, KN_THREADS, 0, st>>>(ids, vals, kk, a0, st_idx, st_val, cnt);
+        WMF_LAUNCH_CHECK("knn_sort_rows_kernel");
+    }
+    knn_scan_kernel<<<1, KN_THREADS, 0, st>>>(cnt, n, w_indptr);
+    WMF_LAUNCH_CHECK("knn_scan_kernel");
+    knn_compact_kernel<<<(unsigned)((n + KN_THREADS / 32 - 1) / (KN_THREADS / 32)), KN_THREADS, 0, st>>>(
+        st_idx, st_val, kk, n, w_indptr, w_indices, w_data);
+    WMF_LAUNCH_CHECK("knn_compact_kernel");
+    return WMF_OK;
+}
+
+int wmf_knn_predict(const int64_t* x_indptr, const int32_t* x_indices, const float* x_data, const int64_t* w_indptr,
+                    const int32_t* w_indices, const double* w_data, const int64_t* users, int64_t user_stride,
+                    const int64_t* items, int64_t count, double* out, void* stream) {
+    WMF_REQUIRE(count >= 0 && user_stride >= 0, "wmf_knn_predict: bad arguments");
+    if (count == 0) return WMF_OK;
+    WMF_REQUIRE(x_indptr && w_indptr && users && items && out, "wmf_knn_predict: null argument");
+    knn_predict_kernel<<<(unsigned)((count + KN_THREADS - 1) / KN_THREADS), KN_THREADS, 0, (cudaStream_t)stream>>>(
+        x_indptr, x_indices, x_data, w_indptr, w_indices, w_data, users, user_stride, items, count, out);
+    WMF_LAUNCH_CHECK("knn_predict_kernel");
+    return WMF_OK;
+}
+
+size_t wmf_knn_score_topk_workspace_bytes(int64_t nu, int64_t n, int topn) {
+    (void)topn;
+    if (nu <= 0 || n <= 0 || n >= (1ll << 31)) return 0;
+    return align_up((size_t)knn_batch(nu, n) * (size_t)n * sizeof(double), 1024);
+}
+
+int wmf_knn_score_topk(const int64_t* x_indptr, const int32_t* x_indices, const float* x_data, const int64_t* w_indptr,
+                       const int32_t* w_indices, const double* w_data, int64_t n, const int64_t* users, int64_t nu,
+                       const int64_t* ex_indptr, const int32_t* ex_indices, int topn, int64_t* out_ids,
+                       double* out_scores, void* ws, size_t ws_bytes, void* stream) {
+    WMF_REQUIRE(n > 0 && n < (1ll << 31), "wmf_knn_score_topk: n=%lld outside 1..2^31-1", (long long)n);
+    WMF_REQUIRE(nu >= 0, "wmf_knn_score_topk: nu=%lld < 0", (long long)nu);
+    if (topn < 1 || topn > n || topn > TK_MAX) {
+        set_error("wmf_knn_score_topk: topn=%d outside 1..min(n=%lld, %d)", topn, (long long)n, TK_MAX);
+        return WMF_ERR_UNSUPPORTED;
+    }
+    if (nu == 0) return WMF_OK;
+    WMF_REQUIRE(x_indptr && w_indptr && users && out_ids, "wmf_knn_score_topk: null argument");
+    const size_t need = wmf_knn_score_topk_workspace_bytes(nu, n, topn);
+    if (ws == nullptr || ws_bytes < need) {
+        set_error("wmf_knn_score_topk: workspace %zu < %zu", ws_bytes, need);
+        return WMF_ERR_WORKSPACE;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    const int64_t ubatch = knn_batch(nu, n);
+    double* S = (double*)ws;
+    for (int64_t u0 = 0; u0 < nu; u0 += ubatch) {
+        const int ub = (int)((nu - u0) < ubatch ? (nu - u0) : ubatch);
+        WMF_CUDA(cudaMemsetAsync(S, 0, (size_t)ub * n * sizeof(double), st));
+        knn_score_tile_kernel<<<(unsigned)((ub + KN_THREADS / 32 - 1) / (KN_THREADS / 32)), KN_THREADS, 0, st>>>(
+            x_indptr, x_indices, x_data, w_indptr, w_indices, w_data, n, users, u0, ub, S);
+        WMF_LAUNCH_CHECK("knn_score_tile_kernel");
+        const int rc = select_topk_double(users, u0, ub, ex_indptr, ex_indices, S, n, topn, out_ids + (size_t)u0 * topn,
+                                          out_scores ? out_scores + (size_t)u0 * topn : nullptr, st);
+        if (rc) return rc;
+    }
+    return WMF_OK;
+}
+
+}  // extern "C"

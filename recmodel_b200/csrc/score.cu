@@ -270,14 +270,15 @@ __global__ __launch_bounds__(TK_THREADS) void topk_rows_kernel(const T* __restri
 }
 
 int select_topk_double(const int64_t* users, int64_t u_begin, int ub, const int64_t* ex_indptr, const int32_t* ex_indices,
-                       double* S, int64_t ni, int topn, int64_t* out_ids, double* out_scores, cudaStream_t st) {
+                       double* S, int64_t ni, int topn, int64_t* out_ids, double* out_scores, cudaStream_t st,
+                       bool marked) {
     if (ex_indptr) {
         score_exclude_kernel<double><<<(unsigned)(ub < 65535 ? ub : 65535), 256, 0, st>>>(users, u_begin, ub, ex_indptr,
                                                                                            ex_indices, ni, S, nullptr);
         WMF_LAUNCH_CHECK("score_exclude_kernel<double>");
     }
     topk_rows_kernel<double><<<ub, TK_THREADS, 0, st>>>(S, ni, topn, nullptr, out_ids, out_scores, nullptr,
-                                                        ex_indptr != nullptr);
+                                                        ex_indptr != nullptr || marked);
     WMF_LAUNCH_CHECK("topk_rows_kernel<double>");
     return WMF_OK;
 }

@@ -1,4 +1,5 @@
-// Shared by the exact (score.cu) and tensor-core (score_tc.cu) ranking paths, and by the EASE ranking (ease.cu).
+// Shared by the exact (score.cu) and tensor-core (score_tc.cu) ranking paths, and by the EASE (ease.cu) and ItemKNN
+// (knn.cu) models.
 #pragma once
 #include "common.cuh"
 
@@ -52,9 +53,12 @@ template <> struct RankKey<double> {
 
 // Exact selection over a [ub x ni] tile of double scores S (row r: user users[u_begin + r]), the kernels of the exact
 // ranking path instantiated for double (score.cu). ex_indptr (nullable) / ex_indices: the exclusion CSR by user id.
-// out_ids / out_scores (nullable) [ub x topn]; topn in 1..min(ni, TK_MAX).
+// out_ids / out_scores (nullable) [ub x topn]; topn in 1..min(ni, TK_MAX). `marked`: S already holds
+// RankKey<double>::excluded() entries of its own (users may then be null when ex_indptr is), which, like excluded
+// items, are reported as id -1 when a row has fewer than topn other entries.
 int select_topk_double(const int64_t* users, int64_t u_begin, int ub, const int64_t* ex_indptr, const int32_t* ex_indices,
-                       double* S, int64_t ni, int topn, int64_t* out_ids, double* out_scores, cudaStream_t st);
+                       double* S, int64_t ni, int topn, int64_t* out_ids, double* out_scores, cudaStream_t st,
+                       bool marked = false);
 
 bool score_tc_supported(int64_t ni, int f, int bias, int topn);
 size_t score_tc_workspace_bytes(int64_t nu, int64_t ni);

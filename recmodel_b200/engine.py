@@ -654,3 +654,69 @@ def ease_score_topk(X_csr, W, users, topn, exclude=None, want_scores=False):
                                        _ptr(None if exclude is None else exclude.indices), int(topn), _ptr(ids),
                                        _ptr(scores), _ptr(ws), ws.numel(), _stream()), "wmf_ease_score_topk")
     return (ids, scores) if want_scores else ids
+
+
+@_device_of(0)
+def knn_train(X_csr, XT_csr, k, similarity, shrink):
+    """The ItemKNN neighbours of the canonical interaction matrix ``X_csr`` (sorted rows, no duplicates, no explicit
+    zeros; ``XT_csr`` its transpose): (indptr int64 [n+1], indices int32, data float64) of the n x n CSR W, rows
+    sorted by id (include/wmf_b200.h: wmf_knn_train). ``similarity``: a key of ``_lib.KNN_SIMILARITIES``."""
+    lib = _lib.load()
+    n = X_csr.shape[1]
+    dev = X_csr.device
+    kk = min(int(k), n)
+    indptr = torch.empty(n + 1, dtype=torch.int64, device=dev)
+    indices = torch.empty(n * kk, dtype=torch.int32, device=dev)
+    data = torch.empty(n * kk, dtype=torch.float64, device=dev)
+    ws = workspace(lib.wmf_knn_train_workspace_bytes(n, int(k)), dev)
+    _lib.check(lib.wmf_knn_train(_ptr(X_csr.indptr), _ptr(X_csr.indices), X_csr.shape[0], _ptr(XT_csr.indptr),
+                                 _ptr(XT_csr.indices), n, int(k), _lib.KNN_SIMILARITIES[similarity], float(shrink),
+                                 _ptr(indptr), _ptr(indices), _ptr(data), _ptr(ws), ws.numel(), _stream()),
+               "wmf_knn_train")
+    nnz = int(indptr[-1])
+    if nnz < n * kk:
+        indices, data = indices[:nnz].clone(), data[:nnz].clone()
+    return indptr, indices, data
+
+
+@_device_of(0)
+def knn_predict(X_csr, W, users, items):
+    """float64 ItemKNN scores s(users[k], items[k]) (include/wmf_b200.h: wmf_knn_predict) for the canonical ``X_csr``
+    and W = (indptr, indices, data) as ``knn_train`` returns it; one user broadcasts."""
+    lib = _lib.load()
+    w_indptr, w_indices, w_data = W
+    n = items.numel()
+    stride = 1
+    if users.numel() == 1 and n != 1:
+        stride = 0
+    elif users.numel() != n:
+        raise ValueError("users and items need to have the same length or only one user needs to be provided.")
+    out = torch.empty(n, dtype=torch.float64, device=w_indptr.device)
+    _lib.check(lib.wmf_knn_predict(_ptr(X_csr.indptr), _ptr(X_csr.indices), _ptr(X_csr.data), _ptr(w_indptr),
+                                   _ptr(w_indices), _ptr(w_data), _ptr(users), stride, _ptr(items), n, _ptr(out),
+                                   _stream()), "wmf_knn_predict")
+    return out
+
+
+@_device_of(0)
+def knn_score_topk(X_csr, W, users, topn, exclude=None, want_scores=False):
+    """``ease_score_topk`` for the ItemKNN scores of ``knn_predict`` (bitwise): top-``topn`` item ids [nu x topn]
+    (int64) over all items minus the stored entries of row ``users[k]`` of ``exclude``, best first, ties to the lower
+    item id, -1 padding (include/wmf_b200.h: wmf_knn_score_topk); with ``want_scores`` (ids, float64 scores)."""
+    lib = _lib.load()
+    w_indptr, w_indices, w_data = W
+    n = w_indptr.numel() - 1
+    nu = users.numel()
+    dev = w_indptr.device
+    assert users.dtype == torch.int64 and X_csr.shape[1] == n
+    if exclude is not None:
+        assert exclude.shape[1] == n and exclude.indices.dtype == torch.int32 and exclude.indptr.dtype == torch.int64
+    ids = torch.empty((nu, topn), dtype=torch.int64, device=dev)
+    scores = torch.empty((nu, topn), dtype=torch.float64, device=dev) if want_scores else None
+    ws = workspace(lib.wmf_knn_score_topk_workspace_bytes(nu, n, topn), dev)
+    _lib.check(lib.wmf_knn_score_topk(_ptr(X_csr.indptr), _ptr(X_csr.indices), _ptr(X_csr.data), _ptr(w_indptr),
+                                      _ptr(w_indices), _ptr(w_data), n, _ptr(users), nu,
+                                      _ptr(None if exclude is None else exclude.indptr),
+                                      _ptr(None if exclude is None else exclude.indices), int(topn), _ptr(ids),
+                                      _ptr(scores), _ptr(ws), ws.numel(), _stream()), "wmf_knn_score_topk")
+    return (ids, scores) if want_scores else ids
