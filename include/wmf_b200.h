@@ -299,6 +299,27 @@ int wmf_knn_score_topk(const int64_t* x_indptr, const int32_t* x_indices, const 
                        const int64_t* ex_indptr, const int32_t* ex_indices, int topn, int64_t* out_ids,
                        double* out_scores, void* ws, size_t ws_bytes, void* stream);
 
+/* SLIM: sparse non-negative item-item regression (DESIGN.md 4.7). No reference call site: the SLIM sources of
+ * RecModel are not part of this repository, and this model is defined here, not ported.
+ * X, X^T and P are those of the knn entries above (canonical X); G = P^T P, so G[a, b] = c_ab. The candidates S_j of
+ * item j are row j of cand_indptr / cand_indices (wmf_knn_train's W with WMF_KNN_COSINE and shrink 0 is the intended
+ * source). Each row must be ascending, hold no self entry (j itself) and be no longer than k: not checked. Column j
+ * of W solves  min_w 1/2 |P[:, j] - P[:, S_j] w|^2 + l1 sum(w) + l2/2 |w|^2,  w >= 0, by cyclic coordinate descent on
+ * G_S = G[S_j, S_j] and b = G[S_j, j] in double, every operation rounded to nearest, none fused:
+ *   w = 0, q = b; per sweep: d = wm = 0; for p in order: z = q[p] + G_S[p,p] w[p];
+ *   new = z > l1 ? (z - l1) / (G_S[p,p] + l2) : 0; if new != w[p]: q[r] -= G_S[r,p] (new - w[p]) for all r, w[p] = new;
+ *   d = max(d, |new - old|), wm = max(wm, |new|); stop when wm == 0, d <= tol wm, or after max_iter sweeps.
+ * W^T is written as an n x n CSR (row j = column j of W: the candidates with w > 0, ascending ids): wt_indptr [n+1],
+ * and wt_indices / wt_data with room for n * min(k, n) entries, of which the first wt_indptr[n] are used.
+ * sweeps [n] (int32) receives the number of sweeps run per column. 1 <= k <= 128, l1 and l2 finite and >= 0,
+ * max_iter >= 1, tol finite and >= 0, 0 < n <= 2^30: else WMF_ERR_INVALID before any CUDA call. The workspace holds
+ * the dense int32 G (n^2 * 4 bytes, 64-bit offsets) and the staged columns. */
+size_t wmf_slim_train_workspace_bytes(int64_t n, int k);
+int wmf_slim_train(const int64_t* x_indptr, const int32_t* x_indices, int64_t rows, const int64_t* xt_indptr,
+                   const int32_t* xt_indices, int64_t n, const int64_t* cand_indptr, const int32_t* cand_indices, int k,
+                   double l1, double l2, int max_iter, double tol, int64_t* wt_indptr, int32_t* wt_indices,
+                   double* wt_data, int32_t* sweeps, void* ws, size_t ws_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -15,6 +15,7 @@ PREPROCESS_LOG, PREPROCESS_LINEAR = 0, 1
 ERR_NAMES = {1: "INVALID", 2: "WORKSPACE", 3: "CUDA", 4: "NO_DEVICE", 5: "UNSUPPORTED"}
 TOPK_MAX = 1024
 KNN_SIMILARITIES = {"cosine": 0, "jaccard": 1, "conditional": 2}  # WMF_KNN_COSINE / _JACCARD / _CONDITIONAL
+SLIM_K_MAX = 128   # longest candidate list wmf_slim_train keeps on chip
 
 _p, _i64, _i32, _f32, _sz = ctypes.c_void_p, ctypes.c_int64, ctypes.c_int, ctypes.c_float, ctypes.c_size_t
 _f64 = ctypes.c_double
@@ -69,6 +70,9 @@ SIGNATURES = {
     "wmf_knn_predict": (_i32, [_p, _p, _p, _p, _p, _p, _p, _i64, _p, _i64, _p, _p]),
     "wmf_knn_score_topk_workspace_bytes": (_sz, [_i64, _i64, _i32]),
     "wmf_knn_score_topk": (_i32, [_p, _p, _p, _p, _p, _p, _i64, _p, _i64, _p, _p, _i32, _p, _p, _p, _sz, _p]),
+    "wmf_slim_train_workspace_bytes": (_sz, [_i64, _i32]),
+    "wmf_slim_train": (_i32, [_p, _p, _i64, _p, _p, _i64, _p, _p, _i32, _f64, _f64, _i32, _f64, _p, _p, _p, _p, _p, _sz,
+                              _p]),
 }
 
 

@@ -5,6 +5,9 @@
 //   s(u, i) = sum over j of row u, ascending, of x_uj W[j, i] -> knn_score_tile_kernel (recommend), knn_predict_kernel
 // Every double operation is an explicit round-to-nearest intrinsic, so a NumPy restatement of the definitions
 // reproduces each similarity and each score bitwise.
+// SLIM (DESIGN.md 4.7) shares the counts, the staging-to-CSR kernels and the scoring: the dense G = P^T P comes from
+// knn_cooc_kernel over all n rows, slim_cd_kernel solves each column's regression on chip, and knn_scan_kernel plus
+// knn_compact_kernel write the CSR of W^T.
 #include "common.cuh"
 #include "score.cuh"
 
@@ -225,6 +228,138 @@ TrainLayout train_layout(int64_t n, int kk) {
     return L;
 }
 
+// ---- SLIM (DESIGN.md 4.7): one non-negative elastic-net regression per item column over its candidates, by cyclic
+// coordinate descent on the Gram G = P^T P, whose dense n x n int32 form knn_cooc_kernel writes (a0 = 0, B = n).
+
+constexpr int SL_MAX = 128;   // largest candidate list: the int32 G_S of 128 x 128 is 64 KB of shared memory
+
+__device__ __forceinline__ double sl_pick(const double (&v)[4], int t) {
+    return t == 0 ? v[0] : t == 1 ? v[1] : t == 2 ? v[2] : v[3];
+}
+
+// the first set bit at or after `from` in the 128-bit mask act, SL_MAX when there is none
+__device__ __forceinline__ int sl_next(const unsigned (&act)[4], int from) {
+#pragma unroll
+    for (int t = 0; t < 4; ++t) {
+        const int lo = from - 32 * t;
+        unsigned mk = lo >= 32 ? 0u : act[t];
+        if (lo > 0 && lo < 32) mk &= ~0u << lo;
+        if (mk) return 32 * t + __ffs(mk) - 1;
+    }
+    return SL_MAX;
+}
+
+// One warp per item column j. Lane l owns coordinates r = l + 32 t (t < 4): the candidate id s_r, q[r] and w[r] in
+// registers. G_S = G[S_j, S_j] (int32, row p at Gs + p m) stays in shared memory for the whole solve; G is symmetric,
+// so the column G_S[:, p] an update reads is row p, one conflict-free word per lane. Every lane runs the scalar part
+// of each step (same values), so the loop bounds, d and wm are warp-uniform. A ballot marks the coordinates that can
+// change (w != 0 or q > l1); the others are skipped, which changes no bit of the defined loop. The positive w go to
+// row j of the [n x kk] staging area in ascending id order, their number to cnt[j].
+__global__ __launch_bounds__(32) void slim_cd_kernel(const int* __restrict__ G, int64_t n,
+                                                     const int64_t* __restrict__ cand_indptr,
+                                                     const int32_t* __restrict__ cand_indices, int kk, double l1,
+                                                     double l2, int max_iter, double tol, int32_t* __restrict__ st_idx,
+                                                     double* __restrict__ st_val, int64_t* __restrict__ cnt,
+                                                     int32_t* __restrict__ sweeps) {
+    extern __shared__ int sl_smem[];
+    int* Gs = sl_smem;
+    int* ids = sl_smem + (size_t)kk * kk;
+    const int64_t j = blockIdx.x;
+    const int lane = threadIdx.x;
+    const int64_t c0 = cand_indptr[j];
+    const int m = (int)(cand_indptr[j + 1] - c0);
+    int s[4];
+    double q[4], w[4];
+#pragma unroll
+    for (int t = 0; t < 4; ++t) {
+        const int r = lane + 32 * t;
+        s[t] = r < m ? cand_indices[c0 + r] : 0;
+        if (r < m) ids[r] = s[t];
+        q[t] = r < m ? (double)G[j * n + s[t]] : 0.0;   // b = G[S_j, j] = G[j, S_j]
+        w[t] = 0.0;
+    }
+    __syncwarp();
+#pragma unroll 4
+    for (int p = 0; p < m; ++p) {
+        const int* grow = G + (int64_t)ids[p] * n;
+#pragma unroll
+        for (int t = 0; t < 4; ++t)
+            if (lane + 32 * t < m) Gs[p * m + lane + 32 * t] = grow[s[t]];
+    }
+    __syncwarp();
+
+    int sweep = 0;
+    bool done = false;
+    while (!done) {
+        ++sweep;
+        double d = 0.0, wm = 0.0;
+        unsigned act[4];
+#pragma unroll
+        for (int t = 0; t < 4; ++t) act[t] = __ballot_sync(0xffffffffu, lane + 32 * t < m && (w[t] != 0.0 || q[t] > l1));
+        for (int p = sl_next(act, 0); p < m; p = sl_next(act, p + 1)) {
+            const int tp = p >> 5, src = p & 31;
+            const double qp = __shfl_sync(0xffffffffu, sl_pick(q, tp), src);
+            const double old = __shfl_sync(0xffffffffu, sl_pick(w, tp), src);
+            const double gpp = (double)Gs[p * m + p];
+            const double z = __dadd_rn(qp, __dmul_rn(gpp, old));
+            const double nw = z > l1 ? __ddiv_rn(__dsub_rn(z, l1), __dadd_rn(gpp, l2)) : 0.0;
+            const double delta = __dsub_rn(nw, old);
+            if (nw != old) {
+#pragma unroll
+                for (int t = 0; t < 4; ++t) {
+                    const int r = lane + 32 * t;
+                    if (r < m) q[t] = __dsub_rn(q[t], __dmul_rn((double)Gs[p * m + r], delta));
+                    if (t == tp && lane == src) w[t] = nw;
+                }
+#pragma unroll
+                for (int t = 0; t < 4; ++t)
+                    act[t] = __ballot_sync(0xffffffffu, lane + 32 * t < m && (w[t] != 0.0 || q[t] > l1));
+            }
+            const double ad = fabs(delta), an = fabs(nw);
+            d = ad > d ? ad : d;
+            wm = an > wm ? an : wm;
+        }
+        done = wm == 0.0 || d <= __dmul_rn(tol, wm) || sweep >= max_iter;
+    }
+
+    int base = 0;
+#pragma unroll
+    for (int t = 0; t < 4; ++t) {
+        const bool pos = lane + 32 * t < m && w[t] > 0.0;
+        const unsigned mk = __ballot_sync(0xffffffffu, pos);
+        if (pos) {
+            const int64_t at = j * kk + base + __popc(mk & ((1u << lane) - 1u));
+            st_idx[at] = s[t];
+            st_val[at] = w[t];
+        }
+        base += __popc(mk);
+    }
+    if (lane == 0) {
+        cnt[j] = base;
+        sweeps[j] = sweep;
+    }
+}
+
+size_t slim_smem_bytes(int kk) { return ((size_t)kk * kk + SL_MAX) * sizeof(int); }
+
+struct SlimLayout {
+    size_t G, st_idx, st_val, cnt, total;
+};
+
+SlimLayout slim_layout(int64_t n, int kk) {
+    SlimLayout L;
+    size_t off = 0;
+    auto take = [&](size_t bytes) { const size_t at = off; off += align_up(bytes, 256); return at; };
+    L.G = take((size_t)n * (size_t)n * 4);
+    L.st_idx = take((size_t)n * kk * 4);
+    L.st_val = take((size_t)n * kk * 8);
+    L.cnt = take((size_t)n * 8);
+    L.total = off;
+    return L;
+}
+
+bool slim_finite_nonneg(double x) { return x >= 0.0 && x <= 1.7976931348623157e308; }
+
 int check_knn_args(const char* name, int64_t n, int k, int similarity, double shrink) {
     WMF_REQUIRE(n > 0 && n < (1ll << 31), "%s: n=%lld outside 1..2^31-1", name, (long long)n);
     WMF_REQUIRE(k >= 1 && k <= TK_MAX, "%s: k=%d outside 1..%d", name, k, TK_MAX);
@@ -342,6 +477,56 @@ int wmf_knn_score_topk(const int64_t* x_indptr, const int32_t* x_indices, const 
                                           out_scores ? out_scores + (size_t)u0 * topn : nullptr, st);
         if (rc) return rc;
     }
+    return WMF_OK;
+}
+
+size_t wmf_slim_train_workspace_bytes(int64_t n, int k) {
+    if (n <= 0 || n > (1ll << 30) || k < 1 || k > SL_MAX) return 0;
+    return slim_layout(n, (int)(k < n ? k : n)).total;
+}
+
+int wmf_slim_train(const int64_t* x_indptr, const int32_t* x_indices, int64_t rows, const int64_t* xt_indptr,
+                   const int32_t* xt_indices, int64_t n, const int64_t* cand_indptr, const int32_t* cand_indices, int k,
+                   double l1, double l2, int max_iter, double tol, int64_t* wt_indptr, int32_t* wt_indices,
+                   double* wt_data, int32_t* sweeps, void* ws, size_t ws_bytes, void* stream) {
+    WMF_REQUIRE(n > 0 && n <= (1ll << 30), "wmf_slim_train: n=%lld outside 1..2^30", (long long)n);
+    WMF_REQUIRE(k >= 1 && k <= SL_MAX, "wmf_slim_train: k=%d outside 1..%d", k, SL_MAX);
+    WMF_REQUIRE(slim_finite_nonneg(l1), "wmf_slim_train: l1=%g is not finite and >= 0", l1);
+    WMF_REQUIRE(slim_finite_nonneg(l2), "wmf_slim_train: l2=%g is not finite and >= 0", l2);
+    WMF_REQUIRE(max_iter >= 1, "wmf_slim_train: max_iter=%d < 1", max_iter);
+    WMF_REQUIRE(slim_finite_nonneg(tol), "wmf_slim_train: tol=%g is not finite and >= 0", tol);
+    WMF_REQUIRE(rows >= 0, "wmf_slim_train: rows=%lld < 0", (long long)rows);
+    WMF_REQUIRE(x_indptr && xt_indptr && cand_indptr && wt_indptr && wt_indices && wt_data && sweeps,
+                "wmf_slim_train: null argument");
+    const size_t need = wmf_slim_train_workspace_bytes(n, k);
+    if (ws == nullptr || ws_bytes < need) {
+        set_error("wmf_slim_train: workspace %zu < %zu", ws_bytes, need);
+        return WMF_ERR_WORKSPACE;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    const int kk = (int)(k < n ? k : n);
+    const SlimLayout L = slim_layout(n, kk);
+    char* base = reinterpret_cast<char*>(ws);
+    int* G = reinterpret_cast<int*>(base + L.G);
+    int32_t* st_idx = reinterpret_cast<int32_t*>(base + L.st_idx);
+    double* st_val = reinterpret_cast<double*>(base + L.st_val);
+    int64_t* cnt = reinterpret_cast<int64_t*>(base + L.cnt);
+    WMF_CUDA(cudaMemsetAsync(G, 0, (size_t)n * (size_t)n * 4, st));
+    if (rows > 0) {
+        knn_cooc_kernel<<<(unsigned)sm_count() * 8, KN_THREADS, 0, st>>>(x_indptr, x_indices, xt_indptr, xt_indices, n,
+                                                                         0, (int)n, G);
+        WMF_LAUNCH_CHECK("knn_cooc_kernel");
+    }
+    const size_t smem = slim_smem_bytes(kk);
+    WMF_CUDA(cudaFuncSetAttribute(slim_cd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    slim_cd_kernel<<<(unsigned)n, 32, smem, st>>>(G, n, cand_indptr, cand_indices, kk, l1, l2, max_iter, tol, st_idx,
+                                                  st_val, cnt, sweeps);
+    WMF_LAUNCH_CHECK("slim_cd_kernel");
+    knn_scan_kernel<<<1, KN_THREADS, 0, st>>>(cnt, n, wt_indptr);
+    WMF_LAUNCH_CHECK("knn_scan_kernel");
+    knn_compact_kernel<<<(unsigned)((n + KN_THREADS / 32 - 1) / (KN_THREADS / 32)), KN_THREADS, 0, st>>>(
+        st_idx, st_val, kk, n, wt_indptr, wt_indices, wt_data);
+    WMF_LAUNCH_CHECK("knn_compact_kernel");
     return WMF_OK;
 }
 

@@ -720,3 +720,36 @@ def knn_score_topk(X_csr, W, users, topn, exclude=None, want_scores=False):
                                       _ptr(None if exclude is None else exclude.indices), int(topn), _ptr(ids),
                                       _ptr(scores), _ptr(ws), ws.numel(), _stream()), "wmf_knn_score_topk")
     return (ids, scores) if want_scores else ids
+
+
+@_device_of(0)
+def slim_train(X_csr, XT_csr, k, l1, l2, max_iter, tol):
+    """The SLIM weights of the canonical interaction matrix ``X_csr`` (``XT_csr`` its transpose): the candidates are
+    the ``knn_train`` cosine neighbours (shrink 0) of each item, then ``wmf_slim_train`` solves every column (include/
+    wmf_b200.h). Returns (W, sweeps): W = (indptr int64 [n+1], indices int32, data float64), the n x n CSR with W[a, j]
+    in row a, ascending ids (the layout ``knn_predict`` and ``knn_score_topk`` take), and sweeps int32 [n]."""
+    lib = _lib.load()
+    n = X_csr.shape[1]
+    dev = X_csr.device
+    kk = min(int(k), n)
+    cand_indptr, cand_indices, _ = knn_train(X_csr, XT_csr, k, "cosine", 0.0)
+    wt_indptr = torch.empty(n + 1, dtype=torch.int64, device=dev)
+    wt_indices = torch.empty(n * kk, dtype=torch.int32, device=dev)
+    wt_data = torch.empty(n * kk, dtype=torch.float64, device=dev)
+    sweeps = torch.empty(n, dtype=torch.int32, device=dev)
+    nbytes = lib.wmf_slim_train_workspace_bytes(n, int(k))
+    if nbytes == 0:
+        raise ValueError(f"SLIM takes 1..{_lib.SLIM_K_MAX} candidates and at most 2^30 items, got k={k}, n={n}")
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)   # the dense n x n G: not kept in the shared workspace
+    _lib.check(lib.wmf_slim_train(_ptr(X_csr.indptr), _ptr(X_csr.indices), X_csr.shape[0], _ptr(XT_csr.indptr),
+                                  _ptr(XT_csr.indices), n, _ptr(cand_indptr), _ptr(cand_indices), int(k), float(l1),
+                                  float(l2), int(max_iter), float(tol), _ptr(wt_indptr), _ptr(wt_indices),
+                                  _ptr(wt_data), _ptr(sweeps), _ptr(ws), ws.numel(), _stream()), "wmf_slim_train")
+    del ws
+    nnz = int(wt_indptr[-1])
+    cols = torch.repeat_interleave(torch.arange(n, device=dev, dtype=torch.int64), wt_indptr[1:] - wt_indptr[:-1],
+                                   output_size=nnz)
+    rows = wt_indices[:nnz].to(torch.int64)
+    keys, order = torch.sort(rows * n + cols, stable=True)   # W^T -> W: by (a, j)
+    indptr = torch.searchsorted(keys, torch.arange(n + 1, device=dev, dtype=torch.int64) * n)
+    return (indptr, cols[order].to(torch.int32), wt_data[:nnz][order]), sweeps

@@ -1,4 +1,5 @@
-"""ItemKNN: an item-item neighbourhood model trained, scored and ranked on the device (DESIGN.md 4.6).
+"""ItemKNN: an item-item neighbourhood model trained, scored and ranked on the device (DESIGN.md 4.6), and
+``ItemItemModel``, the scoring half it shares with ``SLIM`` (slim_model.py).
 
 ``ItemKNN(num_items, num_users)``, ``train(X, k, similarity, shrink, verbose, cores)``, ``predict(users, items)``,
 ``rank(items, users, topn)``, ``recommend`` (top-N over each user's unseen items for many users in one device call),
@@ -30,7 +31,13 @@ def _canonical(M):
     return M
 
 
-class ItemKNN(RecModel):
+class ItemItemModel(RecModel):
+    """The scoring half shared by the item-item models (``ItemKNN``, ``SLIM``): the canonical X and an n x n item
+    weight CSR W on the device, and ``predict``, ``rank``, ``recommend`` and ``eval_ranking`` over
+    s(u, i) = sum over the entries j of row u of X, ascending, of x_uj * W[j, i]. A subclass trains W and names it
+    (``_W_NAME``, the attribute a user sets)."""
+
+    _W_NAME = "W"
 
     def __init__(self, num_items, num_users, device=None):
         self.num_items = num_items
@@ -46,25 +53,23 @@ class ItemKNN(RecModel):
             self._device = engine.default_device()
         return torch.device(self._device)
 
-    @property
-    def neighbors(self):
-        """W as an n x n SciPy CSR (float64, sorted indices): row a holds sim(a, b) for the neighbours b of a.
-        A host copy, made on first access. Assigning any n x n SciPy matrix (canonicalised: duplicates summed,
-        explicit zeros removed, indices sorted) replaces the model."""
+    def _W_host(self):
+        """W as an n x n SciPy CSR (float64, sorted indices), a host copy made on first access."""
         if self._W_h is None and self._W_d is not None:
             indptr, indices, data = (engine.d2h(t) for t in self._W_d)
             n = indptr.shape[0] - 1
             self._W_h = scipy.sparse.csr_matrix((data.copy(), indices.copy(), indptr.copy()), shape=(n, n))
         return self._W_h
 
-    @neighbors.setter
-    def neighbors(self, value):
+    def _set_W(self, value):
+        """Replace W by any n x n SciPy matrix (canonicalised: duplicates summed, explicit zeros removed, indices
+        sorted), or drop it with None."""
         if value is None:
             self._W_h = self._W_d = None
             return
         W = _canonical(value).astype(np.float64)
         if W.shape[0] != W.shape[1]:
-            raise ValueError(f"neighbors must be square, got {W.shape}")
+            raise ValueError(f"{self._W_NAME} must be square, got {W.shape}")
         self._W_h = W
         self._W_d = None
 
@@ -76,43 +81,16 @@ class ItemKNN(RecModel):
                          torch.from_numpy(W.data.astype(np.float64)).to(self.device))
         return self._W_d
 
-    def train(self, X, k=100, similarity="cosine", shrink=0.0, verbose=0, cores=1):
-        """Neighbours of every item from the users x items matrix X (any SciPy format, not modified).
-
-        X is canonicalised on the host (CSR, duplicates summed, explicit zeros removed, sorted rows); that copy is
-        kept for scoring. With P its binary pattern, c_ab = sum_u P[u, a] P[u, b] (exact integers; c_aa is the
-        popularity of a), and in double with every operation rounded to nearest:
-        "cosine" c_ab / (sqrt(c_aa) sqrt(c_bb) + shrink), "jaccard" c_ab / ((c_aa + c_bb - c_ab) + shrink),
-        "conditional" c_ab / (c_aa + shrink) = P(b | a) (not symmetric). The neighbours of a are the top-k items
-        b != a with c_ab > 0 by sim(a, b), ties to the lower id (fewer when a has fewer such items); W[a, b] =
-        sim(a, b) (``neighbors``). k in 1..1024 (k >= num_items keeps every candidate), shrink finite and >= 0."""
-        if similarity not in _lib.KNN_SIMILARITIES:
-            raise ValueError(f"similarity must be one of {sorted(_lib.KNN_SIMILARITIES)}, got {similarity!r}")
-        if isinstance(k, (bool, np.bool_)) or not isinstance(k, (int, np.integer)) or not 1 <= k <= _lib.TOPK_MAX:
-            raise ValueError(f"k must be an int in 1..{_lib.TOPK_MAX}, got {k!r}")
-        shrink = float(shrink)
-        if not (math.isfinite(shrink) and shrink >= 0.0):
-            raise ValueError(f"shrink must be finite and >= 0, got {shrink}")
-        Xc = _canonical(X)
-        if verbose > 0:
-            print("Compute the item neighbourhoods")
-            start = time.time()
-        self._X = DeviceCSR.from_scipy(Xc, self.device)
-        self._W_d = engine.knn_train(self._X, self._X.transpose(), int(k), similarity, shrink)
-        self._W_h = None
-        if verbose > 0:
-            torch.cuda.synchronize(self.device)
-            print(f"Training took {time.time() - start} seconds!")
-
     def _X_and_W(self):
         """(X, W) on the device; ValueError when the model is untrained or W does not fit X."""
         if self._X is None:
             raise ValueError("the model has no interaction matrix X: call train(X, ...) first")
         W = self._W_device()
         if W is None:
-            raise ValueError("the model has no neighbours: call train(X, ...) first")
+            raise ValueError(f"the model has no {self._W_NAME}: call train(X, ...) first")
         if W[0].numel() - 1 != self._X.shape[1]:
-            raise ValueError(f"neighbors is {W[0].numel() - 1} x {W[0].numel() - 1} but X has {self._X.shape[1]} items")
+            raise ValueError(f"{self._W_NAME} is {W[0].numel() - 1} x {W[0].numel() - 1} but X has "
+                             f"{self._X.shape[1]} items")
         return self._X, W
 
     def predict(self, users, items):
@@ -184,3 +162,47 @@ class ItemKNN(RecModel):
             return X.shape[1], X.shape[0]
         return ranking.eval_ranking(lambda users_d, k, ex: self._recommend_ids(users_d, k, ex), dims, "the rows of X",
                                     self.device, test_mat, topn, exclude, users, _EVAL_CHUNK_IDS)
+
+
+class ItemKNN(ItemItemModel):
+
+    _W_NAME = "neighbors"
+
+    @property
+    def neighbors(self):
+        """W as an n x n SciPy CSR (float64, sorted indices): row a holds sim(a, b) for the neighbours b of a.
+        A host copy, made on first access. Assigning any n x n SciPy matrix (canonicalised: duplicates summed,
+        explicit zeros removed, indices sorted) replaces the model."""
+        return self._W_host()
+
+    @neighbors.setter
+    def neighbors(self, value):
+        self._set_W(value)
+
+    def train(self, X, k=100, similarity="cosine", shrink=0.0, verbose=0, cores=1):
+        """Neighbours of every item from the users x items matrix X (any SciPy format, not modified).
+
+        X is canonicalised on the host (CSR, duplicates summed, explicit zeros removed, sorted rows); that copy is
+        kept for scoring. With P its binary pattern, c_ab = sum_u P[u, a] P[u, b] (exact integers; c_aa is the
+        popularity of a), and in double with every operation rounded to nearest:
+        "cosine" c_ab / (sqrt(c_aa) sqrt(c_bb) + shrink), "jaccard" c_ab / ((c_aa + c_bb - c_ab) + shrink),
+        "conditional" c_ab / (c_aa + shrink) = P(b | a) (not symmetric). The neighbours of a are the top-k items
+        b != a with c_ab > 0 by sim(a, b), ties to the lower id (fewer when a has fewer such items); W[a, b] =
+        sim(a, b) (``neighbors``). k in 1..1024 (k >= num_items keeps every candidate), shrink finite and >= 0."""
+        if similarity not in _lib.KNN_SIMILARITIES:
+            raise ValueError(f"similarity must be one of {sorted(_lib.KNN_SIMILARITIES)}, got {similarity!r}")
+        if isinstance(k, (bool, np.bool_)) or not isinstance(k, (int, np.integer)) or not 1 <= k <= _lib.TOPK_MAX:
+            raise ValueError(f"k must be an int in 1..{_lib.TOPK_MAX}, got {k!r}")
+        shrink = float(shrink)
+        if not (math.isfinite(shrink) and shrink >= 0.0):
+            raise ValueError(f"shrink must be finite and >= 0, got {shrink}")
+        Xc = _canonical(X)
+        if verbose > 0:
+            print("Compute the item neighbourhoods")
+            start = time.time()
+        self._X = DeviceCSR.from_scipy(Xc, self.device)
+        self._W_d = engine.knn_train(self._X, self._X.transpose(), int(k), similarity, shrink)
+        self._W_h = None
+        if verbose > 0:
+            torch.cuda.synchronize(self.device)
+            print(f"Training took {time.time() - start} seconds!")
