@@ -443,41 +443,22 @@ int wmf_knn_predict(const int64_t* x_indptr, const int32_t* x_indices, const flo
 
 size_t wmf_knn_score_topk_workspace_bytes(int64_t nu, int64_t n, int topn) {
     (void)topn;
-    if (nu <= 0 || n <= 0 || n >= (1ll << 31)) return 0;
-    return align_up((size_t)knn_batch(nu, n) * (size_t)n * sizeof(double), 1024);
+    return score_topk_double_workspace_bytes(nu, n, knn_batch);
 }
 
 int wmf_knn_score_topk(const int64_t* x_indptr, const int32_t* x_indices, const float* x_data, const int64_t* w_indptr,
                        const int32_t* w_indices, const double* w_data, int64_t n, const int64_t* users, int64_t nu,
                        const int64_t* ex_indptr, const int32_t* ex_indices, int topn, int64_t* out_ids,
                        double* out_scores, void* ws, size_t ws_bytes, void* stream) {
-    WMF_REQUIRE(n > 0 && n < (1ll << 31), "wmf_knn_score_topk: n=%lld outside 1..2^31-1", (long long)n);
-    WMF_REQUIRE(nu >= 0, "wmf_knn_score_topk: nu=%lld < 0", (long long)nu);
-    if (topn < 1 || topn > n || topn > TK_MAX) {
-        set_error("wmf_knn_score_topk: topn=%d outside 1..min(n=%lld, %d)", topn, (long long)n, TK_MAX);
-        return WMF_ERR_UNSUPPORTED;
-    }
-    if (nu == 0) return WMF_OK;
-    WMF_REQUIRE(x_indptr && w_indptr && users && out_ids, "wmf_knn_score_topk: null argument");
-    const size_t need = wmf_knn_score_topk_workspace_bytes(nu, n, topn);
-    if (ws == nullptr || ws_bytes < need) {
-        set_error("wmf_knn_score_topk: workspace %zu < %zu", ws_bytes, need);
-        return WMF_ERR_WORKSPACE;
-    }
-    cudaStream_t st = (cudaStream_t)stream;
-    const int64_t ubatch = knn_batch(nu, n);
-    double* S = (double*)ws;
-    for (int64_t u0 = 0; u0 < nu; u0 += ubatch) {
-        const int ub = (int)((nu - u0) < ubatch ? (nu - u0) : ubatch);
+    return score_topk_double("wmf_knn_score_topk", x_indptr && w_indptr, knn_batch, n, users, nu, ex_indptr, ex_indices,
+                             topn, out_ids, out_scores, ws, ws_bytes, stream,
+                             [&](int64_t u0, int ub, double* S, cudaStream_t st) {
         WMF_CUDA(cudaMemsetAsync(S, 0, (size_t)ub * n * sizeof(double), st));
         knn_score_tile_kernel<<<(unsigned)((ub + KN_THREADS / 32 - 1) / (KN_THREADS / 32)), KN_THREADS, 0, st>>>(
             x_indptr, x_indices, x_data, w_indptr, w_indices, w_data, n, users, u0, ub, S);
         WMF_LAUNCH_CHECK("knn_score_tile_kernel");
-        const int rc = select_topk_double(users, u0, ub, ex_indptr, ex_indices, S, n, topn, out_ids + (size_t)u0 * topn,
-                                          out_scores ? out_scores + (size_t)u0 * topn : nullptr, st);
-        if (rc) return rc;
-    }
-    return WMF_OK;
+        return WMF_OK;
+    });
 }
 
 size_t wmf_slim_train_workspace_bytes(int64_t n, int k) {

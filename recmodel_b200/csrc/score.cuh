@@ -60,6 +60,48 @@ int select_topk_double(const int64_t* users, int64_t u_begin, int ub, const int6
                        double* S, int64_t ni, int topn, int64_t* out_ids, double* out_scores, cudaStream_t st,
                        bool marked = false);
 
+// Bytes of the [user_batch(nu, n) x n] double score tile that score_topk_double needs; 0 when nu or n is out of range.
+inline size_t score_topk_double_workspace_bytes(int64_t nu, int64_t n, int64_t (*user_batch)(int64_t, int64_t)) {
+    if (nu <= 0 || n <= 0 || n >= (1ll << 31)) return 0;
+    return align_up((size_t)user_batch(nu, n) * (size_t)n * sizeof(double), 1024);
+}
+
+// The exact double top-N over all n items of a model that scores users tile by tile (wmf_ease_score_topk,
+// wmf_knn_score_topk; `name` prefixes the messages). The checks run in a fixed order: n, nu, topn (WMF_ERR_UNSUPPORTED),
+// nu == 0 returns WMF_OK before any pointer is looked at, then the pointers (`inputs_ok`: the model's own inputs are
+// non-null) and the workspace. Then, for each batch of ub <= user_batch(nu, n) users from u0, score_tile(u0, ub, S, st)
+// writes their [ub x n] scores into the workspace S and returns a WMF_* code, and select_topk_double ranks them.
+template <typename ScoreTile>
+int score_topk_double(const char* name, bool inputs_ok, int64_t (*user_batch)(int64_t, int64_t), int64_t n,
+                      const int64_t* users, int64_t nu, const int64_t* ex_indptr, const int32_t* ex_indices, int topn,
+                      int64_t* out_ids, double* out_scores, void* ws, size_t ws_bytes, void* stream,
+                      ScoreTile score_tile) {
+    WMF_REQUIRE(n > 0 && n < (1ll << 31), "%s: n=%lld outside 1..2^31-1", name, (long long)n);
+    WMF_REQUIRE(nu >= 0, "%s: nu=%lld < 0", name, (long long)nu);
+    if (topn < 1 || topn > n || topn > TK_MAX) {
+        set_error("%s: topn=%d outside 1..min(n=%lld, %d)", name, topn, (long long)n, TK_MAX);
+        return WMF_ERR_UNSUPPORTED;
+    }
+    if (nu == 0) return WMF_OK;
+    WMF_REQUIRE(inputs_ok && users && out_ids, "%s: null argument", name);
+    const size_t need = score_topk_double_workspace_bytes(nu, n, user_batch);
+    if (ws == nullptr || ws_bytes < need) {
+        set_error("%s: workspace %zu < %zu", name, ws_bytes, need);
+        return WMF_ERR_WORKSPACE;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    const int64_t ubatch = user_batch(nu, n);
+    double* S = (double*)ws;
+    for (int64_t u0 = 0; u0 < nu; u0 += ubatch) {
+        const int ub = (int)((nu - u0) < ubatch ? (nu - u0) : ubatch);
+        if (int rc = score_tile(u0, ub, S, st)) return rc;
+        if (int rc = select_topk_double(users, u0, ub, ex_indptr, ex_indices, S, n, topn, out_ids + (size_t)u0 * topn,
+                                        out_scores ? out_scores + (size_t)u0 * topn : nullptr, st))
+            return rc;
+    }
+    return WMF_OK;
+}
+
 bool score_tc_supported(int64_t ni, int f, int bias, int topn);
 size_t score_tc_workspace_bytes(int64_t nu, int64_t ni);
 int64_t score_tc_user_batch(int64_t nu);

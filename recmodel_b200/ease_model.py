@@ -3,7 +3,8 @@
 Mirror of /root/reference/RecModel/ease_model.py:45-114: ``Ease(num_items, num_users)``, ``train(X, alpha, verbose,
 cores)``, ``predict(users, items)``, ``rank(items, users, topn)``, ``save_mat`` / ``load_mat`` and the inherited
 ``eval_topn``, plus ``recommend`` (top-N over each user's unseen items for many users in one device call) and
-``eval_ranking`` (full-ranking Recall / Precision / NDCG / MAP / hit rate at N), as the WMF model has them. The Gram X^T X + alpha I, its dense inverse and the prediction loop of
+``eval_ranking`` (full-ranking Recall / Precision / NDCG / MAP / hit rate at N) from ``ranking.XWRanking``, which the
+item-item models share. The Gram X^T X + alpha I, its dense inverse and the prediction loop of
 RecModel/fast_utils/ease_utils.pyx:15-30 run in the kernels of csrc/ease.cu behind the C ABI; there is no CPU
 fallback. ``cores`` is accepted and ignored (the reference only sets MKL's thread count with it).
 """
@@ -12,14 +13,16 @@ import time
 import numpy as np
 import torch
 
-from . import _lib, engine, ranking
+from . import engine
 from .base_model import RecModel
 from .engine import DeviceCSR
+from .ranking import XWRanking
 
-_EVAL_CHUNK_IDS = ranking.EVAL_CHUNK_IDS
 
+class Ease(XWRanking, RecModel):
 
-class Ease(RecModel):
+    _score_topk = staticmethod(engine.ease_score_topk)
+    _predict_pairs = staticmethod(engine.ease_predict)
 
     def __init__(self, num_items, num_users, device=None):
         self.num_items = num_items
@@ -28,12 +31,6 @@ class Ease(RecModel):
         self._W_d = None
         self._W_h = None
         self._X = None
-
-    @property
-    def device(self):
-        if self._device is None:
-            self._device = engine.default_device()
-        return torch.device(self._device)
 
     # W is a plain ndarray attribute in the reference (ease_model.py:49,109): host copy on demand
     @property
@@ -99,67 +96,6 @@ class Ease(RecModel):
         if W.shape[0] != self._X.shape[1]:
             raise ValueError(f"W is {W.shape[0]} x {W.shape[1]} but X has {self._X.shape[1]} items")
         return self._X, W
-
-    def recommend(self, users, topn, exclude=None):
-        """int64 [len(users) x topn]: the top-``topn`` of all items for each user, best first, leaving out the stored
-        entries of row ``users[k]`` of ``exclude`` (users x items like X, any SciPy format or a DeviceCSR; every stored
-        entry excludes its item whatever its value). Row k is ``rank(np.delete(np.arange(num_items), seen), users[k],
-        topn)`` followed by -1 where the user has fewer than ``topn`` unseen items; ties go to the lower item id. The
-        scores are those of ``predict`` (float64, bitwise), ranked on the device without rounding to float32."""
-        X, W = self._X_and_W()
-        n = W.shape[0]
-        users = np.ascontiguousarray(users, dtype=np.int64).reshape(-1)
-        if len(users) and (users.min() < 0 or users.max() >= X.shape[0]):
-            raise ValueError(f"user ids must lie in [0, {X.shape[0]}) (the rows of X)")
-        if exclude is not None and tuple(exclude.shape) != tuple(X.shape):
-            raise ValueError(f"exclude has shape {tuple(exclude.shape)}, X {tuple(X.shape)}")
-        topn = int(topn)
-        k = min(topn, n)
-        out = np.full((len(users), topn), -1, dtype=np.int64)
-        if k <= 0 or len(users) == 0:
-            return out
-        ex = None
-        if exclude is not None:
-            ex = exclude if isinstance(exclude, DeviceCSR) else DeviceCSR.from_scipy(exclude, self.device)
-        out[:, :k] = self._recommend_ids(torch.from_numpy(users).to(self.device), k, ex).cpu().numpy()
-        return out
-
-    def _recommend_ids(self, users_d, k, ex):
-        """Device int64 [len(users_d) x k], k <= num_items: the device part of ``recommend`` (``ex``: a DeviceCSR with
-        rows in any order, or None to exclude nothing)."""
-        X, W = self._X_and_W()
-        if k <= _lib.TOPK_MAX:
-            return engine.ease_score_topk(X, W, users_d, k, exclude=ex)
-        # very long lists: exact device scores (ease_predict, the same bits), then stable device sorts
-        n = W.shape[0]
-        return ranking.sort_path_ids(users_d, n, k, ex, lambda chunk, items_d: engine.ease_predict(
-            X, W, chunk.repeat_interleave(n), items_d.repeat(chunk.numel())).view(chunk.numel(), n))
-
-    def eval_ranking(self, test_mat, topn=np.array([10]), exclude=None, users=None):
-        """Full-ranking quality of ``recommend``: for each cutoff k of ``topn`` (an int or at most 16 distinct positive
-        ints) a dict with "Recall@k", "Precision@k", "NDCG@k", "MAP@k" and "HitRate@k" (Python floats, means over the
-        evaluated users) and "users" (their number). Unlike ``eval_topn``, which ranks each held-out item against
-        ``rand_sampled`` random items and divides the hits by nnz(test), this ranks ALL items and averages per user.
-
-        The list of user u is ``recommend(users, K, exclude)`` with K = max(topn) (ties to the lower item id, -1
-        padding never a hit). T_u is the set of distinct columns of row u of ``test_mat`` with a stored non-zero value
-        (duplicates count once; unsorted rows and explicit zeros are fine), h_i the hits among the first i items:
-        Precision@k = h_k / k (k also when the list is padded), Recall@k = h_k / |T_u|, NDCG@k = the sum of
-        1/log2(i+1) over the hits at i <= k over the same sum over i <= min(k, |T_u|) (binary gains), MAP@k = the sum
-        of h_i / i over the hits at i <= k over min(k, |T_u|), HitRate@k = [h_k > 0]. Users with T_u empty are ranked
-        but not counted; an item both in ``exclude`` and in T_u counts in |T_u| and can never be hit.
-
-        ``test_mat`` and ``exclude`` (None: nothing excluded) are users x items SciPy matrices or DeviceCSRs of the
-        shape of X, uploaded once. ``users`` defaults to the rows of ``test_mat`` with stored entries; repeated entries
-        count each time. Lists, metrics and their sums stay on the device (the per-user rows are reduced once, in a
-        fixed order: the result is bitwise reproducible)."""
-        def dims():
-            X, W = self._X_and_W()
-            if tuple(test_mat.shape) != tuple(X.shape):
-                raise ValueError(f"test_mat has shape {tuple(test_mat.shape)}, X {tuple(X.shape)}")
-            return W.shape[0], X.shape[0]
-        return ranking.eval_ranking(lambda users_d, k, ex: self._recommend_ids(users_d, k, ex), dims, "the rows of X",
-                                    self.device, test_mat, topn, exclude, users, _EVAL_CHUNK_IDS)
 
     def load_mat(self, path="W_mat.npy", X=None):
         try:

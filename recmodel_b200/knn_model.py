@@ -15,11 +15,10 @@ import numpy as np
 import scipy.sparse
 import torch
 
-from . import _lib, engine, ranking
+from . import _lib, engine
 from .base_model import RecModel
 from .engine import DeviceCSR
-
-_EVAL_CHUNK_IDS = ranking.EVAL_CHUNK_IDS
+from .ranking import XWRanking
 
 
 def _canonical(M):
@@ -31,13 +30,15 @@ def _canonical(M):
     return M
 
 
-class ItemItemModel(RecModel):
+class ItemItemModel(XWRanking, RecModel):
     """The scoring half shared by the item-item models (``ItemKNN``, ``SLIM``): the canonical X and an n x n item
-    weight CSR W on the device, and ``predict``, ``rank``, ``recommend`` and ``eval_ranking`` over
-    s(u, i) = sum over the entries j of row u of X, ascending, of x_uj * W[j, i]. A subclass trains W and names it
-    (``_W_NAME``, the attribute a user sets)."""
+    weight CSR W on the device, and ``predict`` and ``rank`` over s(u, i) = sum over the entries j of row u of X,
+    ascending, of x_uj * W[j, i]; ``recommend`` and ``eval_ranking`` rank these scores (``ranking.XWRanking``). A
+    subclass trains W and names it (``_W_NAME``, the attribute a user sets)."""
 
     _W_NAME = "W"
+    _score_topk = staticmethod(engine.knn_score_topk)
+    _predict_pairs = staticmethod(engine.knn_predict)
 
     def __init__(self, num_items, num_users, device=None):
         self.num_items = num_items
@@ -46,12 +47,6 @@ class ItemItemModel(RecModel):
         self._X = None
         self._W_d = None      # (indptr int64, indices int32, data float64) on the device
         self._W_h = None
-
-    @property
-    def device(self):
-        if self._device is None:
-            self._device = engine.default_device()
-        return torch.device(self._device)
 
     def _W_host(self):
         """W as an n x n SciPy CSR (float64, sorted indices), a host copy made on first access."""
@@ -116,52 +111,6 @@ class ItemItemModel(RecModel):
         items = np.asarray(items)
         scores = self.predict(np.full(1, users, dtype=np.int64), items)
         return items[np.argsort(-scores, kind="stable")][:topn]
-
-    def recommend(self, users, topn, exclude=None):
-        """int64 [len(users) x topn]: the top-``topn`` of all items for each user, best first, leaving out the stored
-        entries of row ``users[k]`` of ``exclude`` (users x items like X, any SciPy format or a DeviceCSR; every stored
-        entry excludes its item whatever its value). Ties go to the lower item id, and a user with fewer than ``topn``
-        unseen items gets -1 in the rest of its row. The scores are those of ``predict`` (float64, bitwise)."""
-        X, W = self._X_and_W()
-        n = X.shape[1]
-        users = np.ascontiguousarray(users, dtype=np.int64).reshape(-1)
-        if len(users) and (users.min() < 0 or users.max() >= X.shape[0]):
-            raise ValueError(f"user ids must lie in [0, {X.shape[0]}) (the rows of X)")
-        if exclude is not None and tuple(exclude.shape) != tuple(X.shape):
-            raise ValueError(f"exclude has shape {tuple(exclude.shape)}, X {tuple(X.shape)}")
-        topn = int(topn)
-        k = min(topn, n)
-        out = np.full((len(users), topn), -1, dtype=np.int64)
-        if k <= 0 or len(users) == 0:
-            return out
-        ex = None
-        if exclude is not None:
-            ex = exclude if isinstance(exclude, DeviceCSR) else DeviceCSR.from_scipy(exclude, self.device)
-        out[:, :k] = self._recommend_ids(torch.from_numpy(users).to(self.device), k, ex).cpu().numpy()
-        return out
-
-    def _recommend_ids(self, users_d, k, ex):
-        """Device int64 [len(users_d) x k], k <= num_items: the device part of ``recommend``."""
-        X, W = self._X_and_W()
-        if k <= _lib.TOPK_MAX:
-            return engine.knn_score_topk(X, W, users_d, k, exclude=ex)
-        n = X.shape[1]   # very long lists: the scores of predict, then stable device sorts
-        return ranking.sort_path_ids(users_d, n, k, ex, lambda chunk, items_d: engine.knn_predict(
-            X, W, chunk.repeat_interleave(n), items_d.repeat(chunk.numel())).view(chunk.numel(), n))
-
-    def eval_ranking(self, test_mat, topn=np.array([10]), exclude=None, users=None):
-        """Full-ranking quality of ``recommend`` with the definitions of ``Ease.eval_ranking``: for each cutoff k of
-        ``topn`` (an int or at most 16 distinct positive ints) "Recall@k", "Precision@k", "NDCG@k", "MAP@k" and
-        "HitRate@k" averaged over the evaluated users with a stored non-zero test entry, and "users", their number.
-        ``test_mat`` and ``exclude`` are users x items matrices of the shape of X (SciPy or DeviceCSR); ``users``
-        defaults to the rows of ``test_mat`` with stored entries. The sums are bitwise reproducible."""
-        def dims():
-            X, W = self._X_and_W()
-            if tuple(test_mat.shape) != tuple(X.shape):
-                raise ValueError(f"test_mat has shape {tuple(test_mat.shape)}, X {tuple(X.shape)}")
-            return X.shape[1], X.shape[0]
-        return ranking.eval_ranking(lambda users_d, k, ex: self._recommend_ids(users_d, k, ex), dims, "the rows of X",
-                                    self.device, test_mat, topn, exclude, users, _EVAL_CHUNK_IDS)
 
 
 class ItemKNN(ItemItemModel):

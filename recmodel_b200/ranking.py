@@ -1,29 +1,33 @@
-"""Model-independent parts of ``recommend`` and ``eval_ranking``, shared by WMF and Ease: the exact-score sort path for
-lists longer than the selection kernels take, and the full-ranking evaluation around a model's device ranking."""
+"""Model-independent parts of ``recommend`` and ``eval_ranking``, shared by every model: the exact-score sort path for
+lists longer than the selection kernels take, and the full-ranking evaluation around a model's device ranking.
+``XWRanking`` builds both methods on them for the models scored from a device X and an item weight W (``Ease``,
+``ItemKNN``, ``SLIM``)."""
 import numpy as np
 import torch
 
-from . import engine
+from . import _lib, engine
 from .engine import DeviceCSR
 
 EVAL_CHUNK_IDS = 1 << 25  # eval_ranking ranks users in chunks of at most this many list entries (32 M ids, 256 MB)
 
 
-def sort_path_ids(users_d, ni, k, ex, scores):
-    """Device int64 [len(users_d) x k]: each user's items 0..ni-1 in descending order of ``scores(chunk, items_d)``
-    (a device [len(chunk) x ni] tensor of exact scores), ties to the lower item id, with the stored entries of row
-    ``users_d[r]`` of ``ex`` (a DeviceCSR indexed by user id, or None) moved behind every unseen item and reported as
-    -1. The users are scored in chunks of at most ~16 M (user, item) pairs."""
+def sort_path_ids(users_d, ni, k, ex, scores, cand=None):
+    """Device int64 [len(users_d) x k]: each user's ni items ``items_d`` (the device int64 candidate ids ``cand``, or
+    None for the items 0..ni-1) in descending order of ``scores(chunk, items_d)`` (a device [len(chunk) x ni] tensor of
+    exact scores), ties to the lower position, reported as ``items_d[position]``. Only with ``cand`` None, the stored
+    entries of row ``users_d[r]`` of ``ex`` (a DeviceCSR indexed by user id, or None) are moved behind every unseen
+    item and reported as -1. The users are scored in chunks of at most ~16 M (user, item) pairs."""
+    assert ex is None or cand is None, "exclusion is by item id: it needs the candidates 0..ni-1"
     dev = users_d.device
     rows = []
     per = max(1, (1 << 24) // ni)
-    items_d = torch.arange(ni, dtype=torch.int64, device=dev)
+    items_d = torch.arange(ni, dtype=torch.int64, device=dev) if cand is None else cand
     for u0 in range(0, users_d.numel(), per):
         chunk = users_d[u0:u0 + per]
         n = chunk.numel()
         order = torch.sort(scores(chunk, items_d), dim=1, descending=True, stable=True).indices
         if ex is None:
-            rows.append(order[:, :k])
+            rows.append(order[:, :k] if cand is None else cand[order[:, :k]])
             continue
         lo, cnt = ex.indptr[chunk], ex.indptr[chunk + 1] - ex.indptr[chunk]
         total = int(cnt.sum())
@@ -39,13 +43,13 @@ def sort_path_ids(users_d, ni, k, ex, scores):
     return torch.cat(rows) if rows else torch.empty((0, k), dtype=torch.int64, device=dev)
 
 
-def eval_ranking(rank_ids, dims, users_what, device, test_mat, topn, exclude, users, chunk_ids=EVAL_CHUNK_IDS):
-    """The full-ranking evaluation of ``WMF.eval_ranking`` / ``Ease.eval_ranking`` (see their docstrings) for a model
-    whose ``rank_ids(users_d, k, ex)`` returns the device int64 [len(users_d) x k] lists of ``recommend`` (k <= the
+def eval_ranking(rank_ids, dims, users_what, device, test_mat, topn, exclude, users):
+    """The full-ranking evaluation of ``WMF.eval_ranking`` / ``XWRanking.eval_ranking`` (see their docstrings) for a
+    model whose ``rank_ids(users_d, k, ex)`` returns the device int64 [len(users_d) x k] lists of ``recommend`` (k <= the
     number of items; ex: the exclusion DeviceCSR, or None). ``dims()`` returns (items, users) of the model, read once
     ``topn`` is valid: user ids must lie below that number of users and the rows of ``test_mat``; ``users_what`` names
-    what bounds them in the error message. The users are ranked in chunks of at most
-    ``chunk_ids`` list entries (``eval_ranking_sums``)."""
+    what bounds them in the error message. The users are ranked in chunks of at most ``EVAL_CHUNK_IDS`` list entries
+    (``eval_ranking_sums``)."""
     ks = np.asarray(topn)
     if ks.ndim == 0:
         ks = ks.reshape(1)
@@ -74,7 +78,7 @@ def eval_ranking(rank_ids, dims, users_what, device, test_mat, topn, exclude, us
             raise bad_users
     else:
         users_d = torch.from_numpy(users).to(device)
-    sums = eval_ranking_sums(rank_ids, ni, T, ex, users_d, ks, chunk_ids).cpu().numpy()
+    sums = eval_ranking_sums(rank_ids, ni, T, ex, users_d, ks).cpu().numpy()
     count = int(sums[-1])
     out = {}
     for j, kk in enumerate(ks.tolist()):
@@ -84,9 +88,10 @@ def eval_ranking(rank_ids, dims, users_what, device, test_mat, topn, exclude, us
     return out
 
 
-def eval_ranking_sums(rank_ids, ni, T, ex, users_d, ks, chunk_ids=EVAL_CHUNK_IDS):
+def eval_ranking_sums(rank_ids, ni, T, ex, users_d, ks, chunk_ids=None):
     """The device part of ``eval_ranking`` (T: the test DeviceCSR with sorted rows; ex: the exclusion DeviceCSR or
-    None; ks: int64 cutoffs): the users are ranked in chunks of at most ``chunk_ids`` list entries, each chunk's
+    None; ks: int64 cutoffs): the users are ranked in chunks of at most ``chunk_ids`` list entries (None:
+    ``EVAL_CHUNK_IDS`` as it is at the call), each chunk's
     per-user metrics land in one buffer, and one reduce returns the device float64 [len(ks)*5 + 1] sums and the
     evaluated-user count, summed in a fixed order (bitwise reproducible). No ids leave the device."""
     device = users_d.device
@@ -94,7 +99,7 @@ def eval_ranking_sums(rank_ids, ni, T, ex, users_d, ks, chunk_ids=EVAL_CHUNK_IDS
     k = min(K, ni)
     n = users_d.numel()
     per_user = torch.empty((n, len(ks), 5), dtype=torch.float64, device=device)
-    chunk = max(1, chunk_ids // K)
+    chunk = max(1, (EVAL_CHUNK_IDS if chunk_ids is None else chunk_ids) // K)
     for u0 in range(0, n, chunk):
         part = users_d[u0:u0 + chunk]
         ids = rank_ids(part, k, ex)
@@ -102,3 +107,75 @@ def eval_ranking_sums(rank_ids, ni, T, ex, users_d, ks, chunk_ids=EVAL_CHUNK_IDS
             ids = torch.cat((ids, torch.full((part.numel(), K - k), -1, dtype=torch.int64, device=device)), dim=1)
         engine.topn_metrics(ids, part, T, ks, out=per_user[u0:u0 + chunk])
     return engine.topn_metrics_reduce(per_user, len(ks))
+
+
+class XWRanking:
+    """``recommend`` and ``eval_ranking`` of a model whose score s(u, i) is computed on the device from the users x
+    items interaction matrix X and an item weight W (``Ease``, ``ItemItemModel``). A subclass provides ``_X_and_W()``
+    (X as a DeviceCSR and W in the layout of its engine functions, or ValueError when the model cannot score),
+    ``_score_topk(X, W, users_d, k, exclude=ex)``, the device top-k of at most ``_lib.TOPK_MAX`` items, and
+    ``_predict_pairs(X, W, users_d, items_d)``, the float64 scores of (user, item) pairs, which it ranks bitwise."""
+
+    @property
+    def device(self):
+        if self._device is None:
+            self._device = engine.default_device()
+        return torch.device(self._device)
+
+    def recommend(self, users, topn, exclude=None):
+        """int64 [len(users) x topn]: the top-``topn`` of all items for each user, best first, leaving out the stored
+        entries of row ``users[k]`` of ``exclude`` (users x items like X, any SciPy format or a DeviceCSR; every stored
+        entry excludes its item whatever its value). Ties go to the lower item id, and a user with fewer than ``topn``
+        unseen items gets -1 in the rest of its row. The scores are those of ``predict`` (float64, bitwise), ranked on
+        the device without rounding to float32."""
+        X, W = self._X_and_W()
+        users = np.ascontiguousarray(users, dtype=np.int64).reshape(-1)
+        if len(users) and (users.min() < 0 or users.max() >= X.shape[0]):
+            raise ValueError(f"user ids must lie in [0, {X.shape[0]}) (the rows of X)")
+        if exclude is not None and tuple(exclude.shape) != tuple(X.shape):
+            raise ValueError(f"exclude has shape {tuple(exclude.shape)}, X {tuple(X.shape)}")
+        topn = int(topn)
+        k = min(topn, X.shape[1])
+        out = np.full((len(users), topn), -1, dtype=np.int64)
+        if k <= 0 or len(users) == 0:
+            return out
+        ex = None
+        if exclude is not None:
+            ex = exclude if isinstance(exclude, DeviceCSR) else DeviceCSR.from_scipy(exclude, self.device)
+        out[:, :k] = self._recommend_ids(torch.from_numpy(users).to(self.device), k, ex).cpu().numpy()
+        return out
+
+    def _recommend_ids(self, users_d, k, ex):
+        """Device int64 [len(users_d) x k], k <= num_items: the device part of ``recommend`` (``ex``: a DeviceCSR with
+        rows in any order, or None to exclude nothing)."""
+        X, W = self._X_and_W()
+        if k <= _lib.TOPK_MAX:
+            return self._score_topk(X, W, users_d, k, exclude=ex)
+        n = X.shape[1]   # very long lists: the scores of predict, then stable device sorts
+        return sort_path_ids(users_d, n, k, ex, lambda chunk, items_d: self._predict_pairs(
+            X, W, chunk.repeat_interleave(n), items_d.repeat(chunk.numel())).view(chunk.numel(), n))
+
+    def eval_ranking(self, test_mat, topn=np.array([10]), exclude=None, users=None):
+        """Full-ranking quality of ``recommend``: for each cutoff k of ``topn`` (an int or at most 16 distinct positive
+        ints) a dict with "Recall@k", "Precision@k", "NDCG@k", "MAP@k" and "HitRate@k" (Python floats, means over the
+        evaluated users) and "users" (their number). Unlike ``eval_topn``, which ranks each held-out item against
+        ``rand_sampled`` random items and divides the hits by nnz(test), this ranks ALL items and averages per user.
+
+        The list of user u is ``recommend(users, K, exclude)`` with K = max(topn) (ties to the lower item id, -1
+        padding never a hit). T_u is the set of distinct columns of row u of ``test_mat`` with a stored non-zero value
+        (duplicates count once; unsorted rows and explicit zeros are fine), h_i the hits among the first i items:
+        Precision@k = h_k / k (k also when the list is padded), Recall@k = h_k / |T_u|, NDCG@k = the sum of
+        1/log2(i+1) over the hits at i <= k over the same sum over i <= min(k, |T_u|) (binary gains), MAP@k = the sum
+        of h_i / i over the hits at i <= k over min(k, |T_u|), HitRate@k = [h_k > 0]. Users with T_u empty are ranked
+        but not counted; an item both in ``exclude`` and in T_u counts in |T_u| and can never be hit.
+
+        ``test_mat`` and ``exclude`` (None: nothing excluded) are users x items SciPy matrices or DeviceCSRs of the
+        shape of X, uploaded once. ``users`` defaults to the rows of ``test_mat`` with stored entries; repeated entries
+        count each time. Lists, metrics and their sums stay on the device (the per-user rows are reduced once, in a
+        fixed order: the result is bitwise reproducible)."""
+        def dims():
+            X, _ = self._X_and_W()
+            if tuple(test_mat.shape) != tuple(X.shape):
+                raise ValueError(f"test_mat has shape {tuple(test_mat.shape)}, X {tuple(X.shape)}")
+            return X.shape[1], X.shape[0]
+        return eval_ranking(self._recommend_ids, dims, "the rows of X", self.device, test_mat, topn, exclude, users)

@@ -24,7 +24,6 @@ from .engine import DeviceCSR
 
 _ALGOS = {"auto": _lib.ALGO_AUTO, "simt": _lib.ALGO_SIMT, "tcgen05": _lib.ALGO_TCGEN05,
           "tcgen05_direct": _lib.ALGO_TCGEN05_DIRECT}
-_EVAL_CHUNK_IDS = ranking.EVAL_CHUNK_IDS
 
 
 class WMF(RecModel):
@@ -145,30 +144,7 @@ class WMF(RecModel):
         if ni == 0 or k == 0:
             return np.empty((len(users), 0), dtype=items.dtype)
         cand_d = torch.from_numpy(np.ascontiguousarray(items, dtype=np.int64)).to(self.device)
-        U, V = self.users_device, self.items_device
-        rank_id, world = sharding.dist_info()
-        if distributed and world > 1 and k <= _lib.TOPK_MAX:
-            per = -(-len(users) // world)
-            mine = users_d[rank_id * per:(rank_id + 1) * per]
-            local = torch.zeros((per, k), dtype=torch.int64, device=self.device)
-            if mine.numel():
-                local[:mine.numel()] = engine.score_topk(mine, cand_d, U, V, k, bias=self.bias is True)
-            ids = torch.empty((world * per, k), dtype=torch.int64, device=self.device)
-            torch.distributed.all_gather_into_tensor(ids, local)
-            ids = ids[:len(users)]
-        elif k <= _lib.TOPK_MAX:
-            ids = engine.score_topk(users_d, cand_d, U, V, k, bias=self.bias is True)
-        else:  # very long lists: exact device scores, then a stable device sort (ties by position), many users per pass
-            rows = []
-            per = max(1, (1 << 24) // ni)   # at most ~16 M (user, candidate) pairs in flight
-            for u0 in range(0, users_d.numel(), per):
-                chunk = users_d[u0:u0 + per]
-                pu = chunk.repeat_interleave(ni)
-                pi = cand_d.repeat(chunk.numel())
-                s = engine.predict_pairs(pu, pi, U, V, bias=self.bias is True).view(chunk.numel(), ni)
-                order = torch.sort(s, dim=1, descending=True, stable=True).indices[:, :k]
-                rows.append(cand_d[order])
-            ids = torch.cat(rows) if rows else torch.empty((0, k), dtype=torch.int64, device=self.device)
+        ids = self._rank_ids(users_d, cand_d, k, None, distributed)
         return ids.cpu().numpy().astype(items.dtype, copy=False)
 
     def recommend(self, users, topn, exclude=None, distributed=False):
@@ -200,30 +176,35 @@ class WMF(RecModel):
     def _recommend_ids(self, users_d, k, ex, distributed=False):
         """Device int64 [len(users_d) x k], k <= num_items: the device part of ``recommend`` (``ex``: a DeviceCSR with
         sorted rows, or None to exclude nothing, where the lists are those of ``rank_batch`` over all items)."""
-        V = self.items_device
-        ni = V.shape[0]
-        U, bias = self.users_device, self.bias is True
+        return self._rank_ids(users_d, None, k, ex, distributed)
+
+    def _rank_ids(self, users_d, cand_d, k, ex, distributed):
+        """Device int64 [len(users_d) x k]: the lists of ``rank_batch`` over the device candidate ids ``cand_d`` (None:
+        all items), or, with ``ex`` (a DeviceCSR with sorted rows; needs ``cand_d`` None), those of ``recommend``.
+        ``distributed`` as in ``rank_batch``; lists longer than TOPK_MAX are ranked locally."""
+        U, V, bias = self.users_device, self.items_device, self.bias is True
+        if k > _lib.TOPK_MAX:  # very long lists: exact device scores, then stable device sorts, many users per pass
+            ni = V.shape[0] if cand_d is None else cand_d.numel()
+            return ranking.sort_path_ids(users_d, ni, k, ex, lambda chunk, items_d: engine.predict_pairs(
+                chunk.repeat_interleave(ni), items_d.repeat(chunk.numel()), U, V, bias=bias).view(chunk.numel(), ni),
+                cand_d)
 
         def topk(u):
             if ex is None:
-                return engine.score_topk(u, None, U, V, k, bias=bias)
+                return engine.score_topk(u, cand_d, U, V, k, bias=bias)
             return engine.score_topk_exclude(u, ex, U, V, k, bias=bias)[0]
 
         rank_id, world = sharding.dist_info()
-        if distributed and world > 1 and k <= _lib.TOPK_MAX:
-            per = -(-users_d.numel() // world)
-            mine = users_d[rank_id * per:(rank_id + 1) * per]
-            local = torch.full((per, k), -1, dtype=torch.int64, device=self.device)
-            if mine.numel():
-                local[:mine.numel()] = topk(mine)
-            ids = torch.empty((world * per, k), dtype=torch.int64, device=self.device)
-            torch.distributed.all_gather_into_tensor(ids, local)
-            return ids[:users_d.numel()]
-        if k <= _lib.TOPK_MAX:
+        if not (distributed and world > 1):
             return topk(users_d)
-        # very long lists: exact device scores, then stable device sorts with the excluded entries regrouped last
-        return ranking.sort_path_ids(users_d, ni, k, ex, lambda chunk, items_d: engine.predict_pairs(
-            chunk.repeat_interleave(ni), items_d.repeat(chunk.numel()), U, V, bias=bias).view(chunk.numel(), ni))
+        per = -(-users_d.numel() // world)
+        mine = users_d[rank_id * per:(rank_id + 1) * per]
+        local = torch.full((per, k), -1, dtype=torch.int64, device=self.device)
+        if mine.numel():
+            local[:mine.numel()] = topk(mine)
+        ids = torch.empty((world * per, k), dtype=torch.int64, device=self.device)
+        torch.distributed.all_gather_into_tensor(ids, local)
+        return ids[:users_d.numel()]
 
     def eval_ranking(self, test_mat, topn=np.array([10]), exclude=None, users=None, distributed=False):
         """Full-ranking quality of ``recommend``: for each cutoff k of ``topn`` (an int or at most 16 distinct positive
@@ -247,7 +228,7 @@ class WMF(RecModel):
         return ranking.eval_ranking(
             lambda users_d, k, ex: self._recommend_ids(users_d, k, None if ex is None else ex.sorted(), distributed),
             lambda: (self.items_device.shape[0], self.users_device.shape[0]),
-            "the rows of test_mat and of the user factors", self.device, test_mat, topn, exclude, users, _EVAL_CHUNK_IDS)
+            "the rows of test_mat and of the user factors", self.device, test_mat, topn, exclude, users)
 
     # ---------------------------------------------------------------- train (R2, R7, R11)
     def train(self, utility_mat, iterations, verbose=0, eval_mat=None, count_mat=None, alpha=10,

@@ -8,7 +8,7 @@ import torch
 
 from conftest import csr_from, load_golden
 from test_gpu_eval_ranking import oracle_means, oracle_per_user
-from recmodel_b200 import _lib, build, engine, ease_model, utils
+from recmodel_b200 import _lib, build, engine, ranking, utils
 from recmodel_b200.ease_model import Ease
 from recmodel_b200.engine import DeviceCSR
 from recmodel_b200.synthetic import make_counts, split_train_test
@@ -159,7 +159,7 @@ def test_scores_and_lists_independent_of_the_batch(cuda_device, trained):
 
 @gpu
 @pytest.mark.parametrize("ks", [[10, 50, 5], [1200, 10]])    # the second: the sort path and padding past the items
-def test_eval_ranking_equals_the_definitions(cuda_device, monkeypatch, ks):
+def test_eval_ranking_equals_the_definitions_in_any_chunking(cuda_device, monkeypatch, ks):
     full = make_counts(2000, N_ITEMS, 60_000, seed=8, planted_rank=6)
     Train, Test = split_train_test(full)
     m = Ease(num_items=N_ITEMS, num_users=2000)
@@ -183,9 +183,13 @@ def test_eval_ranking_equals_the_definitions(cuda_device, monkeypatch, ks):
     assert res[f"Recall@{K}"] > 0
     assert m.eval_ranking(DeviceCSR.from_scipy(Test, cuda_device), topn=ks,
                           exclude=DeviceCSR.from_scipy(Train, cuda_device)) == res
+    real, calls = engine.topn_metrics, []
+    monkeypatch.setattr(engine, "topn_metrics", lambda *a, **kw: calls.append(1) or real(*a, **kw))
     for chunk in (K * 13, 1):     # chunks of 13 users, then 1 user
-        monkeypatch.setattr(ease_model, "_EVAL_CHUNK_IDS", chunk)
+        monkeypatch.setattr(ranking, "EVAL_CHUNK_IDS", chunk)
+        calls.clear()
         assert m.eval_ranking(Test, topn=ks, exclude=Train) == res
+        assert len(calls) == -(-len(users) // max(1, chunk // K))   # one metrics call per chunk
 
 
 @gpu

@@ -14,7 +14,7 @@ import torch
 
 from conftest import ROOT
 from oracle import wmf_oracle as orc
-from recmodel_b200 import WMF, _lib, build, engine, wmf_model
+from recmodel_b200 import WMF, _lib, build, engine, ranking
 from recmodel_b200.engine import DeviceCSR
 
 gpu = pytest.mark.gpu
@@ -195,18 +195,22 @@ def test_hand_built_closed_form(cuda_device):
 
 
 @gpu
-def test_eval_ranking_reproducible_and_chunk_independent(cuda_device, monkeypatch):
+def test_eval_ranking_reproducible_at_every_chunk_size(cuda_device, monkeypatch):
     ni, nu, ks = 4096, 300, np.array([10, 50, 3])
     m, U, V = make_model(64, False, ni, nu, seed=9)
     X, Test = make_data(U, V, False, 50, seed=9)
     a = m.eval_ranking(Test, topn=ks, exclude=X)
     b = m.eval_ranking(DeviceCSR.from_scipy(Test, cuda_device), topn=ks, exclude=DeviceCSR.from_scipy(X, cuda_device))
     assert a == b
-    for ids in (50 * 7, 50, 1):       # chunks of 7 users, then 1 user
-        monkeypatch.setattr(wmf_model, "_EVAL_CHUNK_IDS", ids)
-        assert m.eval_ranking(Test, topn=ks, exclude=X) == a
-    monkeypatch.undo()
     users = np.flatnonzero(np.diff(Test.indptr) > 0)
+    real, calls = engine.topn_metrics, []
+    monkeypatch.setattr(engine, "topn_metrics", lambda *a, **kw: calls.append(1) or real(*a, **kw))
+    for ids in (50 * 7, 50, 1):       # chunks of 7 users, then 1 user
+        monkeypatch.setattr(ranking, "EVAL_CHUNK_IDS", ids)
+        calls.clear()
+        assert m.eval_ranking(Test, topn=ks, exclude=X) == a
+        assert len(calls) == -(-len(users) // max(1, ids // 50))   # one metrics call per chunk
+    monkeypatch.undo()
     assert a["users"] == oracle_means(oracle_per_user(m.recommend(users, 50, exclude=X), users, Test, ks), ks)["users"]
     # nothing excluded: the lists are recommend(users, K) = rank_batch over all items
     c = m.eval_ranking(Test, topn=ks)
@@ -279,7 +283,7 @@ WORKER = r"""
 import os, sys
 sys.path.insert(0, {root!r})
 import numpy as np, scipy.sparse, torch, torch.distributed as dist
-from recmodel_b200 import WMF, wmf_model
+from recmodel_b200 import WMF, engine, ranking
 rank, local = int(os.environ["RANK"]), int(os.environ["LOCAL_RANK"])
 torch.cuda.set_device(local)
 dist.init_process_group("nccl", device_id=torch.device("cuda", local))
@@ -294,8 +298,11 @@ for ks in ([10, 50], [700, 3]):
     a = m.eval_ranking(T, topn=ks, exclude=X, distributed=True)
     b = m.eval_ranking(T, topn=ks, exclude=X)
     assert a == b, (ks, a, b)
-wmf_model._EVAL_CHUNK_IDS = 50 * 97
+ranking.EVAL_CHUNK_IDS = 50 * 97
+real, calls = engine.topn_metrics, []
+engine.topn_metrics = lambda *a, **kw: calls.append(1) or real(*a, **kw)
 assert m.eval_ranking(T, topn=[10, 50], exclude=X, distributed=True) == m.eval_ranking(T, topn=[10, 50], exclude=X)
+assert len(calls) == 2 * -(-int((np.diff(T.indptr) > 0).sum()) // 97), len(calls)   # chunks of 97 users, both calls
 dist.barrier()
 dist.destroy_process_group()
 print("ok", rank)

@@ -7,7 +7,7 @@ import scipy.sparse
 import torch
 
 from test_gpu_eval_ranking import oracle_means, oracle_per_user
-from recmodel_b200 import ItemKNN, _lib, build, engine, knn_model, utils
+from recmodel_b200 import ItemKNN, _lib, build, engine, ranking, utils
 from recmodel_b200.engine import DeviceCSR
 from recmodel_b200.synthetic import make_counts, split_train_test
 
@@ -292,7 +292,7 @@ def test_lists_independent_of_the_batch(cuda_device, trained):
 
 @gpu
 @pytest.mark.parametrize("ks", [[10, 50, 5], [1200, 10]])    # the second: the sort path and padding past the items
-def test_eval_ranking_equals_the_definitions(cuda_device, monkeypatch, ks):
+def test_eval_ranking_equals_the_definitions_in_any_chunking(cuda_device, monkeypatch, ks):
     full = make_counts(2000, N_ITEMS, 60_000, seed=8, planted_rank=6)
     Train, Test = split_train_test(full)
     m = ItemKNN(num_items=N_ITEMS, num_users=2000)
@@ -313,9 +313,13 @@ def test_eval_ranking_equals_the_definitions(cuda_device, monkeypatch, ks):
     for key in means:
         np.testing.assert_allclose(res[key], means[key], rtol=1e-12, atol=1e-15)
     assert res[f"Recall@{K}"] > 0
+    real, calls = engine.topn_metrics, []
+    monkeypatch.setattr(engine, "topn_metrics", lambda *a, **kw: calls.append(1) or real(*a, **kw))
     for chunk in (K * 13, 1):
-        monkeypatch.setattr(knn_model, "_EVAL_CHUNK_IDS", chunk)
+        monkeypatch.setattr(ranking, "EVAL_CHUNK_IDS", chunk)
+        calls.clear()
         assert m.eval_ranking(Test, topn=ks, exclude=Train) == res
+        assert len(calls) == -(-len(users) // max(1, chunk // K))   # one metrics call per chunk
 
 
 @gpu

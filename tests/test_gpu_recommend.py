@@ -148,6 +148,28 @@ def test_recommend_without_exclusion_is_rank_batch(cuda_device):
     np.testing.assert_array_equal(m.recommend(users, 50, exclude=ex), m.rank_batch(np.arange(3000), users, 50))
 
 
+def test_rank_batch_sort_path_maps_positions_to_candidate_ids(cuda_device):
+    """topn > 1024 over a permuted subset of the items: the stable device sort ranks candidate positions, and the lists
+    must report the candidates' ids, an exact tie in candidate order."""
+    ni, nu, topn = 3000, 24, 1500
+    m, U, V = make_model(64, False, ni, nu, seed=17)
+    cand = np.random.default_rng(17).permutation(ni)[:2400]
+    p, q = 5, 2000                                  # a tie between positions 5 and 2000, the later id first in cand
+    if cand[p] < cand[q]:
+        cand[[p, q]] = cand[[q, p]]
+    V[cand[q]] = V[cand[p]]
+    m.items = V
+    got = m.rank_batch(cand, np.arange(nu), topn)
+    assert got.shape == (nu, topn) and got.dtype == cand.dtype
+    tied = 0
+    for u in range(nu):
+        s = m.predict(np.full(len(cand), u), cand)
+        assert s[p] == s[q]
+        np.testing.assert_array_equal(got[u], cand[np.argsort(-s, kind="stable")][:topn])
+        tied += np.isin(cand[[p, q]], got[u]).all()
+    assert tied > 0                                 # the tie is inside some lists
+
+
 def test_recommend_all_equal_scores_overflow(cuda_device):
     """All scores equal: every candidate list overflows, the exact kernels redo the call (counted in fixup_users),
     and ties go to the lowest unseen item ids."""

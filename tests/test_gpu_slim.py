@@ -10,7 +10,7 @@ import torch
 from test_gpu_eval_ranking import oracle_means, oracle_per_user
 from test_gpu_itemknn import (EMPTY_ITEM, EMPTY_USER, N_ITEMS, canonical, make_X, messy_csr, oracle_lists,
                               oracle_neighbors, oracle_scores, seen_lists)
-from recmodel_b200 import SLIM, _lib, build, knn_model, utils
+from recmodel_b200 import SLIM, _lib, build, engine, ranking, utils
 from recmodel_b200.synthetic import make_counts, split_train_test
 
 gpu = pytest.mark.gpu
@@ -289,7 +289,7 @@ def test_recommend_equals_the_oracle(cuda_device, trained, topn):
 
 
 @gpu
-def test_eval_ranking_equals_the_definitions(cuda_device, monkeypatch):
+def test_eval_ranking_equals_the_definitions_in_any_chunking(cuda_device, monkeypatch):
     ks = [10, 50, 5]
     full = make_counts(2000, N_ITEMS, 60_000, seed=8, planted_rank=6)
     Train, Test = split_train_test(full)
@@ -304,8 +304,11 @@ def test_eval_ranking_equals_the_definitions(cuda_device, monkeypatch):
     for key in means:
         np.testing.assert_allclose(res[key], means[key], rtol=1e-12, atol=1e-15)
     assert res["Recall@50"] > 0
-    monkeypatch.setattr(knn_model, "_EVAL_CHUNK_IDS", 1)
+    real, calls = engine.topn_metrics, []
+    monkeypatch.setattr(engine, "topn_metrics", lambda *a, **kw: calls.append(1) or real(*a, **kw))
+    monkeypatch.setattr(ranking, "EVAL_CHUNK_IDS", 1)
     assert m.eval_ranking(Test, topn=ks, exclude=Train) == res
+    assert len(calls) == len(users)   # chunks of 1 user
 
 
 @gpu
