@@ -275,7 +275,9 @@ int wmf_ease_score_topk(const int64_t* x_indptr, const int32_t* x_indices, const
  * w_indices / w_data with room for n * min(k, n) entries, of which the first w_indptr[n] are used. xt_indptr /
  * xt_indices: the CSR of X^T (wmf_csr_transpose). 1 <= k <= 1024, similarity one of WMF_KNN_*, shrink finite and
  * >= 0, 0 < n < 2^31: else WMF_ERR_INVALID before any CUDA call. The workspace holds an int32 and a double [B x n]
- * tile (B item rows from n and a fixed byte budget) and the selected rows of all n items.
+ * tile (B item rows from n and a fixed byte budget) and the selected rows of all n items. Called with the roles of X
+ * and X^T swapped (x_* = the CSR of X^T, rows = the item count, xt_* = the CSR of X, n = the user count), it writes
+ * the user-user neighbours of UserKNN: c_ab is then the number of items users a and b share.
  * wmf_knn_predict: out[k] = s(users[k*user_stride], items[k]); user_stride 0 broadcasts one user. The score
  * s(u, i) is the sum over the entries j of row u of X, in ascending j, from +0.0, of (double)x_uj * W[j, i], each
  * product and each addition rounded to nearest; an item no entry of W votes for scores +0.0. W is any n x n CSR
@@ -298,6 +300,31 @@ int wmf_knn_score_topk(const int64_t* x_indptr, const int32_t* x_indices, const 
                        const int32_t* w_indices, const double* w_data, int64_t n, const int64_t* users, int64_t nu,
                        const int64_t* ex_indptr, const int32_t* ex_indices, int topn, int64_t* out_ids,
                        double* out_scores, void* ws, size_t ws_bytes, void* stream);
+
+/* UserKNN: a user-user neighbourhood model (DESIGN.md 4.8), defined here, not ported. X is the canonical interaction
+ * matrix of the knn entries above (users x n items; sorted rows, no duplicates, no explicit zeros: not checked, a
+ * duplicate item in a row would race in the score tile). nb_indptr / nb_indices / nb_data: the neighbour CSR N, one
+ * row per user of X with sorted column indices (user ids) and double similarities, as wmf_knn_train writes it for
+ * (X^T, X).
+ * wmf_userknn_predict: out[k] = s(users[k*user_stride], items[k]); user_stride 0 broadcasts one user. The score
+ * s(u, i) is the sum over the entries v of row u of N, in ascending v, from +0.0, of sim(u, v) * (double)x_vi, each
+ * product and each addition rounded to nearest; an item no neighbour of u has scores +0.0. count < 0 or
+ * user_stride < 0: WMF_ERR_INVALID, count 0: WMF_OK with nothing read; a null pointer otherwise: WMF_ERR_INVALID.
+ * All before any CUDA call.
+ * wmf_userknn_score_topk: wmf_knn_score_topk's contract (exclusion CSR by user id, descending scores, ties to the
+ * lower item id, -1 / NaN padding, 1 <= topn <= min(n, 1024) else WMF_ERR_UNSUPPORTED, the same order of checks)
+ * with the scores of wmf_userknn_predict, bitwise. n is the item count. The workspace
+ * (wmf_userknn_score_topk_workspace_bytes, 0 for nu <= 0 or n outside 1..2^31-1) holds one [ub x n] double score
+ * tile, ub from n and a fixed byte budget. */
+int wmf_userknn_predict(const int64_t* x_indptr, const int32_t* x_indices, const float* x_data,
+                        const int64_t* nb_indptr, const int32_t* nb_indices, const double* nb_data,
+                        const int64_t* users, int64_t user_stride, const int64_t* items, int64_t count, double* out,
+                        void* stream);
+size_t wmf_userknn_score_topk_workspace_bytes(int64_t nu, int64_t n, int topn);
+int wmf_userknn_score_topk(const int64_t* x_indptr, const int32_t* x_indices, const float* x_data,
+                           const int64_t* nb_indptr, const int32_t* nb_indices, const double* nb_data, int64_t n,
+                           const int64_t* users, int64_t nu, const int64_t* ex_indptr, const int32_t* ex_indices,
+                           int topn, int64_t* out_ids, double* out_scores, void* ws, size_t ws_bytes, void* stream);
 
 /* SLIM: sparse non-negative item-item regression (DESIGN.md 4.7). No reference call site: the SLIM sources of
  * RecModel are not part of this repository, and this model is defined here, not ported.

@@ -2,8 +2,8 @@
 titoeb/RecModel behind the reference's own ``WMF`` class API. See DESIGN.md."""
 from .wmf_model import WMF, WMFModel  # noqa: F401
 from .ease_model import Ease  # noqa: F401
-from .knn_model import ItemKNN  # noqa: F401
+from .knn_model import ItemKNN, UserKNN  # noqa: F401
 from .slim_model import SLIM  # noqa: F401
 from .utils import test_coverage, train_test_split_sparse_mat  # noqa: F401
 
-__all__ = ["WMF", "WMFModel", "Ease", "ItemKNN", "SLIM", "train_test_split_sparse_mat", "test_coverage"]
+__all__ = ["WMF", "WMFModel", "Ease", "ItemKNN", "UserKNN", "SLIM", "train_test_split_sparse_mat", "test_coverage"]

@@ -70,6 +70,9 @@ SIGNATURES = {
     "wmf_knn_predict": (_i32, [_p, _p, _p, _p, _p, _p, _p, _i64, _p, _i64, _p, _p]),
     "wmf_knn_score_topk_workspace_bytes": (_sz, [_i64, _i64, _i32]),
     "wmf_knn_score_topk": (_i32, [_p, _p, _p, _p, _p, _p, _i64, _p, _i64, _p, _p, _i32, _p, _p, _p, _sz, _p]),
+    "wmf_userknn_predict": (_i32, [_p, _p, _p, _p, _p, _p, _p, _i64, _p, _i64, _p, _p]),
+    "wmf_userknn_score_topk_workspace_bytes": (_sz, [_i64, _i64, _i32]),
+    "wmf_userknn_score_topk": (_i32, [_p, _p, _p, _p, _p, _p, _i64, _p, _i64, _p, _p, _i32, _p, _p, _p, _sz, _p]),
     "wmf_slim_train_workspace_bytes": (_sz, [_i64, _i32]),
     "wmf_slim_train": (_i32, [_p, _p, _i64, _p, _p, _i64, _p, _p, _i32, _f64, _f64, _i32, _f64, _p, _p, _p, _p, _p, _sz,
                               _p]),

@@ -8,6 +8,8 @@
 // SLIM (DESIGN.md 4.7) shares the counts, the staging-to-CSR kernels and the scoring: the dense G = P^T P comes from
 // knn_cooc_kernel over all n rows, slim_cd_kernel solves each column's regression on chip, and knn_scan_kernel plus
 // knn_compact_kernel write the CSR of W^T.
+// UserKNN (DESIGN.md 4.8) trains with wmf_knn_train on (X^T, X) and scores with userknn_score_tile_kernel and
+// userknn_predict_kernel, which walk the neighbours' rows of X.
 #include "common.cuh"
 #include "score.cuh"
 
@@ -196,6 +198,69 @@ __global__ __launch_bounds__(KN_THREADS) void knn_predict_kernel(
             if (w_indices[mid] < it) lo = mid + 1; else hi = mid;
         }
         if (lo < w_indptr[j + 1] && w_indices[lo] == it) acc = __dadd_rn(acc, __dmul_rn((double)x_data[e], w_data[lo]));
+    }
+    out[k] = acc;
+}
+
+// ---- UserKNN (DESIGN.md 4.8): the neighbour CSR N (n_users x n_users) is wmf_knn_train's W for (X^T, X), and a
+// user's neighbours vote through their rows of X: s(u, i) = sum over v of row u of N, ascending, of sim(u, v) x_vi.
+
+// S[r][i] = s(users[u_begin + r], i) on a zeroed [ub x n] tile. One CTA per user: the neighbours v of row u of N are
+// staged KN_THREADS at a time (X row bounds, similarity) in shared memory, then walked in ascending v with the
+// threads over the entries of X row v, which are distinct items. X rows are long-tailed (thousands of entries), so a
+// whole CTA walks each one. The __syncthreads between rows v orders the read-modify-writes of one item, so every
+// score is summed from +0.0 in ascending v without atomics: the sum of userknn_predict_kernel.
+__global__ __launch_bounds__(KN_THREADS) void userknn_score_tile_kernel(
+    const int64_t* __restrict__ x_indptr, const int32_t* __restrict__ x_indices, const float* __restrict__ x_data,
+    const int64_t* __restrict__ nb_indptr, const int32_t* __restrict__ nb_indices, const double* __restrict__ nb_data,
+    int64_t n, const int64_t* __restrict__ users, int64_t u_begin, double* S) {
+    __shared__ int64_t s_lo[KN_THREADS], s_hi[KN_THREADS];
+    __shared__ double s_sim[KN_THREADS];
+    const int64_t r = blockIdx.x;
+    const int64_t u = users[u_begin + r];
+    const int64_t hi = nb_indptr[u + 1];
+    double* srow = S + r * n;
+    for (int64_t e0 = nb_indptr[u]; e0 < hi; e0 += KN_THREADS) {
+        const int m = (int)(hi - e0 < KN_THREADS ? hi - e0 : KN_THREADS);
+        if ((int)threadIdx.x < m) {
+            const int32_t v = nb_indices[e0 + threadIdx.x];
+            s_lo[threadIdx.x] = x_indptr[v];
+            s_hi[threadIdx.x] = x_indptr[v + 1];
+            s_sim[threadIdx.x] = nb_data[e0 + threadIdx.x];
+        }
+        __syncthreads();
+        for (int q = 0; q < m; ++q) {
+            const double sim = s_sim[q];
+            const int64_t end = s_hi[q];
+            for (int64_t t = s_lo[q] + threadIdx.x; t < end; t += KN_THREADS) {
+                const int32_t i = x_indices[t];
+                srow[i] = __dadd_rn(srow[i], __dmul_rn(sim, (double)x_data[t]));
+            }
+            __syncthreads();   // also ends the reads of the staged chunk before the next one overwrites it
+        }
+    }
+}
+
+// out[k] = s(users[k * user_stride], items[k]): row u of N in ascending v, a binary search of the item in X row v
+__global__ __launch_bounds__(KN_THREADS) void userknn_predict_kernel(
+    const int64_t* __restrict__ x_indptr, const int32_t* __restrict__ x_indices, const float* __restrict__ x_data,
+    const int64_t* __restrict__ nb_indptr, const int32_t* __restrict__ nb_indices, const double* __restrict__ nb_data,
+    const int64_t* __restrict__ users, int64_t user_stride, const int64_t* __restrict__ items, int64_t count,
+    double* __restrict__ out) {
+    const int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= count) return;
+    const int64_t u = users[k * user_stride];
+    const int32_t it = (int32_t)items[k];
+    double acc = 0.0;
+    for (int64_t e = nb_indptr[u]; e < nb_indptr[u + 1]; ++e) {
+        const int32_t v = nb_indices[e];
+        int64_t lo = x_indptr[v], hi = x_indptr[v + 1];   // first entry >= it
+        while (lo < hi) {
+            const int64_t mid = (lo + hi) >> 1;
+            if (x_indices[mid] < it) lo = mid + 1; else hi = mid;
+        }
+        if (lo < x_indptr[v + 1] && x_indices[lo] == it)
+            acc = __dadd_rn(acc, __dmul_rn(nb_data[e], (double)x_data[lo]));
     }
     out[k] = acc;
 }
@@ -457,6 +522,39 @@ int wmf_knn_score_topk(const int64_t* x_indptr, const int32_t* x_indices, const 
         knn_score_tile_kernel<<<(unsigned)((ub + KN_THREADS / 32 - 1) / (KN_THREADS / 32)), KN_THREADS, 0, st>>>(
             x_indptr, x_indices, x_data, w_indptr, w_indices, w_data, n, users, u0, ub, S);
         WMF_LAUNCH_CHECK("knn_score_tile_kernel");
+        return WMF_OK;
+    });
+}
+
+int wmf_userknn_predict(const int64_t* x_indptr, const int32_t* x_indices, const float* x_data,
+                        const int64_t* nb_indptr, const int32_t* nb_indices, const double* nb_data,
+                        const int64_t* users, int64_t user_stride, const int64_t* items, int64_t count, double* out,
+                        void* stream) {
+    WMF_REQUIRE(count >= 0 && user_stride >= 0, "wmf_userknn_predict: bad arguments");
+    if (count == 0) return WMF_OK;
+    WMF_REQUIRE(x_indptr && nb_indptr && users && items && out, "wmf_userknn_predict: null argument");
+    userknn_predict_kernel<<<(unsigned)((count + KN_THREADS - 1) / KN_THREADS), KN_THREADS, 0, (cudaStream_t)stream>>>(
+        x_indptr, x_indices, x_data, nb_indptr, nb_indices, nb_data, users, user_stride, items, count, out);
+    WMF_LAUNCH_CHECK("userknn_predict_kernel");
+    return WMF_OK;
+}
+
+size_t wmf_userknn_score_topk_workspace_bytes(int64_t nu, int64_t n, int topn) {
+    (void)topn;
+    return score_topk_double_workspace_bytes(nu, n, knn_batch);
+}
+
+int wmf_userknn_score_topk(const int64_t* x_indptr, const int32_t* x_indices, const float* x_data,
+                           const int64_t* nb_indptr, const int32_t* nb_indices, const double* nb_data, int64_t n,
+                           const int64_t* users, int64_t nu, const int64_t* ex_indptr, const int32_t* ex_indices,
+                           int topn, int64_t* out_ids, double* out_scores, void* ws, size_t ws_bytes, void* stream) {
+    return score_topk_double("wmf_userknn_score_topk", x_indptr && nb_indptr, knn_batch, n, users, nu, ex_indptr,
+                             ex_indices, topn, out_ids, out_scores, ws, ws_bytes, stream,
+                             [&](int64_t u0, int ub, double* S, cudaStream_t st) {
+        WMF_CUDA(cudaMemsetAsync(S, 0, (size_t)ub * n * sizeof(double), st));
+        userknn_score_tile_kernel<<<(unsigned)ub, KN_THREADS, 0, st>>>(x_indptr, x_indices, x_data, nb_indptr,
+                                                                      nb_indices, nb_data, n, users, u0, S);
+        WMF_LAUNCH_CHECK("userknn_score_tile_kernel");
         return WMF_OK;
     });
 }

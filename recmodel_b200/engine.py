@@ -660,7 +660,8 @@ def ease_score_topk(X_csr, W, users, topn, exclude=None, want_scores=False):
 def knn_train(X_csr, XT_csr, k, similarity, shrink):
     """The ItemKNN neighbours of the canonical interaction matrix ``X_csr`` (sorted rows, no duplicates, no explicit
     zeros; ``XT_csr`` its transpose): (indptr int64 [n+1], indices int32, data float64) of the n x n CSR W, rows
-    sorted by id (include/wmf_b200.h: wmf_knn_train). ``similarity``: a key of ``_lib.KNN_SIMILARITIES``."""
+    sorted by id (include/wmf_b200.h: wmf_knn_train). ``similarity``: a key of ``_lib.KNN_SIMILARITIES``. Called as
+    ``knn_train(X.transpose(), X, ...)`` it returns the UserKNN neighbours of X (n = the number of users)."""
     lib = _lib.load()
     n = X_csr.shape[1]
     dev = X_csr.device
@@ -719,6 +720,50 @@ def knn_score_topk(X_csr, W, users, topn, exclude=None, want_scores=False):
                                       _ptr(None if exclude is None else exclude.indptr),
                                       _ptr(None if exclude is None else exclude.indices), int(topn), _ptr(ids),
                                       _ptr(scores), _ptr(ws), ws.numel(), _stream()), "wmf_knn_score_topk")
+    return (ids, scores) if want_scores else ids
+
+
+@_device_of(0)
+def userknn_predict(X_csr, N, users, items):
+    """float64 UserKNN scores s(users[k], items[k]) (include/wmf_b200.h: wmf_userknn_predict) for the canonical
+    ``X_csr`` and the user-user neighbours N = (indptr, indices, data) as ``knn_train(X_csr.transpose(), X_csr, ...)``
+    returns them; one user broadcasts."""
+    lib = _lib.load()
+    nb_indptr, nb_indices, nb_data = N
+    n = items.numel()
+    stride = 1
+    if users.numel() == 1 and n != 1:
+        stride = 0
+    elif users.numel() != n:
+        raise ValueError("users and items need to have the same length or only one user needs to be provided.")
+    out = torch.empty(n, dtype=torch.float64, device=nb_indptr.device)
+    _lib.check(lib.wmf_userknn_predict(_ptr(X_csr.indptr), _ptr(X_csr.indices), _ptr(X_csr.data), _ptr(nb_indptr),
+                                       _ptr(nb_indices), _ptr(nb_data), _ptr(users), stride, _ptr(items), n, _ptr(out),
+                                       _stream()), "wmf_userknn_predict")
+    return out
+
+
+@_device_of(0)
+def userknn_score_topk(X_csr, N, users, topn, exclude=None, want_scores=False):
+    """``knn_score_topk`` for the UserKNN scores of ``userknn_predict`` (bitwise): top-``topn`` item ids [nu x topn]
+    (int64) over all items minus the stored entries of row ``users[k]`` of ``exclude``, best first, ties to the lower
+    item id, -1 padding (include/wmf_b200.h: wmf_userknn_score_topk); with ``want_scores`` (ids, float64 scores)."""
+    lib = _lib.load()
+    nb_indptr, nb_indices, nb_data = N
+    n = X_csr.shape[1]
+    nu = users.numel()
+    dev = nb_indptr.device
+    assert users.dtype == torch.int64 and nb_indptr.numel() - 1 == X_csr.shape[0]
+    if exclude is not None:
+        assert exclude.shape[1] == n and exclude.indices.dtype == torch.int32 and exclude.indptr.dtype == torch.int64
+    ids = torch.empty((nu, topn), dtype=torch.int64, device=dev)
+    scores = torch.empty((nu, topn), dtype=torch.float64, device=dev) if want_scores else None
+    ws = workspace(lib.wmf_userknn_score_topk_workspace_bytes(nu, n, topn), dev)
+    _lib.check(lib.wmf_userknn_score_topk(_ptr(X_csr.indptr), _ptr(X_csr.indices), _ptr(X_csr.data), _ptr(nb_indptr),
+                                          _ptr(nb_indices), _ptr(nb_data), n, _ptr(users), nu,
+                                          _ptr(None if exclude is None else exclude.indptr),
+                                          _ptr(None if exclude is None else exclude.indices), int(topn), _ptr(ids),
+                                          _ptr(scores), _ptr(ws), ws.numel(), _stream()), "wmf_userknn_score_topk")
     return (ids, scores) if want_scores else ids
 
 

@@ -1,5 +1,6 @@
-"""ItemKNN: an item-item neighbourhood model trained, scored and ranked on the device (DESIGN.md 4.6), and
-``ItemItemModel``, the scoring half it shares with ``SLIM`` (slim_model.py).
+"""ItemKNN: an item-item neighbourhood model trained, scored and ranked on the device (DESIGN.md 4.6), UserKNN, its
+user-user counterpart (DESIGN.md 4.8), and ``ItemItemModel``, the scoring half both share with ``SLIM``
+(slim_model.py).
 
 ``ItemKNN(num_items, num_users)``, ``train(X, k, similarity, shrink, verbose, cores)``, ``predict(users, items)``,
 ``rank(items, users, topn)``, ``recommend`` (top-N over each user's unseen items for many users in one device call),
@@ -30,13 +31,27 @@ def _canonical(M):
     return M
 
 
+def _check_knn_args(k, similarity, shrink):
+    """shrink as a float; ValueError for an unknown similarity, a k outside 1..1024 or a shrink not finite and >= 0."""
+    if similarity not in _lib.KNN_SIMILARITIES:
+        raise ValueError(f"similarity must be one of {sorted(_lib.KNN_SIMILARITIES)}, got {similarity!r}")
+    if isinstance(k, (bool, np.bool_)) or not isinstance(k, (int, np.integer)) or not 1 <= k <= _lib.TOPK_MAX:
+        raise ValueError(f"k must be an int in 1..{_lib.TOPK_MAX}, got {k!r}")
+    shrink = float(shrink)
+    if not (math.isfinite(shrink) and shrink >= 0.0):
+        raise ValueError(f"shrink must be finite and >= 0, got {shrink}")
+    return shrink
+
+
 class ItemItemModel(XWRanking, RecModel):
     """The scoring half shared by the item-item models (``ItemKNN``, ``SLIM``): the canonical X and an n x n item
     weight CSR W on the device, and ``predict`` and ``rank`` over s(u, i) = sum over the entries j of row u of X,
     ascending, of x_uj * W[j, i]; ``recommend`` and ``eval_ranking`` rank these scores (``ranking.XWRanking``). A
-    subclass trains W and names it (``_W_NAME``, the attribute a user sets)."""
+    subclass trains W and names it (``_W_NAME``, the attribute a user sets). ``UserKNN`` scores from a users x users W
+    instead: it names the axis of X whose size W must have (``_W_AXIS``) and its own engine functions."""
 
     _W_NAME = "W"
+    _W_AXIS = 1   # W is square over the columns of X (the items)
     _score_topk = staticmethod(engine.knn_score_topk)
     _predict_pairs = staticmethod(engine.knn_predict)
 
@@ -83,9 +98,9 @@ class ItemItemModel(XWRanking, RecModel):
         W = self._W_device()
         if W is None:
             raise ValueError(f"the model has no {self._W_NAME}: call train(X, ...) first")
-        if W[0].numel() - 1 != self._X.shape[1]:
+        if W[0].numel() - 1 != self._X.shape[self._W_AXIS]:
             raise ValueError(f"{self._W_NAME} is {W[0].numel() - 1} x {W[0].numel() - 1} but X has "
-                             f"{self._X.shape[1]} items")
+                             f"{self._X.shape[self._W_AXIS]} {('users', 'items')[self._W_AXIS]}")
         return self._X, W
 
     def predict(self, users, items):
@@ -103,7 +118,7 @@ class ItemItemModel(XWRanking, RecModel):
             return np.empty(0, dtype=np.float64)
         u = torch.from_numpy(users).to(self.device)
         i = torch.from_numpy(items).to(self.device)
-        return engine.knn_predict(X, W, u, i).cpu().numpy()
+        return self._predict_pairs(X, W, u, i).cpu().numpy()
 
     def rank(self, items, users, topn=None):
         """The candidate ``items`` for one user in descending ``predict`` order, ties by candidate position; the
@@ -138,19 +153,64 @@ class ItemKNN(ItemItemModel):
         "conditional" c_ab / (c_aa + shrink) = P(b | a) (not symmetric). The neighbours of a are the top-k items
         b != a with c_ab > 0 by sim(a, b), ties to the lower id (fewer when a has fewer such items); W[a, b] =
         sim(a, b) (``neighbors``). k in 1..1024 (k >= num_items keeps every candidate), shrink finite and >= 0."""
-        if similarity not in _lib.KNN_SIMILARITIES:
-            raise ValueError(f"similarity must be one of {sorted(_lib.KNN_SIMILARITIES)}, got {similarity!r}")
-        if isinstance(k, (bool, np.bool_)) or not isinstance(k, (int, np.integer)) or not 1 <= k <= _lib.TOPK_MAX:
-            raise ValueError(f"k must be an int in 1..{_lib.TOPK_MAX}, got {k!r}")
-        shrink = float(shrink)
-        if not (math.isfinite(shrink) and shrink >= 0.0):
-            raise ValueError(f"shrink must be finite and >= 0, got {shrink}")
+        shrink = _check_knn_args(k, similarity, shrink)
         Xc = _canonical(X)
         if verbose > 0:
             print("Compute the item neighbourhoods")
             start = time.time()
         self._X = DeviceCSR.from_scipy(Xc, self.device)
         self._W_d = engine.knn_train(self._X, self._X.transpose(), int(k), similarity, shrink)
+        self._W_h = None
+        if verbose > 0:
+            torch.cuda.synchronize(self.device)
+            print(f"Training took {time.time() - start} seconds!")
+
+
+class UserKNN(ItemItemModel):
+    """A user-user neighbourhood model (DESIGN.md 4.8): each user's top-k most similar users vote for their items."""
+
+    _W_NAME = "neighbors"
+    _W_AXIS = 0   # the neighbours are users x users
+    _score_topk = staticmethod(engine.userknn_score_topk)
+    _predict_pairs = staticmethod(engine.userknn_predict)
+
+    @property
+    def neighbors(self):
+        """The neighbours as a num_users x num_users SciPy CSR (float64, sorted indices): row u holds sim(u, v) for
+        the neighbours v of u. A host copy, made on first access. Assigning any square SciPy matrix (canonicalised:
+        duplicates summed, explicit zeros removed, indices sorted) replaces the model; it must have one row per row
+        of X."""
+        return self._W_host()
+
+    @neighbors.setter
+    def neighbors(self, value):
+        self._set_W(value)
+
+    def predict(self, users, items):
+        """float64 s(u, i) per (user, item) pair (one user broadcasts): the sum over the neighbours v of u, in
+        ascending v, from +0.0, of sim(u, v) * (double)x_vi with x_vi the float32 entry of the canonical X, each
+        product and each addition rounded to nearest; +0.0 when no neighbour of u has i."""
+        return super().predict(users, items)
+
+    def train(self, X, k=100, similarity="cosine", shrink=0.0, verbose=0, cores=1):
+        """Neighbours of every user from the users x items matrix X (any SciPy format, not modified).
+
+        X is canonicalised on the host (CSR, duplicates summed, explicit zeros removed, sorted rows); that copy is
+        kept for scoring. With P its binary pattern, c_ab = sum_i P[a, i] P[b, i] is the number of items users a and
+        b share (exact integers; c_aa is the number of items of a), and the similarities are ItemKNN's, applied to
+        users: in double with every operation rounded to nearest, "cosine" c_ab / (sqrt(c_aa) sqrt(c_bb) + shrink),
+        "jaccard" c_ab / ((c_aa + c_bb - c_ab) + shrink), "conditional" c_ab / (c_aa + shrink) (not symmetric). The
+        neighbours of u are the top-k users v != u with c_uv > 0 by sim(u, v), ties to the lower id (fewer when u has
+        fewer such users); ``neighbors[u, v]`` = sim(u, v), which equals ``ItemKNN`` trained on X^T bit for bit.
+        k in 1..1024 (k >= num_users keeps every candidate), shrink finite and >= 0. ``cores`` is accepted and
+        ignored."""
+        shrink = _check_knn_args(k, similarity, shrink)
+        Xc = _canonical(X)
+        if verbose > 0:
+            print("Compute the user neighbourhoods")
+            start = time.time()
+        self._X = DeviceCSR.from_scipy(Xc, self.device)
+        self._W_d = engine.knn_train(self._X.transpose(), self._X, int(k), similarity, shrink)
         self._W_h = None
         if verbose > 0:
             torch.cuda.synchronize(self.device)
