@@ -347,6 +347,26 @@ int wmf_slim_train(const int64_t* x_indptr, const int32_t* x_indices, int64_t ro
                    double l1, double l2, int max_iter, double tol, int64_t* wt_indptr, int32_t* wt_indices,
                    double* wt_data, int32_t* sweeps, void* ws, size_t ws_bytes, void* stream);
 
+/* RP3beta: a three-step random walk user -> item -> user -> item in closed form (DESIGN.md 4.9), defined here, not
+ * ported. P (p_indptr / p_indices, `rows` x n) is the binary pattern of the canonical X of the knn entries above (sorted
+ * rows, no duplicates: not checked, a duplicate item in a row would race in the tile); pt_* is the CSR of P^T
+ * (wmf_csr_transpose: each item's users ascending); nnz = p_indptr[rows] = pt_indptr[n]. du [rows], ra [n], cb [n] are
+ * the caller's scales (deg_u^-alpha, pop_a^-alpha, pop_b^-beta, computed on the host; entries of empty rows and
+ * columns are not read); no device code calls pow. In double, every operation rounded to nearest, none fused:
+ *   S_ab = sum over the users u of both a and b, ascending, from +0.0, of du[u];   W'_ab = (ra[a] * S_ab) * cb[b].
+ * Row a of W holds the top-min(k, n) items b != a with S_ab > 0 by W'_ab, ties to the lower id, fewer when a has fewer
+ * such items; W[a, b] = W'_ab, written like wmf_knn_train's W (n x n CSR, sorted rows, room for n * min(k, n)
+ * entries, the first w_indptr[n] used), so wmf_knn_predict and wmf_knn_score_topk score it. 1 <= k <= 1024,
+ * 0 < n < 2^31, rows >= 0, 0 <= nnz < 2^40, non-null pointers (p_indices / pt_indices may be null when nnz is 0, du
+ * when rows is 0): else WMF_ERR_INVALID before any CUDA call; a short workspace: WMF_ERR_WORKSPACE. The workspace
+ * (wmf_rp3beta_train_workspace_bytes, 0 for arguments out of range) holds a double [B x n] tile (B item rows from n
+ * and a fixed byte budget), the selected rows of all n items, the item order and nnz walk weights. */
+size_t wmf_rp3beta_train_workspace_bytes(int64_t n, int64_t nnz, int k);
+int wmf_rp3beta_train(const int64_t* p_indptr, const int32_t* p_indices, int64_t rows, const int64_t* pt_indptr,
+                      const int32_t* pt_indices, int64_t n, int64_t nnz, const double* du, const double* ra,
+                      const double* cb, int k, int64_t* w_indptr, int32_t* w_indices, double* w_data, void* ws,
+                      size_t ws_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

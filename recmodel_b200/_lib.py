@@ -76,6 +76,8 @@ SIGNATURES = {
     "wmf_slim_train_workspace_bytes": (_sz, [_i64, _i32]),
     "wmf_slim_train": (_i32, [_p, _p, _i64, _p, _p, _i64, _p, _p, _i32, _f64, _f64, _i32, _f64, _p, _p, _p, _p, _p, _sz,
                               _p]),
+    "wmf_rp3beta_train_workspace_bytes": (_sz, [_i64, _i64, _i32]),
+    "wmf_rp3beta_train": (_i32, [_p, _p, _i64, _p, _p, _i64, _i64, _p, _p, _p, _i32, _p, _p, _p, _p, _sz, _p]),
 }
 
 

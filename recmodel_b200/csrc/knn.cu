@@ -10,6 +10,9 @@
 // knn_compact_kernel write the CSR of W^T.
 // UserKNN (DESIGN.md 4.8) trains with wmf_knn_train on (X^T, X) and scores with userknn_score_tile_kernel and
 // userknn_predict_kernel, which walk the neighbours' rows of X.
+// RP3beta (DESIGN.md 4.9) sums its walk weights into a [B x n] tile with userknn_score_tile_kernel over (P^T, P), rows
+// grouped by walk length (rp3_chain_kernel, rp3_order_kernel), scales them (rp3_weight_kernel), selects like ItemKNN
+// and sorts each row into the staging row of its item (rp3_sort_rows_kernel); W is then scored like ItemKNN's.
 #include "common.cuh"
 #include "score.cuh"
 
@@ -70,17 +73,14 @@ __global__ __launch_bounds__(KN_THREADS) void knn_similarity_kernel(const int* _
     S[e] = s;
 }
 
-// One CTA per block row: the selected (id, similarity) pairs (ids -1 where the row had fewer than kk candidates)
-// sorted by id into row a0 + r of the [n x kk] staging area; cnt[a0 + r] = their number. The rank of an entry is the
-// number of selected ids below it (ids are distinct).
-__global__ __launch_bounds__(KN_THREADS) void knn_sort_rows_kernel(const int64_t* __restrict__ ids,
-                                                                   const double* __restrict__ vals, int kk, int64_t a0,
-                                                                   int32_t* __restrict__ st_idx,
-                                                                   double* __restrict__ st_val,
-                                                                   int64_t* __restrict__ cnt) {
+// The body of the row sorts below, for one CTA: the selected (id, value) pairs of selection row r (ids -1 where the
+// row had fewer than kk candidates) sorted by id into row `row` of the [n x kk] staging area; cnt[row] = their number.
+// The rank of an entry is the number of selected ids below it (ids are distinct).
+__device__ __forceinline__ void knn_sort_row(const int64_t* __restrict__ ids, const double* __restrict__ vals, int kk,
+                                             int64_t r, int64_t row, int32_t* __restrict__ st_idx,
+                                             double* __restrict__ st_val, int64_t* __restrict__ cnt) {
     __shared__ int32_t sid[TK_MAX];
     __shared__ unsigned s_m;
-    const int64_t r = blockIdx.x, row = a0 + r;
     if (threadIdx.x == 0) s_m = 0;
     __syncthreads();
     for (int t = threadIdx.x; t < kk; t += KN_THREADS) {
@@ -98,6 +98,15 @@ __global__ __launch_bounds__(KN_THREADS) void knn_sort_rows_kernel(const int64_t
         st_val[row * kk + pos] = vals[r * kk + t];
     }
     if (threadIdx.x == 0) cnt[row] = s_m;
+}
+
+// One CTA per block row: selection row r into staging row a0 + r
+__global__ __launch_bounds__(KN_THREADS) void knn_sort_rows_kernel(const int64_t* __restrict__ ids,
+                                                                   const double* __restrict__ vals, int kk, int64_t a0,
+                                                                   int32_t* __restrict__ st_idx,
+                                                                   double* __restrict__ st_val,
+                                                                   int64_t* __restrict__ cnt) {
+    knn_sort_row(ids, vals, kk, blockIdx.x, a0 + blockIdx.x, st_idx, st_val, cnt);
 }
 
 // indptr[0] = 0, indptr[a + 1] = cnt[0] + ... + cnt[a]: one CTA, chunks of KN_THREADS rows
@@ -425,6 +434,109 @@ SlimLayout slim_layout(int64_t n, int kk) {
 
 bool slim_finite_nonneg(double x) { return x >= 0.0 && x <= 1.7976931348623157e308; }
 
+// ---- RP3beta (DESIGN.md 4.9): S_ab = sum over the common users u of a and b, ascending, of du[u], then
+// W'_ab = (ra[a] S_ab) cb[b] and the top-k per row. The S tile is userknn_score_tile_kernel's score tile for "users"
+// = items, "neighbours" = the users of the item (P^T, values du[u]) and "X" = P with every value 1.0f, so each
+// product is du[u] exactly and each S_ab is summed from +0.0 in ascending u, one CTA per row, without atomics.
+
+// nb_val[e] = du[pt_indices[e]] (the per-entry walk weights) and one[e] = 1.0f (the values of P)
+__global__ __launch_bounds__(KN_THREADS) void rp3_gather_kernel(const int32_t* __restrict__ pt_indices, int64_t nnz,
+                                                                const double* __restrict__ du,
+                                                                double* __restrict__ nb_val, float* __restrict__ one) {
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < nnz; e += stride) {
+        nb_val[e] = du[pt_indices[e]];
+        one[e] = 1.0f;
+    }
+}
+
+// chain[a] = sum over the users u of a of ceil(deg_u / KN_THREADS): the barrier steps of tile row a in
+// userknn_score_tile_kernel. One warp per item.
+__global__ __launch_bounds__(KN_THREADS) void rp3_chain_kernel(const int64_t* __restrict__ p_indptr,
+                                                               const int64_t* __restrict__ pt_indptr,
+                                                               const int32_t* __restrict__ pt_indices, int64_t n,
+                                                               int64_t* __restrict__ chain) {
+    const int64_t a = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (a >= n) return;
+    const int lane = threadIdx.x & 31;
+    int64_t s = 0;
+    for (int64_t t = pt_indptr[a] + lane; t < pt_indptr[a + 1]; t += 32) {
+        const int32_t u = pt_indices[t];
+        s += (p_indptr[u + 1] - p_indptr[u] + KN_THREADS - 1) / KN_THREADS;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) s += __shfl_down_sync(0xffffffffu, s, o);
+    if (lane == 0) chain[a] = s;
+}
+
+// order[rank(a)] = a with rank(a) = #{b : chain[b] > chain[a] or (chain[b] == chain[a] and b < a)}: the items by
+// descending chain, ties by id (a permutation, so the same order every run). n^2 comparisons against KN_THREADS-item
+// chunks staged in shared memory; training writes n^2 tile entries anyway.
+__global__ __launch_bounds__(KN_THREADS) void rp3_order_kernel(const int64_t* __restrict__ chain, int64_t n,
+                                                               int64_t* __restrict__ order) {
+    __shared__ int64_t s_chain[KN_THREADS];
+    const int64_t a = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int64_t ca = a < n ? chain[a] : 0;
+    int64_t rank = 0;
+    for (int64_t b0 = 0; b0 < n; b0 += KN_THREADS) {
+        __syncthreads();
+        if (b0 + threadIdx.x < n) s_chain[threadIdx.x] = chain[b0 + threadIdx.x];
+        __syncthreads();
+        const int m = (int)(n - b0 < KN_THREADS ? n - b0 : KN_THREADS);
+        for (int q = 0; q < m; ++q) {
+            const int64_t cb = s_chain[q];
+            rank += cb > ca || (cb == ca && b0 + q < a);
+        }
+    }
+    if (a < n) order[rank] = a;
+}
+
+// S[r][b] = W'(a, b) for a = order[a0 + r]: (ra[a] S_ab) cb[b], rounded to nearest; self and S_ab = 0 (no common user)
+// get RankKey<double>::excluded()
+__global__ __launch_bounds__(KN_THREADS) void rp3_weight_kernel(double* __restrict__ S,
+                                                                const int64_t* __restrict__ order, int64_t a0,
+                                                                int64_t n, const double* __restrict__ ra,
+                                                                const double* __restrict__ cb) {
+    const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= n) return;
+    const int64_t r = blockIdx.y, a = order[a0 + r], e = r * n + b;
+    const double s = S[e];
+    S[e] = s > 0.0 && b != a ? __dmul_rn(__dmul_rn(ra[a], s), cb[b]) : RankKey<double>::excluded();
+}
+
+// One CTA per block row: selection row r into staging row order[a0 + r]
+__global__ __launch_bounds__(KN_THREADS) void rp3_sort_rows_kernel(const int64_t* __restrict__ ids,
+                                                                   const double* __restrict__ vals, int kk,
+                                                                   const int64_t* __restrict__ order, int64_t a0,
+                                                                   int32_t* __restrict__ st_idx,
+                                                                   double* __restrict__ st_val,
+                                                                   int64_t* __restrict__ cnt) {
+    knn_sort_row(ids, vals, kk, blockIdx.x, order[a0 + blockIdx.x], st_idx, st_val, cnt);
+}
+
+struct Rp3Layout {
+    size_t S, ids, vals, st_idx, st_val, cnt, chain, order, nb_val, one, total;
+};
+
+Rp3Layout rp3_layout(int64_t n, int64_t nnz, int kk) {
+    const size_t B = (size_t)knn_batch(n, n);
+    Rp3Layout L;
+    size_t off = 0;
+    auto take = [&](size_t bytes) { const size_t at = off; off += align_up(bytes, 256); return at; };
+    L.S = take(B * n * 8);
+    L.ids = take(B * kk * 8);
+    L.vals = take(B * kk * 8);
+    L.st_idx = take((size_t)n * kk * 4);
+    L.st_val = take((size_t)n * kk * 8);
+    L.cnt = take((size_t)n * 8);
+    L.chain = take((size_t)n * 8);
+    L.order = take((size_t)n * 8);
+    L.nb_val = take((size_t)nnz * 8);
+    L.one = take((size_t)nnz * 4);
+    L.total = off;
+    return L;
+}
+
 int check_knn_args(const char* name, int64_t n, int k, int similarity, double shrink) {
     WMF_REQUIRE(n > 0 && n < (1ll << 31), "%s: n=%lld outside 1..2^31-1", name, (long long)n);
     WMF_REQUIRE(k >= 1 && k <= TK_MAX, "%s: k=%d outside 1..%d", name, k, TK_MAX);
@@ -605,6 +717,73 @@ int wmf_slim_train(const int64_t* x_indptr, const int32_t* x_indices, int64_t ro
     WMF_LAUNCH_CHECK("knn_scan_kernel");
     knn_compact_kernel<<<(unsigned)((n + KN_THREADS / 32 - 1) / (KN_THREADS / 32)), KN_THREADS, 0, st>>>(
         st_idx, st_val, kk, n, wt_indptr, wt_indices, wt_data);
+    WMF_LAUNCH_CHECK("knn_compact_kernel");
+    return WMF_OK;
+}
+
+size_t wmf_rp3beta_train_workspace_bytes(int64_t n, int64_t nnz, int k) {
+    if (n <= 0 || n >= (1ll << 31) || nnz < 0 || nnz >= (1ll << 40) || k < 1 || k > TK_MAX) return 0;
+    return rp3_layout(n, nnz, (int)(k < n ? k : n)).total;
+}
+
+int wmf_rp3beta_train(const int64_t* p_indptr, const int32_t* p_indices, int64_t rows, const int64_t* pt_indptr,
+                      const int32_t* pt_indices, int64_t n, int64_t nnz, const double* du, const double* ra,
+                      const double* cb, int k, int64_t* w_indptr, int32_t* w_indices, double* w_data, void* ws,
+                      size_t ws_bytes, void* stream) {
+    WMF_REQUIRE(n > 0 && n < (1ll << 31), "wmf_rp3beta_train: n=%lld outside 1..2^31-1", (long long)n);
+    WMF_REQUIRE(k >= 1 && k <= TK_MAX, "wmf_rp3beta_train: k=%d outside 1..%d", k, TK_MAX);
+    WMF_REQUIRE(rows >= 0, "wmf_rp3beta_train: rows=%lld < 0", (long long)rows);
+    WMF_REQUIRE(nnz >= 0 && nnz < (1ll << 40), "wmf_rp3beta_train: nnz=%lld outside 0..2^40-1", (long long)nnz);
+    WMF_REQUIRE(p_indptr && pt_indptr && (du || rows == 0) && ra && cb && w_indptr && w_indices && w_data &&
+                    ((p_indices && pt_indices) || nnz == 0),
+                "wmf_rp3beta_train: null argument");
+    const size_t need = wmf_rp3beta_train_workspace_bytes(n, nnz, k);
+    if (ws == nullptr || ws_bytes < need) {
+        set_error("wmf_rp3beta_train: workspace %zu < %zu", ws_bytes, need);
+        return WMF_ERR_WORKSPACE;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    const int kk = (int)(k < n ? k : n);
+    const Rp3Layout L = rp3_layout(n, nnz, kk);
+    char* base = reinterpret_cast<char*>(ws);
+    double* S = reinterpret_cast<double*>(base + L.S);
+    int64_t* ids = reinterpret_cast<int64_t*>(base + L.ids);
+    double* vals = reinterpret_cast<double*>(base + L.vals);
+    int32_t* st_idx = reinterpret_cast<int32_t*>(base + L.st_idx);
+    double* st_val = reinterpret_cast<double*>(base + L.st_val);
+    int64_t* cnt = reinterpret_cast<int64_t*>(base + L.cnt);
+    int64_t* chain = reinterpret_cast<int64_t*>(base + L.chain);
+    int64_t* order = reinterpret_cast<int64_t*>(base + L.order);
+    double* nb_val = reinterpret_cast<double*>(base + L.nb_val);
+    float* one = reinterpret_cast<float*>(base + L.one);
+    if (nnz > 0) {
+        rp3_gather_kernel<<<(unsigned)sm_count() * 8, KN_THREADS, 0, st>>>(pt_indices, nnz, du, nb_val, one);
+        WMF_LAUNCH_CHECK("rp3_gather_kernel");
+    }
+    rp3_chain_kernel<<<(unsigned)((n + KN_THREADS / 32 - 1) / (KN_THREADS / 32)), KN_THREADS, 0, st>>>(
+        p_indptr, pt_indptr, pt_indices, n, chain);
+    WMF_LAUNCH_CHECK("rp3_chain_kernel");
+    rp3_order_kernel<<<(unsigned)((n + KN_THREADS - 1) / KN_THREADS), KN_THREADS, 0, st>>>(chain, n, order);
+    WMF_LAUNCH_CHECK("rp3_order_kernel");
+    const int64_t bmax = knn_batch(n, n);
+    for (int64_t a0 = 0; a0 < n; a0 += bmax) {
+        const int B = (int)(n - a0 < bmax ? n - a0 : bmax);
+        WMF_CUDA(cudaMemsetAsync(S, 0, (size_t)B * n * sizeof(double), st));
+        userknn_score_tile_kernel<<<(unsigned)B, KN_THREADS, 0, st>>>(p_indptr, p_indices, one, pt_indptr, pt_indices,
+                                                                     nb_val, n, order, a0, S);
+        WMF_LAUNCH_CHECK("userknn_score_tile_kernel");
+        rp3_weight_kernel<<<dim3((unsigned)((n + KN_THREADS - 1) / KN_THREADS), (unsigned)B), KN_THREADS, 0, st>>>(
+            S, order, a0, n, ra, cb);
+        WMF_LAUNCH_CHECK("rp3_weight_kernel");
+        const int rc = select_topk_double(nullptr, 0, B, nullptr, nullptr, S, n, kk, ids, vals, st, true);
+        if (rc) return rc;
+        rp3_sort_rows_kernel<<<(unsigned)B, KN_THREADS, 0, st>>>(ids, vals, kk, order, a0, st_idx, st_val, cnt);
+        WMF_LAUNCH_CHECK("rp3_sort_rows_kernel");
+    }
+    knn_scan_kernel<<<1, KN_THREADS, 0, st>>>(cnt, n, w_indptr);
+    WMF_LAUNCH_CHECK("knn_scan_kernel");
+    knn_compact_kernel<<<(unsigned)((n + KN_THREADS / 32 - 1) / (KN_THREADS / 32)), KN_THREADS, 0, st>>>(
+        st_idx, st_val, kk, n, w_indptr, w_indices, w_data);
     WMF_LAUNCH_CHECK("knn_compact_kernel");
     return WMF_OK;
 }

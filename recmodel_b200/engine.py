@@ -681,6 +681,32 @@ def knn_train(X_csr, XT_csr, k, similarity, shrink):
 
 
 @_device_of(0)
+def rp3beta_train(P_csr, PT_csr, du, ra, cb, k):
+    """The RP3beta weights of the binary pattern ``P_csr`` of a canonical interaction matrix (``PT_csr`` its
+    transpose) from the float64 device scales du [users], ra [items] and cb [items] (include/wmf_b200.h:
+    wmf_rp3beta_train): (indptr int64 [n+1], indices int32, data float64) of the n x n CSR W, rows sorted by id, the
+    layout ``knn_predict`` and ``knn_score_topk`` take."""
+    lib = _lib.load()
+    n = P_csr.shape[1]
+    dev = P_csr.device
+    assert du.dtype == ra.dtype == cb.dtype == torch.float64 and du.numel() == P_csr.shape[0]
+    assert ra.numel() == cb.numel() == n and PT_csr.nnz == P_csr.nnz
+    kk = min(int(k), n)
+    indptr = torch.empty(n + 1, dtype=torch.int64, device=dev)
+    indices = torch.empty(n * kk, dtype=torch.int32, device=dev)
+    data = torch.empty(n * kk, dtype=torch.float64, device=dev)
+    ws = workspace(lib.wmf_rp3beta_train_workspace_bytes(n, P_csr.nnz, int(k)), dev)
+    _lib.check(lib.wmf_rp3beta_train(_ptr(P_csr.indptr), _ptr(P_csr.indices), P_csr.shape[0], _ptr(PT_csr.indptr),
+                                     _ptr(PT_csr.indices), n, P_csr.nnz, _ptr(du), _ptr(ra), _ptr(cb), int(k),
+                                     _ptr(indptr), _ptr(indices), _ptr(data), _ptr(ws), ws.numel(), _stream()),
+               "wmf_rp3beta_train")
+    nnz = int(indptr[-1])
+    if nnz < n * kk:
+        indices, data = indices[:nnz].clone(), data[:nnz].clone()
+    return indptr, indices, data
+
+
+@_device_of(0)
 def knn_predict(X_csr, W, users, items):
     """float64 ItemKNN scores s(users[k], items[k]) (include/wmf_b200.h: wmf_knn_predict) for the canonical ``X_csr``
     and W = (indptr, indices, data) as ``knn_train`` returns it; one user broadcasts."""

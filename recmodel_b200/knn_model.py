@@ -44,9 +44,9 @@ def _check_knn_args(k, similarity, shrink):
 
 
 class ItemItemModel(XWRanking, RecModel):
-    """The scoring half shared by the item-item models (``ItemKNN``, ``SLIM``): the canonical X and an n x n item
-    weight CSR W on the device, and ``predict`` and ``rank`` over s(u, i) = sum over the entries j of row u of X,
-    ascending, of x_uj * W[j, i]; ``recommend`` and ``eval_ranking`` rank these scores (``ranking.XWRanking``). A
+    """The scoring half shared by the item-item models (``ItemKNN``, ``SLIM``, ``RP3beta``): the canonical X and an
+    n x n item weight CSR W on the device, and ``predict`` and ``rank`` over s(u, i) = sum over the entries j of row u
+    of X, ascending, of x_uj * W[j, i]; ``recommend`` and ``eval_ranking`` rank these scores (``ranking.XWRanking``). A
     subclass trains W and names it (``_W_NAME``, the attribute a user sets). ``UserKNN`` scores from a users x users W
     instead: it names the axis of X whose size W must have (``_W_AXIS``) and its own engine functions."""
 

@@ -23,7 +23,7 @@ def test_coverage(cls, Train, topN):
     """``item_counts[i]`` = number of users whose top-``topN`` over their unseen items contains item i
     (utils.py:3-18). Like the reference the result has ``Train.shape[0]`` entries (it sizes the array by the
     row count, utils.py:7). ``cls`` is any model with the RecModel ``rank``; models with ``recommend`` (WMF,
-    Ease, ItemKNN, UserKNN, SLIM) rank every user's unseen items on the device in one call, with the stored entries of ``Train`` excluded
+    Ease, ItemKNN, UserKNN, SLIM, RP3beta) rank every user's unseen items on the device in one call, with the stored entries of ``Train`` excluded
     there (ties are ordered by item id, as ``rank`` orders them over the ascending candidate list)."""
     Train = Train.tocsr()
     n_users, n_items = Train.shape
