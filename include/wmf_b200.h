@@ -326,6 +326,26 @@ int wmf_userknn_score_topk(const int64_t* x_indptr, const int32_t* x_indices, co
                            const int64_t* users, int64_t nu, const int64_t* ex_indptr, const int32_t* ex_indices,
                            int topn, int64_t* out_ids, double* out_scores, void* ws, size_t ws_bytes, void* stream);
 
+/* UserKNN fold-in (DESIGN.md 4.10): the neighbours among the m training users of nq new histories that are not rows
+ * of X. q_indptr / q_indices: the new rows, canonical like X (sorted, no duplicates, no explicit zeros: not checked,
+ * a duplicate would count twice), column ids below n_items. xt_indptr / xt_indices: the CSR of the training X^T
+ * (n_items rows, each item's users); x_indptr: the m + 1 row offsets of the training X. With q_r the pattern of new
+ * row r and P_v that of training user v, c_rv = |q_r ∩ P_v|, c_rr = |q_r| and c_vv = |P_v| (exact integers), and
+ * sim(r, v) is wmf_knn_train's formula for `similarity` and `shrink`. Row r of the output N' holds the top-min(k, m)
+ * training users v with c_rv > 0 by sim(r, v), ties to the lower id (no self exclusion: r is not a training user);
+ * N'[r, v] = sim(r, v). N' is written as an nq x m CSR with sorted column indices (out_indptr [nq+1], out_indices /
+ * out_data with room for nq * min(k, m) entries, the first out_indptr[nq] used): the layout wmf_userknn_predict and
+ * wmf_userknn_score_topk take, indexed by new-row id. 1 <= k <= 1024, similarity one of WMF_KNN_*, shrink finite and
+ * >= 0, 0 < m < 2^31, 0 < nq < 2^31, n_items >= 0, non-null pointers (q_indices / xt_indices may be null when they
+ * hold no entry): else WMF_ERR_INVALID before any CUDA call; a short workspace: WMF_ERR_WORKSPACE. The workspace
+ * (wmf_userknn_fold_in_workspace_bytes, 0 for arguments out of range) holds an int32 and a double [B x m] tile (B new
+ * rows from m and a fixed byte budget) and the selected rows of all nq histories. */
+size_t wmf_userknn_fold_in_workspace_bytes(int64_t nq, int64_t m, int k);
+int wmf_userknn_fold_in(const int64_t* q_indptr, const int32_t* q_indices, int64_t nq, const int64_t* xt_indptr,
+                        const int32_t* xt_indices, int64_t n_items, const int64_t* x_indptr, int64_t m, int k,
+                        int similarity, double shrink, int64_t* out_indptr, int32_t* out_indices, double* out_data,
+                        void* ws, size_t ws_bytes, void* stream);
+
 /* SLIM: sparse non-negative item-item regression (DESIGN.md 4.7). No reference call site: the SLIM sources of
  * RecModel are not part of this repository, and this model is defined here, not ported.
  * X, X^T and P are those of the knn entries above (canonical X); G = P^T P, so G[a, b] = c_ab. The candidates S_j of

@@ -73,6 +73,8 @@ SIGNATURES = {
     "wmf_userknn_predict": (_i32, [_p, _p, _p, _p, _p, _p, _p, _i64, _p, _i64, _p, _p]),
     "wmf_userknn_score_topk_workspace_bytes": (_sz, [_i64, _i64, _i32]),
     "wmf_userknn_score_topk": (_i32, [_p, _p, _p, _p, _p, _p, _i64, _p, _i64, _p, _p, _i32, _p, _p, _p, _sz, _p]),
+    "wmf_userknn_fold_in_workspace_bytes": (_sz, [_i64, _i64, _i32]),
+    "wmf_userknn_fold_in": (_i32, [_p, _p, _i64, _p, _p, _i64, _p, _i64, _i32, _i32, _f64, _p, _p, _p, _p, _sz, _p]),
     "wmf_slim_train_workspace_bytes": (_sz, [_i64, _i32]),
     "wmf_slim_train": (_i32, [_p, _p, _i64, _p, _p, _i64, _p, _p, _i32, _f64, _f64, _i32, _f64, _p, _p, _p, _p, _p, _sz,
                               _p]),

@@ -9,7 +9,9 @@
 // knn_cooc_kernel over all n rows, slim_cd_kernel solves each column's regression on chip, and knn_scan_kernel plus
 // knn_compact_kernel write the CSR of W^T.
 // UserKNN (DESIGN.md 4.8) trains with wmf_knn_train on (X^T, X) and scores with userknn_score_tile_kernel and
-// userknn_predict_kernel, which walk the neighbours' rows of X.
+// userknn_predict_kernel, which walk the neighbours' rows of X. Its fold-in (DESIGN.md 4.10, wmf_userknn_fold_in)
+// counts new rows against the training users with knn_cooc_kernel, scores them with
+// userknn_cross_similarity_kernel and selects and writes the neighbours like wmf_knn_train.
 // RP3beta (DESIGN.md 4.9) sums its walk weights into a [B x n] tile with userknn_score_tile_kernel over (P^T, P), rows
 // grouped by walk length (rp3_chain_kernel, rp3_order_kernel), scales them (rp3_weight_kernel), selects like ItemKNN
 // and sorts each row into the staging row of its item (rp3_sort_rows_kernel); W is then scored like ItemKNN's.
@@ -51,6 +53,15 @@ __global__ __launch_bounds__(KN_THREADS) void knn_cooc_kernel(const int64_t* __r
     }
 }
 
+// sim(a, b) from c_ab, c_aa and c_bb: the formulas of wmf_knn_train, every operation rounded to nearest, none fused
+__device__ __forceinline__ double knn_sim(int sim, double cab, double caa, double cbb, double shrink) {
+    double den;
+    if (sim == WMF_KNN_COSINE) den = __dadd_rn(__dmul_rn(__dsqrt_rn(caa), __dsqrt_rn(cbb)), shrink);
+    else if (sim == WMF_KNN_JACCARD) den = __dadd_rn(__dsub_rn(__dadd_rn(caa, cbb), cab), shrink);
+    else den = __dadd_rn(caa, shrink);
+    return __ddiv_rn(cab, den);
+}
+
 // S[r][b] = sim(a0 + r, b) from the counts; self and c_ab = 0 get RankKey<double>::excluded(). c_bb is the column
 // count of X (X^T row length): the canonical X stores each (u, b) once.
 __global__ __launch_bounds__(KN_THREADS) void knn_similarity_kernel(const int* __restrict__ C,
@@ -62,14 +73,7 @@ __global__ __launch_bounds__(KN_THREADS) void knn_similarity_kernel(const int* _
     const int64_t r = blockIdx.y, a = a0 + r, e = r * n + b;
     const int c = C[e];
     double s = RankKey<double>::excluded();
-    if (c != 0 && b != a) {
-        const double cab = (double)c, caa = knn_pop(xt_indptr, a), cbb = knn_pop(xt_indptr, b);
-        double den;
-        if (sim == WMF_KNN_COSINE) den = __dadd_rn(__dmul_rn(__dsqrt_rn(caa), __dsqrt_rn(cbb)), shrink);
-        else if (sim == WMF_KNN_JACCARD) den = __dadd_rn(__dsub_rn(__dadd_rn(caa, cbb), cab), shrink);
-        else den = __dadd_rn(caa, shrink);
-        s = __ddiv_rn(cab, den);
-    }
+    if (c != 0 && b != a) s = knn_sim(sim, (double)c, knn_pop(xt_indptr, a), knn_pop(xt_indptr, b), shrink);
     S[e] = s;
 }
 
@@ -274,6 +278,22 @@ __global__ __launch_bounds__(KN_THREADS) void userknn_predict_kernel(
     out[k] = acc;
 }
 
+// Fold-in (DESIGN.md 4.10): S[r][v] = sim(q_{r0 + r}, v) between new row r0 + r of Q and training user v from the
+// counts C[r][v] = |q_r ∩ P_v|; c_rr is the Q row length, c_vv the X row length (both canonical). c_rv = 0 gets
+// RankKey<double>::excluded(); there is no self to exclude, r is not a training user.
+__global__ __launch_bounds__(KN_THREADS) void userknn_cross_similarity_kernel(const int* __restrict__ C,
+                                                                              const int64_t* __restrict__ q_indptr,
+                                                                              const int64_t* __restrict__ x_indptr,
+                                                                              int64_t m, int64_t r0, int sim,
+                                                                              double shrink, double* __restrict__ S) {
+    const int64_t v = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (v >= m) return;
+    const int64_t r = blockIdx.y, e = r * m + v;
+    const int c = C[e];
+    S[e] = c != 0 ? knn_sim(sim, (double)c, knn_pop(q_indptr, r0 + r), knn_pop(x_indptr, v), shrink)
+                  : RankKey<double>::excluded();
+}
+
 // rows per [B x n] similarity tile (and users per score tile): the double tile near KN_TILE_BYTES, at least one row
 int64_t knn_batch(int64_t rows, int64_t n) {
     int64_t b = (int64_t)(KN_TILE_BYTES / ((size_t)n * 8));
@@ -286,8 +306,14 @@ struct TrainLayout {
     size_t C, S, ids, vals, st_idx, st_val, cnt, total;
 };
 
-TrainLayout train_layout(int64_t n, int kk) {
-    const size_t B = (size_t)knn_batch(n, n);
+// rows per fold-in tile: knn_batch, at most 65535 (the similarity kernel's grid rows; training tiles stay below 2 897)
+int64_t fold_in_batch(int64_t nq, int64_t m) {
+    const int64_t b = knn_batch(nq, m);
+    return b < 65535 ? b : 65535;
+}
+
+// `rows` selection rows over n columns in tiles of B rows: wmf_knn_train has rows = n, the fold-in one row per history
+TrainLayout train_layout(int64_t rows, int64_t n, int kk, size_t B) {
     TrainLayout L;
     size_t off = 0;
     auto take = [&](size_t bytes) { const size_t at = off; off += align_up(bytes, 256); return at; };
@@ -295,9 +321,9 @@ TrainLayout train_layout(int64_t n, int kk) {
     L.S = take(B * n * 8);
     L.ids = take(B * kk * 8);
     L.vals = take(B * kk * 8);
-    L.st_idx = take((size_t)n * kk * 4);
-    L.st_val = take((size_t)n * kk * 8);
-    L.cnt = take((size_t)n * 8);
+    L.st_idx = take((size_t)rows * kk * 4);
+    L.st_val = take((size_t)rows * kk * 8);
+    L.cnt = take((size_t)rows * 8);
     L.total = off;
     return L;
 }
@@ -556,7 +582,7 @@ extern "C" {
 
 size_t wmf_knn_train_workspace_bytes(int64_t n, int k) {
     if (n <= 0 || n >= (1ll << 31) || k < 1 || k > TK_MAX) return 0;
-    return train_layout(n, (int)(k < n ? k : n)).total;
+    return train_layout(n, n, (int)(k < n ? k : n), (size_t)knn_batch(n, n)).total;
 }
 
 int wmf_knn_train(const int64_t* x_indptr, const int32_t* x_indices, int64_t rows, const int64_t* xt_indptr,
@@ -572,7 +598,7 @@ int wmf_knn_train(const int64_t* x_indptr, const int32_t* x_indices, int64_t row
     }
     cudaStream_t st = (cudaStream_t)stream;
     const int kk = (int)(k < n ? k : n);
-    const TrainLayout L = train_layout(n, kk);
+    const TrainLayout L = train_layout(n, n, kk, (size_t)knn_batch(n, n));
     char* base = reinterpret_cast<char*>(ws);
     int* C = reinterpret_cast<int*>(base + L.C);
     double* S = reinterpret_cast<double*>(base + L.S);
@@ -669,6 +695,61 @@ int wmf_userknn_score_topk(const int64_t* x_indptr, const int32_t* x_indices, co
         WMF_LAUNCH_CHECK("userknn_score_tile_kernel");
         return WMF_OK;
     });
+}
+
+size_t wmf_userknn_fold_in_workspace_bytes(int64_t nq, int64_t m, int k) {
+    if (nq <= 0 || nq >= (1ll << 31) || m <= 0 || m >= (1ll << 31) || k < 1 || k > TK_MAX) return 0;
+    return train_layout(nq, m, (int)(k < m ? k : m), (size_t)fold_in_batch(nq, m)).total;
+}
+
+int wmf_userknn_fold_in(const int64_t* q_indptr, const int32_t* q_indices, int64_t nq, const int64_t* xt_indptr,
+                        const int32_t* xt_indices, int64_t n_items, const int64_t* x_indptr, int64_t m, int k,
+                        int similarity, double shrink, int64_t* out_indptr, int32_t* out_indices, double* out_data,
+                        void* ws, size_t ws_bytes, void* stream) {
+    if (int rc = check_knn_args("wmf_userknn_fold_in", m, k, similarity, shrink)) return rc;
+    WMF_REQUIRE(nq > 0 && nq < (1ll << 31), "wmf_userknn_fold_in: nq=%lld outside 1..2^31-1", (long long)nq);
+    WMF_REQUIRE(n_items >= 0, "wmf_userknn_fold_in: n_items=%lld < 0", (long long)n_items);
+    WMF_REQUIRE(q_indptr && xt_indptr && x_indptr && out_indptr && out_indices && out_data,
+                "wmf_userknn_fold_in: null argument");
+    const size_t need = wmf_userknn_fold_in_workspace_bytes(nq, m, k);
+    if (ws == nullptr || ws_bytes < need) {
+        set_error("wmf_userknn_fold_in: workspace %zu < %zu", ws_bytes, need);
+        return WMF_ERR_WORKSPACE;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    const int kk = (int)(k < m ? k : m);
+    const int64_t bmax = fold_in_batch(nq, m);
+    const TrainLayout L = train_layout(nq, m, kk, (size_t)bmax);
+    char* base = reinterpret_cast<char*>(ws);
+    int* C = reinterpret_cast<int*>(base + L.C);
+    double* S = reinterpret_cast<double*>(base + L.S);
+    int64_t* ids = reinterpret_cast<int64_t*>(base + L.ids);
+    double* vals = reinterpret_cast<double*>(base + L.vals);
+    int32_t* st_idx = reinterpret_cast<int32_t*>(base + L.st_idx);
+    double* st_val = reinterpret_cast<double*>(base + L.st_val);
+    int64_t* cnt = reinterpret_cast<int64_t*>(base + L.cnt);
+    const unsigned cooc_grid = (unsigned)sm_count() * 8;
+    for (int64_t r0 = 0; r0 < nq; r0 += bmax) {
+        const int B = (int)(nq - r0 < bmax ? nq - r0 : bmax);
+        WMF_CUDA(cudaMemsetAsync(C, 0, (size_t)B * m * 4, st));
+        if (n_items > 0) {   // the new rows are the "X^T" of the counts (rows -> items), the training X^T their "X"
+            knn_cooc_kernel<<<cooc_grid, KN_THREADS, 0, st>>>(xt_indptr, xt_indices, q_indptr, q_indices, m, r0, B, C);
+            WMF_LAUNCH_CHECK("knn_cooc_kernel");
+        }
+        userknn_cross_similarity_kernel<<<dim3((unsigned)((m + KN_THREADS - 1) / KN_THREADS), (unsigned)B), KN_THREADS,
+                                          0, st>>>(C, q_indptr, x_indptr, m, r0, similarity, shrink, S);
+        WMF_LAUNCH_CHECK("userknn_cross_similarity_kernel");
+        const int rc = select_topk_double(nullptr, 0, B, nullptr, nullptr, S, m, kk, ids, vals, st, true);
+        if (rc) return rc;
+        knn_sort_rows_kernel<<<(unsigned)B, KN_THREADS, 0, st>>>(ids, vals, kk, r0, st_idx, st_val, cnt);
+        WMF_LAUNCH_CHECK("knn_sort_rows_kernel");
+    }
+    knn_scan_kernel<<<1, KN_THREADS, 0, st>>>(cnt, nq, out_indptr);
+    WMF_LAUNCH_CHECK("knn_scan_kernel");
+    knn_compact_kernel<<<(unsigned)((nq + KN_THREADS / 32 - 1) / (KN_THREADS / 32)), KN_THREADS, 0, st>>>(
+        st_idx, st_val, kk, nq, out_indptr, out_indices, out_data);
+    WMF_LAUNCH_CHECK("knn_compact_kernel");
+    return WMF_OK;
 }
 
 size_t wmf_slim_train_workspace_bytes(int64_t n, int k) {

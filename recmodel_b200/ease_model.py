@@ -2,9 +2,9 @@
 
 Mirror of /root/reference/RecModel/ease_model.py:45-114: ``Ease(num_items, num_users)``, ``train(X, alpha, verbose,
 cores)``, ``predict(users, items)``, ``rank(items, users, topn)``, ``save_mat`` / ``load_mat`` and the inherited
-``eval_topn``, plus ``recommend`` (top-N over each user's unseen items for many users in one device call) and
-``eval_ranking`` (full-ranking Recall / Precision / NDCG / MAP / hit rate at N) from ``ranking.XWRanking``, which the
-item-item models share. The Gram X^T X + alpha I, its dense inverse and the prediction loop of
+``eval_topn``, plus ``recommend`` (top-N over each user's unseen items for many users in one device call),
+``eval_ranking`` (full-ranking Recall / Precision / NDCG / MAP / hit rate at N) and their forms for users outside X,
+``recommend_for`` and ``eval_ranking_for``, from ``ranking.XWRanking``, which the item-item models share. The Gram X^T X + alpha I, its dense inverse and the prediction loop of
 RecModel/fast_utils/ease_utils.pyx:15-30 run in the kernels of csrc/ease.cu behind the C ABI; there is no CPU
 fallback. ``cores`` is accepted and ignored (the reference only sets MKL's thread count with it).
 """
@@ -50,8 +50,14 @@ class Ease(XWRanking, RecModel):
             self._W_d = torch.from_numpy(np.ascontiguousarray(self._W_h)).to(self.device)
         return self._W_d
 
+    @staticmethod
+    def _rows(X):
+        """The CSR the scores read for the users x items matrix X: a copy, stored order and duplicates kept
+        (ease_model.py:86); ``train`` keeps it for X, ``recommend_for`` scores the new histories from it."""
+        return X.copy().tocsr()
+
     def _set_X(self, X):
-        X_csr = X.copy().tocsr()          # ease_model.py:86: prediction needs the training interactions
+        X_csr = self._rows(X)             # ease_model.py:86: prediction needs the training interactions
         self.X_indptr = X_csr.indptr.astype(np.int32)
         self.X_idx = X_csr.indices.astype(np.int32)
         self.X_data = X_csr.data.astype(np.float32)

@@ -773,13 +773,15 @@ def userknn_predict(X_csr, N, users, items):
 def userknn_score_topk(X_csr, N, users, topn, exclude=None, want_scores=False):
     """``knn_score_topk`` for the UserKNN scores of ``userknn_predict`` (bitwise): top-``topn`` item ids [nu x topn]
     (int64) over all items minus the stored entries of row ``users[k]`` of ``exclude``, best first, ties to the lower
-    item id, -1 padding (include/wmf_b200.h: wmf_userknn_score_topk); with ``want_scores`` (ids, float64 scores)."""
+    item id, -1 padding (include/wmf_b200.h: wmf_userknn_score_topk); with ``want_scores`` (ids, float64 scores).
+    ``users`` index the rows of N and N's column ids the rows of ``X_csr``: N is the training neighbours or the
+    ``userknn_fold_in`` rows of new histories."""
     lib = _lib.load()
     nb_indptr, nb_indices, nb_data = N
     n = X_csr.shape[1]
     nu = users.numel()
     dev = nb_indptr.device
-    assert users.dtype == torch.int64 and nb_indptr.numel() - 1 == X_csr.shape[0]
+    assert users.dtype == torch.int64
     if exclude is not None:
         assert exclude.shape[1] == n and exclude.indices.dtype == torch.int32 and exclude.indptr.dtype == torch.int64
     ids = torch.empty((nu, topn), dtype=torch.int64, device=dev)
@@ -791,6 +793,33 @@ def userknn_score_topk(X_csr, N, users, topn, exclude=None, want_scores=False):
                                           _ptr(None if exclude is None else exclude.indices), int(topn), _ptr(ids),
                                           _ptr(scores), _ptr(ws), ws.numel(), _stream()), "wmf_userknn_score_topk")
     return (ids, scores) if want_scores else ids
+
+
+@_device_of(1)
+def userknn_fold_in(Q_csr, XT_csr, X_csr, k, similarity, shrink):
+    """The UserKNN neighbours N' among the training users of the rows of ``Q_csr`` (new histories, canonical like X)
+    for the canonical training ``X_csr`` (``XT_csr`` its transpose): (indptr int64 [nq+1], indices int32, data float64)
+    of the nq x m CSR, rows sorted by user id (include/wmf_b200.h: wmf_userknn_fold_in), the layout
+    ``userknn_predict`` and ``userknn_score_topk`` take with user ids = rows of ``Q_csr``."""
+    lib = _lib.load()
+    nq, m = Q_csr.shape[0], X_csr.shape[0]
+    dev = XT_csr.device
+    assert Q_csr.shape[1] == XT_csr.shape[0] == X_csr.shape[1] and XT_csr.shape[1] == m
+    kk = min(int(k), m)
+    indptr = torch.zeros(nq + 1, dtype=torch.int64, device=dev)
+    indices = torch.empty(nq * kk, dtype=torch.int32, device=dev)
+    data = torch.empty(nq * kk, dtype=torch.float64, device=dev)
+    if nq == 0:
+        return indptr, indices, data
+    ws = workspace(lib.wmf_userknn_fold_in_workspace_bytes(nq, m, int(k)), dev)
+    _lib.check(lib.wmf_userknn_fold_in(_ptr(Q_csr.indptr), _ptr(Q_csr.indices), nq, _ptr(XT_csr.indptr),
+                                       _ptr(XT_csr.indices), XT_csr.shape[0], _ptr(X_csr.indptr), m, int(k),
+                                       _lib.KNN_SIMILARITIES[similarity], float(shrink), _ptr(indptr), _ptr(indices),
+                                       _ptr(data), _ptr(ws), ws.numel(), _stream()), "wmf_userknn_fold_in")
+    nnz = int(indptr[-1])
+    if nnz < nq * kk:
+        indices, data = indices[:nnz].clone(), data[:nnz].clone()
+    return indptr, indices, data
 
 
 @_device_of(0)

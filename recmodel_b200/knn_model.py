@@ -4,7 +4,8 @@ user-user counterpart (DESIGN.md 4.8), and ``ItemItemModel``, the scoring half b
 
 ``ItemKNN(num_items, num_users)``, ``train(X, k, similarity, shrink, verbose, cores)``, ``predict(users, items)``,
 ``rank(items, users, topn)``, ``recommend`` (top-N over each user's unseen items for many users in one device call),
-``eval_ranking`` (full-ranking Recall / Precision / NDCG / MAP / hit rate at N) and the inherited ``eval_topn``. The
+``eval_ranking`` (full-ranking Recall / Precision / NDCG / MAP / hit rate at N), ``recommend_for`` and
+``eval_ranking_for`` (the same for users that are not rows of X, DESIGN.md 4.10) and the inherited ``eval_topn``. The
 co-occurrence counts, similarities, neighbour selection and scores run in the kernels of csrc/knn.cu behind the C ABI;
 there is no CPU fallback. The similarities and scores are defined exactly (``train`` and ``predict``), so a NumPy
 restatement reproduces every value bitwise. ``cores`` is accepted and ignored.
@@ -54,6 +55,7 @@ class ItemItemModel(XWRanking, RecModel):
     _W_AXIS = 1   # W is square over the columns of X (the items)
     _score_topk = staticmethod(engine.knn_score_topk)
     _predict_pairs = staticmethod(engine.knn_predict)
+    _rows = staticmethod(_canonical)   # X as train keeps it, and the new histories of recommend_for
 
     def __init__(self, num_items, num_users, device=None):
         self.num_items = num_items
@@ -154,7 +156,7 @@ class ItemKNN(ItemItemModel):
         b != a with c_ab > 0 by sim(a, b), ties to the lower id (fewer when a has fewer such items); W[a, b] =
         sim(a, b) (``neighbors``). k in 1..1024 (k >= num_items keeps every candidate), shrink finite and >= 0."""
         shrink = _check_knn_args(k, similarity, shrink)
-        Xc = _canonical(X)
+        Xc = self._rows(X)
         if verbose > 0:
             print("Compute the item neighbourhoods")
             start = time.time()
@@ -186,6 +188,16 @@ class UserKNN(ItemItemModel):
     def neighbors(self, value):
         self._set_W(value)
 
+    _fold_in_args = None   # (similarity, shrink, k) of the last train
+
+    def _fold_in(self, user_items):
+        """(X, N'): the training X and the neighbours N' among the training users of the rows of ``user_items``
+        (canonicalised like X), by the similarity, shrink and k of ``train`` (DESIGN.md 4.10)."""
+        X, _ = self._X_and_W()
+        similarity, shrink, k = self._fold_in_args
+        Q = DeviceCSR.from_scipy(self._rows(user_items), self.device)
+        return X, engine.userknn_fold_in(Q, X.transpose(), X, k, similarity, shrink)
+
     def predict(self, users, items):
         """float64 s(u, i) per (user, item) pair (one user broadcasts): the sum over the neighbours v of u, in
         ascending v, from +0.0, of sim(u, v) * (double)x_vi with x_vi the float32 entry of the canonical X, each
@@ -203,15 +215,17 @@ class UserKNN(ItemItemModel):
         neighbours of u are the top-k users v != u with c_uv > 0 by sim(u, v), ties to the lower id (fewer when u has
         fewer such users); ``neighbors[u, v]`` = sim(u, v), which equals ``ItemKNN`` trained on X^T bit for bit.
         k in 1..1024 (k >= num_users keeps every candidate), shrink finite and >= 0. ``cores`` is accepted and
-        ignored."""
+        ignored. ``recommend_for`` and ``eval_ranking_for`` find the neighbours of a new history among the training
+        users with the same similarity, shrink and k (DESIGN.md 4.10)."""
         shrink = _check_knn_args(k, similarity, shrink)
-        Xc = _canonical(X)
+        Xc = self._rows(X)
         if verbose > 0:
             print("Compute the user neighbourhoods")
             start = time.time()
         self._X = DeviceCSR.from_scipy(Xc, self.device)
         self._W_d = engine.knn_train(self._X.transpose(), self._X, int(k), similarity, shrink)
         self._W_h = None
+        self._fold_in_args = (similarity, shrink, int(k))
         if verbose > 0:
             torch.cuda.synchronize(self.device)
             print(f"Training took {time.time() - start} seconds!")

@@ -1,8 +1,10 @@
 """Model-independent parts of ``recommend`` and ``eval_ranking``, shared by every model: the exact-score sort path for
-lists longer than the selection kernels take, and the full-ranking evaluation around a model's device ranking.
-``XWRanking`` builds both methods on them for the models scored from a device X and an item weight W (``Ease``,
-``ItemKNN``, ``SLIM``)."""
+lists longer than the selection kernels take, the full-ranking evaluation around a model's device ranking, and the
+bodies of ``recommend_for`` / ``eval_ranking_for``, which rank users that are not rows of the training matrix from a
+representation folded in from their histories (DESIGN.md 4.10). ``XWRanking`` builds these methods on them for the
+models scored from a device X and a weight W (``Ease``, ``ItemKNN``, ``UserKNN``, ``SLIM``, ``RP3beta``)."""
 import numpy as np
+import scipy.sparse
 import torch
 
 from . import _lib, engine
@@ -109,12 +111,65 @@ def eval_ranking_sums(rank_ids, ni, T, ex, users_d, ks, chunk_ids=None):
     return engine.topn_metrics_reduce(per_user, len(ks))
 
 
+def check_fold_in(user_items, ni, exclude, test_mat=None):
+    """ValueError unless ``user_items`` is a 2-D SciPy matrix with ``ni`` columns, ``exclude`` is True, None or a matrix
+    of its shape, and ``test_mat`` (when given) has its shape."""
+    if not scipy.sparse.issparse(user_items) or len(user_items.shape) != 2:
+        raise ValueError(f"user_items must be a 2-D SciPy sparse matrix, got {type(user_items).__name__}")
+    if user_items.shape[1] != ni:
+        raise ValueError(f"user_items has {user_items.shape[1]} columns but the model has {ni} items")
+    shape = tuple(user_items.shape)
+    if not (exclude is True or exclude is None) and tuple(getattr(exclude, "shape", ())) != shape:
+        raise ValueError(f"exclude must be True, None or a matrix of the shape of user_items {shape}")
+    if test_mat is not None and tuple(test_mat.shape) != shape:
+        raise ValueError(f"test_mat has shape {tuple(test_mat.shape)}, user_items {shape}")
+
+
+def recommend_for(fold_in, rank_ids, ni, device, user_items, topn, exclude):
+    """The body of every model's ``recommend_for`` for a model of ``ni`` items: ``fold_in(user_items)`` computes the
+    representation of the new rows once, and ``rank_ids(rep, users_d, k, ex)`` returns the device int64 lists of the
+    rows ``users_d`` (ids into ``user_items``), k <= ni, leaving out the stored entries of row ``users_d[r]`` of ``ex``
+    (a DeviceCSR, or None). ``exclude`` True excludes each row's own stored entries."""
+    check_fold_in(user_items, ni, exclude)
+    topn = int(topn)
+    k = min(topn, ni)
+    nq = user_items.shape[0]
+    out = np.full((nq, topn), -1, dtype=np.int64)
+    if k <= 0 or nq == 0:
+        return out
+    rep = fold_in(user_items)
+    ex = None
+    if exclude is not None:
+        ex = exclude if isinstance(exclude, DeviceCSR) else DeviceCSR.from_scipy(
+            user_items if exclude is True else exclude, device)
+    out[:, :k] = rank_ids(rep, torch.arange(nq, dtype=torch.int64, device=device), k, ex).cpu().numpy()
+    return out
+
+
+def eval_ranking_for(fold_in, rank_ids, ni, device, user_items, test_mat, topn, exclude, users):
+    """The body of every model's ``eval_ranking_for``: ``eval_ranking`` over the lists of ``recommend_for`` (``fold_in``
+    and ``rank_ids`` as there). The representation is folded in once, when the first chunk is ranked, after every
+    argument check."""
+    check_fold_in(user_items, ni, exclude, test_mat)
+    rep = []
+
+    def ranked(users_d, k, ex):
+        if not rep:
+            rep.append(fold_in(user_items))
+        return rank_ids(rep[0], users_d, k, ex)
+    return eval_ranking(ranked, lambda: (ni, user_items.shape[0]), "the rows of user_items", device, test_mat, topn,
+                        user_items if exclude is True else exclude, users)
+
+
 class XWRanking:
-    """``recommend`` and ``eval_ranking`` of a model whose score s(u, i) is computed on the device from the users x
-    items interaction matrix X and an item weight W (``Ease``, ``ItemItemModel``). A subclass provides ``_X_and_W()``
-    (X as a DeviceCSR and W in the layout of its engine functions, or ValueError when the model cannot score),
-    ``_score_topk(X, W, users_d, k, exclude=ex)``, the device top-k of at most ``_lib.TOPK_MAX`` items, and
-    ``_predict_pairs(X, W, users_d, items_d)``, the float64 scores of (user, item) pairs, which it ranks bitwise."""
+    """``recommend``, ``eval_ranking``, ``recommend_for`` and ``eval_ranking_for`` of a model whose score s(u, i) is
+    computed on the device from the users x items interaction matrix X and a weight W (``Ease``, ``ItemItemModel``). A
+    subclass provides ``_X_and_W()`` (X as a DeviceCSR and W in the layout of its engine functions, or ValueError when
+    the model cannot score), ``_score_topk(X, W, users_d, k, exclude=ex)``, the device top-k of at most
+    ``_lib.TOPK_MAX`` items, ``_predict_pairs(X, W, users_d, items_d)``, the float64 scores of (user, item) pairs,
+    which it ranks bitwise, and ``_fold_in(user_items)``, the (X', W') that score the rows of ``user_items`` as users
+    0..len-1. The default ``_fold_in`` is (``_rows(user_items)`` on the device, W): the row preparation ``train``
+    applies to X, then the trained W."""
 
     @property
     def device(self):
@@ -142,13 +197,13 @@ class XWRanking:
         ex = None
         if exclude is not None:
             ex = exclude if isinstance(exclude, DeviceCSR) else DeviceCSR.from_scipy(exclude, self.device)
-        out[:, :k] = self._recommend_ids(torch.from_numpy(users).to(self.device), k, ex).cpu().numpy()
+        out[:, :k] = self._recommend_ids(X, W, torch.from_numpy(users).to(self.device), k, ex).cpu().numpy()
         return out
 
-    def _recommend_ids(self, users_d, k, ex):
-        """Device int64 [len(users_d) x k], k <= num_items: the device part of ``recommend`` (``ex``: a DeviceCSR with
-        rows in any order, or None to exclude nothing)."""
-        X, W = self._X_and_W()
+    def _recommend_ids(self, X, W, users_d, k, ex):
+        """Device int64 [len(users_d) x k], k <= num_items: the device part of ``recommend`` and ``recommend_for`` for
+        the rows ``users_d`` of the device X scored with W (``ex``: a DeviceCSR with rows in any order, or None to
+        exclude nothing)."""
         if k <= _lib.TOPK_MAX:
             return self._score_topk(X, W, users_d, k, exclude=ex)
         n = X.shape[1]   # very long lists: the scores of predict, then stable device sorts
@@ -178,4 +233,30 @@ class XWRanking:
             if tuple(test_mat.shape) != tuple(X.shape):
                 raise ValueError(f"test_mat has shape {tuple(test_mat.shape)}, X {tuple(X.shape)}")
             return X.shape[1], X.shape[0]
-        return eval_ranking(self._recommend_ids, dims, "the rows of X", self.device, test_mat, topn, exclude, users)
+        return eval_ranking(lambda users_d, k, ex: self._recommend_ids(*self._X_and_W(), users_d, k, ex), dims,
+                            "the rows of X", self.device, test_mat, topn, exclude, users)
+
+    def _fold_in(self, user_items):
+        _, W = self._X_and_W()
+        return DeviceCSR.from_scipy(self._rows(user_items), self.device), W
+
+    def recommend_for(self, user_items, topn, exclude=True):
+        """int64 [user_items.shape[0] x topn]: ``recommend`` for users that are not rows of X. Row r is the top-``topn``
+        of all items for the history in row r of ``user_items`` (new users x items, any SciPy format, in the form
+        ``train`` takes X; not modified), best first, ties to the lower item id, -1 padding. The history is prepared
+        as ``train`` prepares X and scored with the trained model, so a copy of row u of X gets the list and the scores
+        of ``recommend([u], topn, exclude=X)``. ``exclude``: True leaves out each row's own stored entries (whatever
+        their value), None nothing, a SciPy matrix or DeviceCSR of the shape of ``user_items`` its stored entries."""
+        X, _ = self._X_and_W()
+        return recommend_for(self._fold_in, lambda XW, users_d, k, ex: self._recommend_ids(*XW, users_d, k, ex),
+                             X.shape[1], self.device, user_items, topn, exclude)
+
+    def eval_ranking_for(self, user_items, test_mat, topn=np.array([10]), exclude=True, users=None):
+        """``eval_ranking`` (the same metrics and definitions) over the lists of ``recommend_for(user_items, K,
+        exclude)``, K = max(topn): the strong-generalisation protocol, where the evaluated users are not rows of X.
+        ``test_mat`` has the shape of ``user_items``; ``users`` (ids into its rows) defaults to the rows of ``test_mat``
+        with stored entries. The histories are folded in once per call; no list leaves the device and the result is
+        bitwise reproducible."""
+        X, _ = self._X_and_W()
+        return eval_ranking_for(self._fold_in, lambda XW, users_d, k, ex: self._recommend_ids(*XW, users_d, k, ex),
+                                X.shape[1], self.device, user_items, test_mat, topn, exclude, users)

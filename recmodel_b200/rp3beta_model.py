@@ -1,7 +1,8 @@
 """RP3beta: a three-step random-walk item model trained, scored and ranked on the device (DESIGN.md 4.9).
 
 ``RP3beta(num_items, num_users)``, ``train(X, alpha, beta, k, verbose, cores)``, a settable ``W``, and from
-``ItemItemModel`` ``predict``, ``rank``, ``recommend`` and ``eval_ranking``. The walk sums, the weights, the neighbour
+``ItemItemModel`` ``predict``, ``rank``, ``recommend``, ``eval_ranking``, ``recommend_for`` and
+``eval_ranking_for``. The walk sums, the weights, the neighbour
 selection and the scores run in the kernels of csrc/knn.cu behind the C ABI; there is no CPU fallback. The powers
 are per-user and per-item scalars computed on the host with NumPy, so the device only adds and multiplies and a NumPy
 restatement reproduces every weight and every score bitwise (Paudel et al. 2016; Dacrema et al., RecSys 2019).
@@ -14,8 +15,8 @@ import torch
 
 from . import _lib, engine
 from .engine import DeviceCSR
-from .knn_model import ItemItemModel, _canonical
-from .slim_model import _int_in
+from .knn_model import ItemItemModel
+from .slim_model import _int_in, _pattern
 
 
 def _exponent(name, v):
@@ -34,6 +35,8 @@ def _scale(counts, exponent):
 
 
 class RP3beta(ItemItemModel):
+
+    _rows = staticmethod(_pattern)   # P: training and scores see the pattern only
 
     @property
     def W(self):
@@ -62,8 +65,7 @@ class RP3beta(ItemItemModel):
         alpha = _exponent("alpha", alpha)
         beta = _exponent("beta", beta)
         k = _int_in("k", k, 1, _lib.TOPK_MAX)
-        Xc = _canonical(X)
-        Xc.data = np.ones_like(Xc.data, dtype=np.float32)   # P: training and scores see the pattern only
+        Xc = self._rows(X)
         deg = np.diff(Xc.indptr)
         pop = np.bincount(Xc.indices, minlength=Xc.shape[1])
         if verbose > 0:

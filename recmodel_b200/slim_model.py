@@ -1,7 +1,8 @@
 """SLIM: sparse non-negative item-item regression trained, scored and ranked on the device (DESIGN.md 4.7).
 
 ``SLIM(num_items, num_users)``, ``train(X, l1, l2, k, max_iter, tol, verbose, cores)``, a settable ``W`` and
-``sweeps``, and from ``ItemItemModel`` ``predict``, ``rank``, ``recommend`` and ``eval_ranking``. The Gram, the
+``sweeps``, and from ``ItemItemModel`` ``predict``, ``rank``, ``recommend``, ``eval_ranking``, ``recommend_for`` and
+``eval_ranking_for``. The Gram, the
 candidates, the coordinate descent and the scores run in the kernels of csrc/knn.cu behind the C ABI; there is no CPU
 fallback. The model is this project's own definition (the reference's SLIM sources are not in this repository); its
 optimum is the one scikit-learn's ``ElasticNet(positive=True)`` finds on the same problem.
@@ -23,6 +24,13 @@ def _int_in(name, v, lo, hi=None):
     return int(v)
 
 
+def _pattern(M):
+    """The binary pattern P of the canonical M (float32 ones): what SLIM and RP3beta train on and score."""
+    P = _canonical(M)
+    P.data = np.ones_like(P.data, dtype=np.float32)
+    return P
+
+
 def _finite_nonneg(name, v):
     v = float(v)
     if not (math.isfinite(v) and v >= 0.0):
@@ -31,6 +39,8 @@ def _finite_nonneg(name, v):
 
 
 class SLIM(ItemItemModel):
+
+    _rows = staticmethod(_pattern)   # P: training and scores see the pattern only
 
     def __init__(self, num_items, num_users, device=None):
         super().__init__(num_items, num_users, device)
@@ -81,8 +91,7 @@ class SLIM(ItemItemModel):
         k = _int_in("k", k, 1, _lib.SLIM_K_MAX)
         max_iter = _int_in("max_iter", max_iter, 1, 2 ** 31 - 1)
         tol = _finite_nonneg("tol", tol)
-        Xc = _canonical(X)
-        Xc.data = np.ones_like(Xc.data, dtype=np.float32)   # P: training and scores see the pattern only
+        Xc = self._rows(X)
         if verbose > 0:
             print("Compute the SLIM weights")
             start = time.time()

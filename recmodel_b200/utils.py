@@ -5,6 +5,8 @@
 * ``test_coverage`` (utils.py:3-18): how often each item appears in the users' top-N over the items they
   have not interacted with; the ranking runs on the device in one ``recommend`` call instead of one ``rank``
   call per user.
+* ``split_users``: the strong-generalisation split of Liang et al. 2018 and Steck 2019 (held-out users, part of
+  each one's history folded in), the protocol of ``recommend_for`` / ``eval_ranking_for``.
 """
 import numpy as np
 
@@ -42,3 +44,20 @@ def test_coverage(cls, Train, topN):
 
 
 test_coverage.__test__ = False  # a library function, not a pytest test
+
+
+def split_users(matrix, held_out, fold_in=0.8, seed=1993):
+    """(Train, FoldIn, Test, held): the strong-generalisation split. ``held`` is the sorted int64 ids
+    ``np.random.default_rng(seed).choice(n_users, held_out, replace=False)``; ``Train`` is the CSR of the other users'
+    rows, in row order; ``FoldIn`` and ``Test`` (``held_out`` rows each, row r for user ``held[r]``) are
+    ``split_train_test(matrix[held], train=fold_in, seed=seed)``: the histories to fold in and the entries to predict.
+    ``matrix`` is not modified."""
+    matrix = matrix.tocsr()
+    n_users = matrix.shape[0]
+    if isinstance(held_out, (bool, np.bool_)) or not isinstance(held_out, (int, np.integer)) or not 0 <= held_out <= n_users:
+        raise ValueError(f"held_out must be an int in 0..{n_users}, got {held_out!r}")
+    held = np.sort(np.random.default_rng(seed).choice(n_users, int(held_out), replace=False)).astype(np.int64)
+    keep = np.ones(n_users, dtype=bool)
+    keep[held] = False
+    fold, test = split_train_test(matrix[held], train=fold_in, seed=seed)
+    return matrix[np.flatnonzero(keep)], fold, test, held

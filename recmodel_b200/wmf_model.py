@@ -16,6 +16,7 @@ Deliberate differences (documented, none changes results beyond rounding):
 import time
 
 import numpy as np
+import scipy.sparse
 import torch
 
 from . import _lib, engine, ranking, sharding
@@ -55,6 +56,9 @@ class WMF(RecModel):
             raise ValueError(f"algo must be one of {sorted(_ALGOS)}")
         self.algo = algo
         self.last_train_stats = {}
+        # the confidence transform of the last train: (pre_process_count, alpha, beta, preprocess_mat), train's defaults
+        # until then, so that a model with assigned factors folds in like a freshly trained one
+        self._transform = ("log", 10, 1, False)
 
     # ---------------------------------------------------------------- factor storage (T2)
     @property
@@ -144,7 +148,7 @@ class WMF(RecModel):
         if ni == 0 or k == 0:
             return np.empty((len(users), 0), dtype=items.dtype)
         cand_d = torch.from_numpy(np.ascontiguousarray(items, dtype=np.int64)).to(self.device)
-        ids = self._rank_ids(users_d, cand_d, k, None, distributed)
+        ids = self._rank_ids(self.users_device, users_d, cand_d, k, None, distributed)
         return ids.cpu().numpy().astype(items.dtype, copy=False)
 
     def recommend(self, users, topn, exclude=None, distributed=False):
@@ -176,13 +180,14 @@ class WMF(RecModel):
     def _recommend_ids(self, users_d, k, ex, distributed=False):
         """Device int64 [len(users_d) x k], k <= num_items: the device part of ``recommend`` (``ex``: a DeviceCSR with
         sorted rows, or None to exclude nothing, where the lists are those of ``rank_batch`` over all items)."""
-        return self._rank_ids(users_d, None, k, ex, distributed)
+        return self._rank_ids(self.users_device, users_d, None, k, ex, distributed)
 
-    def _rank_ids(self, users_d, cand_d, k, ex, distributed):
-        """Device int64 [len(users_d) x k]: the lists of ``rank_batch`` over the device candidate ids ``cand_d`` (None:
-        all items), or, with ``ex`` (a DeviceCSR with sorted rows; needs ``cand_d`` None), those of ``recommend``.
-        ``distributed`` as in ``rank_batch``; lists longer than TOPK_MAX are ranked locally."""
-        U, V, bias = self.users_device, self.items_device, self.bias is True
+    def _rank_ids(self, U, users_d, cand_d, k, ex, distributed):
+        """Device int64 [len(users_d) x k]: the lists of ``rank_batch`` for the rows ``users_d`` of the user factors U
+        over the device candidate ids ``cand_d`` (None: all items), or, with ``ex`` (a DeviceCSR with sorted rows; needs
+        ``cand_d`` None), those of ``recommend``. ``distributed`` as in ``rank_batch``; lists longer than TOPK_MAX are
+        ranked locally."""
+        V, bias = self.items_device, self.bias is True
         if k > _lib.TOPK_MAX:  # very long lists: exact device scores, then stable device sorts, many users per pass
             ni = V.shape[0] if cand_d is None else cand_d.numel()
             return ranking.sort_path_ids(users_d, ni, k, ex, lambda chunk, items_d: engine.predict_pairs(
@@ -230,6 +235,67 @@ class WMF(RecModel):
             lambda: (self.items_device.shape[0], self.users_device.shape[0]),
             "the rows of test_mat and of the user factors", self.device, test_mat, topn, exclude, users)
 
+    # ---------------------------------------------------------------- fold-in (DESIGN.md 4.10)
+    def _confidence(self, rows_d, counts):
+        """The uploaded users x items DeviceCSR ``rows_d`` with the transform of the last ``train`` applied to its
+        values: ``counts`` True for the count matrix of weighted training (always transformed), False for the
+        utility matrix (transformed only with ``preprocess_mat``)."""
+        mode, alpha, beta, preprocess_mat = self._transform
+        if counts:
+            return rows_d.with_data(engine.preprocess_(rows_d.data, mode, alpha, beta))
+        if preprocess_mat == True and mode in ("log", "linear"):  # noqa: E712  (wmf_model.py:65-70)
+            return rows_d.with_data(engine.preprocess_(rows_d.data.clone(), mode, alpha, beta))
+        return rows_d
+
+    def _fold_in_device(self, count_rows):
+        """Device float32 [rows x f]: the user half-step of ``train`` for the rows of ``count_rows`` (new users x items
+        SciPy, counts for weighted models, utilities otherwise) against the fixed item factors."""
+        V = self.items_device
+        if V is None:
+            raise ValueError("the model has no item factors")
+        if not scipy.sparse.issparse(count_rows) or count_rows.shape[1] != V.shape[0]:
+            raise ValueError(f"count_rows must be a SciPy sparse matrix with {V.shape[0]} columns (the items), got "
+                             f"{getattr(count_rows, 'shape', type(count_rows).__name__)}")
+        if count_rows.shape[0] == 0:
+            return torch.empty((0, V.shape[1]), dtype=torch.float32, device=self.device)
+        weighted = self.weighted is True
+        C = self._confidence(DeviceCSR.from_scipy(count_rows, self.device), counts=weighted)
+        if not weighted:
+            return engine.unweighted_half_step(C, V, self.gamma)                      # :85
+        bias = self.bias is True
+        G = engine.gram(V, self.gamma, ones_col0=bias)                                 # epoch.ResidentEpoch, stage 0
+        return engine.half_step(C, V, G, bias=bias, algo=_ALGOS[self.algo])
+
+    def fold_in(self, count_rows):
+        """float32 [rows x f] (a new ndarray): the user factors of the new users whose histories are the rows of
+        ``count_rows`` (new users x items, any SciPy format, in the form ``train`` takes: ``count_mat`` when weighted,
+        ``utility_mat`` otherwise; not modified), solved against the fixed item factors. This is the user half-step of
+        ``train`` with its confidence transform (pre_process_count, alpha, beta, preprocess_mat of the last ``train``,
+        its defaults before one): a row's factors are bitwise those ``train`` gives the same row, whatever other rows
+        share the call."""
+        return self._fold_in_device(count_rows).cpu().numpy()
+
+    def recommend_for(self, user_items, topn, exclude=True):
+        """int64 [user_items.shape[0] x topn]: ``recommend`` for users that are not rows of the user factors. Row r is
+        the top-``topn`` of all items for the user whose factors ``fold_in`` solves from row r of ``user_items``, best
+        first, ties to the lower item id, -1 padding. ``exclude``: True leaves out each row's own stored entries
+        (whatever their value), None nothing, a SciPy matrix or DeviceCSR of the shape of ``user_items`` its stored
+        entries. A local call (no ``distributed``)."""
+        return ranking.recommend_for(self._fold_in_device, self._fold_in_rank_ids, self.items_device.shape[0],
+                                     self.device, user_items, topn, exclude)
+
+    def eval_ranking_for(self, user_items, test_mat, topn=np.array([10]), exclude=True, users=None):
+        """``eval_ranking`` (the same metrics and definitions) over the lists of ``recommend_for(user_items, K,
+        exclude)``, K = max(topn): the strong-generalisation protocol, where the evaluated users are not rows of the
+        user factors. ``test_mat`` has the shape of ``user_items``; ``users`` (ids into its rows) defaults to the rows of
+        ``test_mat`` with stored entries. The factors are folded in once per call; no list leaves the device and the
+        result is bitwise reproducible."""
+        return ranking.eval_ranking_for(self._fold_in_device, self._fold_in_rank_ids, self.items_device.shape[0],
+                                        self.device, user_items, test_mat, topn, exclude, users)
+
+    def _fold_in_rank_ids(self, U, users_d, k, ex):
+        return self._rank_ids(U, users_d, None, k, None if ex is None else ex.sorted(), False)
+
     # ---------------------------------------------------------------- train (R2, R7, R11)
     def train(self, utility_mat, iterations, verbose=0, eval_mat=None, count_mat=None, alpha=10,
               cores=4, stopping_rounds=3, dtype="float64", min_improvement=0.0001,
@@ -245,11 +311,10 @@ class WMF(RecModel):
         dev = self.device
         t_start = self._t_train_start = time.perf_counter()
 
+        self._transform = (pre_process_count, alpha, beta, preprocess_mat)
         util_d = None
         if preprocess_mat == True or verbose > 1 or self.weighted is not True:  # noqa: E712
-            util_d = DeviceCSR.from_scipy(utility_mat, dev)
-            if preprocess_mat == True and pre_process_count in ("log", "linear"):  # noqa: E712  (:65-70)
-                util_d = util_d.with_data(engine.preprocess_(util_d.data.clone(), pre_process_count, alpha, beta))
+            util_d = self._confidence(DeviceCSR.from_scipy(utility_mat, dev), counts=False)
 
         stats = {"half_step_ms": [], "eval_ms": [], "setup_ms": 0.0}
         if self.weighted is not True:
@@ -264,7 +329,7 @@ class WMF(RecModel):
             # the matrix between the GPUs instead cost more than it saved (31 ms against 22 ms at 2 GPUs, round 1).
             C_full = DeviceCSR.from_scipy(count_mat, dev)
             stats["host_marks_ms"] = [("upload issued", (time.perf_counter() - t_start) * 1e3)]
-            C_full = C_full.with_data(engine.preprocess_(C_full.data, pre_process_count, alpha, beta))
+            C_full = self._confidence(C_full, counts=True)
             CT_full = C_full.transpose()  # count_mat.T.tocsr()  (:128)
             stats["host_marks_ms"].append(("transpose issued", (time.perf_counter() - t_start) * 1e3))
             it = self._train_weighted(C_full, CT_full, util_d, iterations, verbose, eval_mat, cores, stopping_rounds,

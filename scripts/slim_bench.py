@@ -114,10 +114,11 @@ def main():
     users_d = torch.from_numpy(users).to(dev)
 
     def rec():
-        return m._recommend_ids(users_d, TOPN, ex)
+        return m._recommend_ids(*m._X_and_W(), users_d, TOPN, ex)
 
     def ev_device():
-        return ranking.eval_ranking_sums(m._recommend_ids, ITEMS, T, ex, users_d, np.asarray(KS, np.int64))
+        return ranking.eval_ranking_sums(lambda u, k, e: m._recommend_ids(*m._X_and_W(), u, k, e), ITEMS, T, ex,
+                                         users_d, np.asarray(KS, np.int64))
 
     ids0 = rec()
     sums0 = ev_device()
